@@ -68,7 +68,12 @@ def parse_args():
     ap.add_argument("--cpu-queries", type=int, default=2_000)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--refine", action="store_true", help="VSB_FLAG_BUILD_REFINE: vsb_build ends with one refinement pass")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the keys and distances the last timed step returned to DIR/*.npy "
+                         "(pin --search-width when comparing two builds: it is otherwise picked by timing)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     cfg = CONFIGS[a.config]
     if a.n is None:
         a.n = cfg["n"]
@@ -98,6 +103,27 @@ def load_peaks():
         except Exception:
             pass
     return 6650.0, 1666.0, "fallback (B200_PROFILING.md)"
+
+
+DUMP_BUDGET = 64 << 20  # bytes --dump-outputs may write
+
+
+def dump_outputs(out_dir, keys, dists, budget=DUMP_BUDGET):
+    """One step's results, [queries, k] each, for an output-by-output comparison of two builds: keys.npy (float64: keys
+    below 2^53 are exact, the empty-slot key 2^64 - 1 reads 2^64), distances.npy (float32) and query_rows.npy (float64,
+    the query of each row, numbered through the step's batches).  Above `budget` bytes a fixed seeded sample of the
+    queries is written.  Inputs, graph build and search are deterministic: the same arguments give the same arrays."""
+    keys = np.asarray(keys, dtype=np.uint64)
+    dists = np.asarray(dists, dtype=np.float32)
+    n, k = keys.shape
+    rows = np.arange(n)
+    per_row = k * (8 + 4) + 8
+    if n * per_row > budget - 1024:  # 1024: the three .npy headers
+        rows = np.sort(np.random.default_rng(0).choice(n, (budget - 1024) // per_row, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "keys.npy"), keys[rows].astype(np.float64))
+    np.save(os.path.join(out_dir, "distances.npy"), dists[rows])
+    np.save(os.path.join(out_dir, "query_rows.npy"), rows.astype(np.float64))
 
 
 class ClockSampler:
@@ -207,8 +233,10 @@ def cpu_hnsw_run(a, steps, warmup, full_line):
         h.search(q, a.k)
     t0 = time.perf_counter()
     for _ in range(steps):
-        h.search(q, a.k)
+        hk, hd = h.search(q, a.k)
     dt = time.perf_counter() - t0
+    if full_line and a.dump_outputs:
+        dump_outputs(a.dump_outputs, hk, hd)
     qps = steps * len(q) / dt
     lat = []
     for i in range(200):
@@ -386,7 +414,8 @@ def main():
                 "d": [torch.empty((B, k), dtype=torch.float32, device=dev) for _ in range(2)],
                 "searched": [torch.cuda.Event() for _ in range(2)], "exchanged": [torch.cuda.Event() for _ in range(2)]}
 
-    def search_batch_pipelined(q_ptr, timed):
+    def search_batch_pipelined(q_ptr, timed, out=None):
+        out_k, out_d = out if out is not None else (out_k0, out_d0)
         p = pipe["j"] % 2
         pipe["j"] += 1
         main = torch.cuda.current_stream()
@@ -399,7 +428,7 @@ def main():
             if timed:
                 e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
                 e0.record(sx)
-            xchg.allgather_merge(pipe["k"][p].data_ptr(), pipe["d"][p].data_ptr(), B, k, out_k0.data_ptr(), out_d0.data_ptr(), 0,
+            xchg.allgather_merge(pipe["k"][p].data_ptr(), pipe["d"][p].data_ptr(), B, k, out_k.data_ptr(), out_d.data_ptr(), 0,
                                  sx.cuda_stream)
             if timed:
                 e1.record(sx)
@@ -501,14 +530,22 @@ def main():
     bytes_per_query = E * (trav_row_bytes + 4) + P * st["graph_degree"] * 4  # +4: the row's norm (cosine)
 
     # ---- timed region 1: inputs resident in HBM ----
-    def dev_step(timed=False):
+    def dev_step(timed=False, outs=None):
         for j in range(R):
+            out = None if outs is None else outs[j]
             if pipe is not None:
-                search_batch_pipelined(q_dev[j % NB].data_ptr(), timed)
+                search_batch_pipelined(q_dev[j % NB].data_ptr(), timed, out)
             else:
-                search_batch_dev(q_dev[j % NB].data_ptr(), timed=timed)
+                search_batch_dev(q_dev[j % NB].data_ptr(), timed=timed, out=out)
         if pipe is not None:
             torch.cuda.current_stream().wait_stream(pipe["stream"])  # the step ends when its last exchange has merged
+
+    # --dump-outputs: every batch of the last timed step writes its own result buffers (the last batch the usual ones,
+    # which recall_of reads), so the whole step's results are still there after it
+    last_outs = None
+    if a.dump_outputs:
+        last_outs = [(torch.empty((B, k), dtype=torch.int64, device=dev), torch.empty((B, k), dtype=torch.float32, device=dev))
+                     for _ in range(R - 1)] + [(out_k0, out_d0)]
 
     for i in range(a.warmup):
         dev_step()
@@ -521,7 +558,7 @@ def main():
     sampler.mark_begin()
     ev0.record()
     for i in range(a.steps):
-        dev_step(timed=True)
+        dev_step(timed=True, outs=last_outs if i == a.steps - 1 else None)
     ev1.record()
     barrier()
     sampler.mark_end()
@@ -538,6 +575,9 @@ def main():
     ms = float(t.item())
     value = n_batches * B / (ms * 1e-3)
     recall_timed = recall_of((R - 1) % NB)
+    if last_outs is not None and rank == 0:
+        dump_outputs(a.dump_outputs, torch.cat([o[0] for o in last_outs]).cpu().numpy().view(np.uint64),
+                     torch.cat([o[1] for o in last_outs]).cpu().numpy())
 
     k4_ms = st["graph_search_ns"] / 1e6 / max(st["graph_search_launches"], 1)
     peak, tensor_peak, peak_src = load_peaks()

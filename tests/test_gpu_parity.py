@@ -555,6 +555,28 @@ def test_hybrid_build_allpairs_prefix_plus_streaming():
     assert np.all(gc == k) and r >= 0.93
 
 
+def test_streamed_build_is_deterministic(monkeypatch):
+    # K7 links the rows beyond the all-pairs prefix in batches of 8192, and the reverse links of one batch compete for
+    # the same old rows: two builds of the same rows must still give the same graph bit for bit, and the same results
+    n, dim, k = 60000, 64, 10
+    x = embedding_like(n, dim, n_clusters=32)
+    q = embedding_like(500, dim, seed=4321, n_clusters=32)
+    keys = np.arange(n, dtype=np.uint64)
+    monkeypatch.setenv("VSB_ALLPAIRS_MAX", "10000")                   # read when the index is created
+    monkeypatch.setenv("VSB_ALLPAIRS_PREFIX", "10000")
+    runs = []
+    for _ in range(2):
+        idx = make_index(x, keys, O.COS, O.BF16)
+        idx.build()
+        assert idx.build_stats()["stream_rows"] == n - 10000
+        rows, _ = idx.export_graph()
+        runs.append((rows, idx.search_batch(q, k)))
+        idx.close()
+    (g0, r0), (g1, r1) = runs
+    assert np.array_equal(g0, g1), f"{(g0 != g1).any(axis=1).sum()} rows differ"
+    assert all(np.array_equal(a, b) for a, b in zip(r0, r1))
+
+
 def test_snapshot_roundtrip(tmp_path):
     # N3: save / load reproduces exact and ANN results (keys, tombstones, rows, graph)
     n, dim, k = 20000, 64, 10

@@ -226,8 +226,11 @@ void launch_merge_graph(const uint32_t* fwd, const uint32_t* rev, const uint32_t
 //                     keep the R candidates with the smallest (detour, j) — a diverse neighbourhood instead of
 //                     the R closest, which is what keeps recall from decaying between refinement passes.
 //   stream_link_rev : each of the R/2 first neighbours v of u gets u written into the reverse half of row(v):
-//                     an empty slot if there is one, otherwise a pseudo-randomly chosen one is replaced
-//                     (single-word atomics, so concurrent inserts into the same row never tear it).
+//                     an empty slot if there is one, otherwise a pseudo-randomly chosen one is replaced.  The
+//                     batch's proposals are radix sorted by (v, rank, u) and one warp applies all proposals to
+//                     row(v) in that order: the closest links first, as when the batch's warps step through
+//                     their ranks together, but independent of the order warps run in.  A reverse edge is one
+//                     32-bit store: searches walking the same buffer never see a torn row.
 // Rows of one batch do not link to each other; refinement passes re-optimise the graph.
 namespace vsb {
 namespace {
@@ -327,34 +330,44 @@ __global__ void __launch_bounds__(K7_WARPS * 32) stream_link_fwd_kernel(const ui
     for (uint32_t r = count + lane; r < graph_stride; r += 32) out[r] = kInvalidSlot;
 }
 
-__global__ void __launch_bounds__(128) stream_link_rev_kernel(uint32_t n_new, uint32_t first_slot, uint32_t R,
-                                                              uint32_t* __restrict__ graph, uint32_t graph_stride) {
+// reverse-edge proposals of one batch: key = v << 32 | r * n_new + (u - first_slot)  (n_new * half < 2^32)
+__global__ void stream_proposals_kernel(const uint32_t* __restrict__ graph, uint32_t graph_stride, uint32_t n_new,
+                                        uint32_t first_slot, uint32_t half, uint64_t* __restrict__ out) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (size_t)n_new * half) return;
+    const uint32_t u = first_slot + (uint32_t)(i / half), r = (uint32_t)(i % half);
+    const uint32_t v = graph[(size_t)u * graph_stride + r];
+    out[i] = (v == kInvalidSlot || v >= first_slot) ? kInvalidPacked
+                                                    : (((uint64_t)v << 32) | ((uint64_t)r * n_new + (u - first_slot)));
+}
+
+// one warp per target row v (the warp of its segment's first entry) applies the segment's proposals in sorted order;
+// the lanes scan the reverse half of row(v) 32 slots at a time
+__global__ void __launch_bounds__(256) stream_link_rev_kernel(const uint64_t* __restrict__ sorted, size_t m, uint32_t n_new,
+                                                              uint32_t first_slot, uint32_t R, uint32_t* __restrict__ graph,
+                                                              uint32_t graph_stride) {
     const int lane = threadIdx.x & 31;
-    const uint32_t i = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-    if (i >= n_new) return;
-    const uint32_t u = first_slot + i;
+    const size_t i = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (i >= m || sorted[i] == kInvalidPacked) return;  // uniform across the warp
+    const uint32_t v = (uint32_t)(sorted[i] >> 32);
+    if (i > 0 && (uint32_t)(sorted[i - 1] >> 32) == v) return;
     const uint32_t half = R / 2;
-    const uint32_t* row = graph + (size_t)u * graph_stride;
-    for (uint32_t r = 0; r < half; ++r) {
-        const uint32_t v = row[r];
-        if (v == kInvalidSlot || v >= first_slot) continue;  // uniform across the warp
-        uint32_t* vrow = graph + (size_t)v * graph_stride;
-        const uint32_t pos = half + lane;
-        const uint32_t cur = pos < R ? vrow[pos] : 0u;
-        if (__ballot_sync(kFullMask, pos < R && cur == u) != 0) continue;  // already linked
-        const uint32_t empties = __ballot_sync(kFullMask, pos < R && cur == kInvalidSlot);
-        bool done = false;
-        if (empties != 0) {
-            const int src = __ffs(empties) - 1;
-            uint32_t old = kInvalidSlot;
-            if (lane == src) old = atomicCAS(&vrow[pos], kInvalidSlot, u);
-            old = __shfl_sync(kFullMask, old, src);
-            done = old == kInvalidSlot;
+    uint32_t* vrow = graph + (size_t)v * graph_stride;
+    for (size_t e = i; e < m && (uint32_t)(sorted[e] >> 32) == v; ++e) {  // kInvalidPacked >> 32 is no slot
+        const uint32_t idx = (uint32_t)sorted[e];
+        const uint32_t u = first_slot + idx % n_new, r = idx / n_new;
+        bool linked = false;
+        uint32_t empty = kInvalidSlot;
+        for (uint32_t base = half; base < R; base += 32) {
+            const uint32_t pos = base + lane;
+            const uint32_t cur = pos < R ? vrow[pos] : 0u;
+            linked |= __ballot_sync(kFullMask, pos < R && cur == u) != 0;
+            const uint32_t empties = __ballot_sync(kFullMask, pos < R && cur == kInvalidSlot);
+            if (empty == kInvalidSlot && empties != 0) empty = base + __ffs(empties) - 1;
         }
-        if (!done && lane == 0) {
-            const uint32_t p = half + ((u * 0x9E3779B1u + r * 0x85EBCA6Bu) >> 16) % (R - half);
-            atomicExch(&vrow[p], u);
-        }
+        if (!linked && lane == 0)
+            vrow[empty != kInvalidSlot ? empty : half + ((u * 0x9E3779B1u + r * 0x85EBCA6Bu) >> 16) % (R - half)] = u;
+        __syncwarp();  // the next proposal's scan sees this store
     }
 }
 
@@ -371,13 +384,35 @@ __global__ void remap_graph_kernel(const uint32_t* __restrict__ graph, uint32_t 
 }
 }  // namespace
 
-void launch_stream_link(const uint64_t* cand, uint32_t n_new, uint32_t cand_stride, uint32_t first_slot, uint32_t R,
-                        uint32_t* graph, uint32_t graph_stride, cudaStream_t stream) {
-    if (n_new == 0) return;
+size_t stream_link_scratch_bytes(uint32_t n_new, uint32_t R) {
+    const size_t m = (size_t)n_new * (R / 2);
+    size_t temp = 0;
+    cub::DeviceRadixSort::SortKeys(nullptr, temp, (const uint64_t*)nullptr, (uint64_t*)nullptr, m, 0, 64);
+    return align_up(m * 8, 256) * 2 + align_up(temp, 256);
+}
+
+cudaError_t launch_stream_link(const uint64_t* cand, uint32_t n_new, uint32_t cand_stride, uint32_t first_slot, uint32_t R,
+                               uint32_t* graph, uint32_t graph_stride, void* scratch, size_t scratch_bytes,
+                               cudaStream_t stream) {
+    if (n_new == 0) return cudaSuccess;
     stream_link_fwd_kernel<<<(n_new + K7_WARPS - 1) / K7_WARPS, K7_WARPS * 32, 0, stream>>>(cand, n_new, cand_stride, first_slot,
                                                                                             R, graph, graph_stride);
-    stream_link_rev_kernel<<<(n_new + 3) / 4, 128, 0, stream>>>(n_new, first_slot, R, graph, graph_stride);
+    const size_t m = (size_t)n_new * (R / 2);
+    uint8_t* base = static_cast<uint8_t*>(scratch);
+    uint64_t* prop = reinterpret_cast<uint64_t*>(base);
+    uint64_t* sorted = reinterpret_cast<uint64_t*>(base + align_up(m * 8, 256));
+    size_t temp_bytes = scratch_bytes - 2 * align_up(m * 8, 256);
+    const int T = 256;
+    stream_proposals_kernel<<<(unsigned)((m + T - 1) / T), T, 0, stream>>>(graph, graph_stride, n_new, first_slot, R / 2, prop);
     g_kernel_launches += 2;
+    // targets are below first_slot: the key's high word needs bit_width(first_slot - 1) bits (kInvalidPacked still sorts last)
+    const int end_bit = 32 + (first_slot > 1 ? 32 - __builtin_clz(first_slot - 1) : 1);
+    cudaError_t e = cub::DeviceRadixSort::SortKeys(base + 2 * align_up(m * 8, 256), temp_bytes, prop, sorted, m, 0, end_bit,
+                                                   stream);
+    if (e != cudaSuccess) return e;
+    stream_link_rev_kernel<<<(unsigned)((m * 32 + T - 1) / T), T, 0, stream>>>(sorted, m, n_new, first_slot, R, graph, graph_stride);
+    g_kernel_launches += 1;  // + the CUB radix-sort passes, which are library kernels and not counted
+    return cudaGetLastError();
 }
 
 void launch_remap_graph(const uint32_t* graph, uint32_t n_old, uint32_t stride, const uint32_t* old2new, uint32_t* out,

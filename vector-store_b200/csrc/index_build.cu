@@ -369,9 +369,11 @@ vsb_status vsb_index::stream_insert() {
     run.max_iters = 0;
     run.n_seeds = 32;
     run.search_width = build_search_width;
-    DevBuf cand;
+    DevBuf cand, link_scratch;
     const uint32_t QB = 8192;
     CU(cand.alloc((size_t)QB * C * 8));
+    const size_t link_bytes = vsb::stream_link_scratch_bytes(QB, R);
+    CU(link_scratch.alloc(link_bytes));
     EvTimer t(mstream);
     while (w.n_graphed < w.n_slots) {
         // the entry points follow the graph: a sample drawn when the graph was half its size (at the start of a bulk
@@ -395,8 +397,8 @@ vsb_status vsb_index::stream_insert() {
         }
         ST(graph_block(w, ms, run, qv, nb, C, nullptr, nullptr, nullptr, cand.as<uint64_t>(), trav16 ? &q16 : nullptr, mstream,
                        -1, false, &bstats.stream_evals, &bstats.stream_parents));
-        vsb::launch_stream_link(cand.as<uint64_t>(), nb, C, t0, R, w.gr->g.as<uint32_t>(), graph_stride, mstream);
-        CU(cudaGetLastError());
+        CU(vsb::launch_stream_link(cand.as<uint64_t>(), nb, C, t0, R, w.gr->g.as<uint32_t>(), graph_stride, link_scratch.p,
+                                   link_bytes, mstream));
         w.n_graphed = t0 + nb;  // later batches may link to these rows (stream order)
         churn_since_refine += nb;
         bstats.stream_rows += nb;

@@ -118,9 +118,11 @@ void launch_remap_graph(const uint32_t* graph, uint32_t n_old, uint32_t stride, 
                         cudaStream_t stream);
 
 // K7 (graph_build.cu): link a batch of already-searched new rows into the graph (detour-pruned forward rows,
-// then reverse edges); cand = [n_new][cand_stride] packed ascending candidates
-void launch_stream_link(const uint64_t* cand, uint32_t n_new, uint32_t cand_stride, uint32_t first_slot, uint32_t R,
-                        uint32_t* graph, uint32_t graph_stride, cudaStream_t stream);
+// then reverse edges in a deterministic order); cand = [n_new][cand_stride] packed ascending candidates
+size_t stream_link_scratch_bytes(uint32_t n_new, uint32_t R);
+cudaError_t launch_stream_link(const uint64_t* cand, uint32_t n_new, uint32_t cand_stride, uint32_t first_slot, uint32_t R,
+                               uint32_t* graph, uint32_t graph_stride, void* scratch, size_t scratch_bytes,
+                               cudaStream_t stream);
 
 // K4 (graph_search.cu) ---------------------------------------------------------------------------
 struct SearchParams {
