@@ -237,6 +237,16 @@ vsb_status vsb_search_exact(vsb_index* index, const float* queries, uint64_t q, 
 vsb_status vsb_search_filtered(vsb_index* index, const float* queries, uint64_t q, uint32_t k,
                                const uint32_t* allow_bitmap, uint64_t bitmap_bits,
                                uint64_t* keys, float* distances, uint32_t* counts);
+/* filtered_search for q queries that each carry their own predicate.  allow_bitmaps: n_filters bitmaps
+ * back to back, each ceil(bitmap_bits/32) words, same bit convention as vsb_search_filtered; query i is
+ * filtered by bitmap filter_of_query[i] (< n_filters).  Per filter, the same rule as vsb_search_filtered
+ * picks the graph or the exact bitmap scan, so one call may use both; results come back in the caller's
+ * query order.  With n_filters = 1 the results are those of vsb_search_filtered.  VSB_EINVAL for a null
+ * pointer (counts may be NULL), n_filters == 0, n_filters > q or any filter_of_query[i] >= n_filters. */
+vsb_status vsb_search_filtered_multi(vsb_index* index, const float* queries, uint64_t q, uint32_t k,
+                                     const uint32_t* allow_bitmaps, uint32_t n_filters, uint64_t bitmap_bits,
+                                     const uint32_t* filter_of_query,
+                                     uint64_t* keys, float* distances, uint32_t* counts);
 
 /* Device-resident variants: d_* are device pointers on the index's device,
  * `stream` is a cudaStream_t.  No host synchronisation, except `exact` != 0 (brute force) on float rows,

@@ -16,6 +16,7 @@
  * (usearch.rs:515-624).  A GPU wants batches and needs no gate (libvsb200 searches a published view while mutators
  * prepare the next one), so the loop drains what is already queued and coalesces RUNS of compatible messages:
  *   Ann x n on one partition         -> one vsb_search(q = n)
+ *   FilteredAnn x n on one partition -> one vsb_search_filtered_multi(q = n), one bitmap per distinct predicate
  *   AddVector x n on one partition   -> one vsb_add_each(n)     (per-row status: one bad row fails alone)
  *   RemoveVector x n                 -> one vsb_remove(n)
  * Order inside a partition is preserved (an update is RemoveVector followed by AddVector of the same row).
@@ -51,6 +52,7 @@ use crate::worker::WorkerExt;
 use anyhow::anyhow;
 use anyhow::bail;
 use std::collections::BTreeMap;
+use std::collections::HashMap;
 use std::sync::Arc;
 use std::sync::Mutex;
 use std::sync::RwLock;
@@ -231,46 +233,67 @@ impl GpuIndex {
 
     /// The host predicate of usearch.rs:224-248 becomes a bitmap over row ids, built once per request over the rows
     /// that are in the index, and the graph is traversed on the device with the bit tested where a result is emitted.
-    fn search_filtered(
+    /// A run of q requests is one call: `predicate(i, id)` is request i's predicate, identical bitmaps are sent once,
+    /// every request is answered with its own bitmap and k, and the answers come back in request order.
+    fn search_filtered_many(
         &self,
-        query: &[f32],
+        queries: &[f32],
+        q: usize,
         k: usize,
-        predicate: impl Fn(PrimaryId) -> bool,
-    ) -> anyhow::Result<Vec<(PrimaryId, Distance)>> {
-        let allow: Vec<u32> = {
+        predicate: impl Fn(usize, PrimaryId) -> bool,
+    ) -> anyhow::Result<Vec<Vec<(PrimaryId, Distance)>>> {
+        let (allow, n_filters, words, filter_of_query) = {
             let live = self.live_rows.lock().unwrap();
-            live.iter()
-                .enumerate()
-                .map(|(w, word)| {
-                    let mut out = 0u32;
-                    let mut bits = *word;
-                    while bits != 0 {
-                        let b = bits.trailing_zeros();
-                        bits &= bits - 1;
-                        // the epoch is not part of the row id the table is asked about (Idx::idx masks it off)
-                        if predicate(PrimaryId::from((w as u64) * 32 + b as u64)) {
-                            out |= 1u32 << b;
+            let words = live.len();
+            let mut allow: Vec<u32> = Vec::new();
+            let mut seen: HashMap<Vec<u32>, u32> = HashMap::new();
+            let mut filter_of_query = Vec::with_capacity(q);
+            for i in 0..q {
+                let bitmap: Vec<u32> = live
+                    .iter()
+                    .enumerate()
+                    .map(|(w, word)| {
+                        let mut out = 0u32;
+                        let mut bits = *word;
+                        while bits != 0 {
+                            let b = bits.trailing_zeros();
+                            bits &= bits - 1;
+                            // the epoch is not part of the row id the table is asked about (Idx::idx masks it off)
+                            if predicate(i, PrimaryId::from((w as u64) * 32 + b as u64)) {
+                                out |= 1u32 << b;
+                            }
                         }
-                    }
-                    out
-                })
-                .collect()
+                        out
+                    })
+                    .collect();
+                let next = seen.len() as u32;
+                let f = *seen.entry(bitmap).or_insert_with_key(|bitmap| {
+                    allow.extend_from_slice(bitmap);
+                    next
+                });
+                filter_of_query.push(f);
+            }
+            (allow, seen.len(), words, filter_of_query)
         };
-        let (mut keys, mut dists, mut count) = (vec![0u64; k], vec![0f32; k], 0u32);
+        let (mut keys, mut dists, mut counts) = (vec![0u64; q * k], vec![0f32; q * k], vec![0u32; q]);
         check(unsafe {
-            sys::vsb_search_filtered(
+            sys::vsb_search_filtered_multi(
                 self.h,
-                query.as_ptr(),
-                1,
+                queries.as_ptr(),
+                q as u64,
                 k as u32,
                 allow.as_ptr(),
-                (allow.len() * 32) as u64,
+                n_filters as u32,
+                (words * 32) as u64,
+                filter_of_query.as_ptr(),
                 keys.as_mut_ptr(),
                 dists.as_mut_ptr(),
-                &mut count,
+                counts.as_mut_ptr(),
             )
         })?;
-        self.unpack(&keys, &dists, count as usize)
+        (0..q)
+            .map(|i| self.unpack(&keys[i * k..(i + 1) * k], &dists[i * k..(i + 1) * k], counts[i] as usize))
+            .collect()
     }
 }
 
@@ -335,10 +358,10 @@ enum Run {
     },
     FilteredAnn {
         partition: Arc<PartitionState>,
-        embedding: Vector,
-        filter: Filter,
-        limit: Limit,
-        tx: oneshot::Sender<AnnR>,
+        queries: Vec<f32>,
+        filters: Vec<Filter>,
+        limits: Vec<usize>,
+        txs: Vec<oneshot::Sender<AnnR>>,
     },
 }
 
@@ -421,26 +444,35 @@ fn execute(run: Run, table: &RwLock<impl TableSearch>, index_size: &AtomicUsize)
         }
         Run::FilteredAnn {
             partition,
-            embedding,
-            filter,
-            limit,
-            tx,
+            queries,
+            filters,
+            limits,
+            txs,
         } => {
-            let id_ok = |primary_id: PrimaryId| {
+            let id_ok = |i: usize, primary_id: PrimaryId| {
                 let table = table.read().unwrap();
-                filter
+                filters[i]
                     .restrictions
                     .iter()
                     .all(|restriction| table.is_valid_for(partition.partition_id, primary_id, restriction))
             };
-            tx.send(
-                partition
-                    .idx
-                    .search_filtered(embedding.as_slice(), limit.0.get(), id_ok)
-                    .map_err(|err| anyhow!("filtered search failed: {err}"))
-                    .map(|hits| to_primary_keys(&partition, table, hits)),
-            )
-            .unwrap_or_else(|_| trace!("the requester of an ann went away"));
+            let k = limits.iter().copied().max().unwrap_or(1);
+            match partition.idx.search_filtered_many(&queries, txs.len(), k, id_ok) {
+                Err(err) => {
+                    let msg = err.to_string();
+                    for tx in txs {
+                        tx.send(Err(anyhow!("filtered search failed: {msg}")))
+                            .unwrap_or_else(|_| trace!("the requester of an ann went away"));
+                    }
+                }
+                Ok(per_query) => {
+                    for ((hits, limit), tx) in per_query.into_iter().zip(limits).zip(txs) {
+                        let hits = hits.into_iter().take(limit).collect();
+                        tx.send(Ok(to_primary_keys(&partition, table, hits)))
+                            .unwrap_or_else(|_| trace!("the requester of an ann went away"));
+                    }
+                }
+            }
         }
     }
 }
@@ -625,15 +657,33 @@ fn enqueue(
                         _ = tx.send(Err(err));
                         return;
                     }
+                    let filter = Filter {
+                        restrictions,
+                        allow_filtering: filter.allow_filtering,
+                    };
+                    // consecutive FilteredAnn requests on one partition share one call, like Ann runs (push_ann)
+                    if let Some(Run::FilteredAnn {
+                        partition: p,
+                        queries,
+                        filters,
+                        limits,
+                        txs,
+                    }) = runs.last_mut()
+                        && same(p, &partition)
+                        && txs.len() < MAX_RUN
+                    {
+                        queries.extend_from_slice(embedding.as_slice());
+                        filters.push(filter);
+                        limits.push(limit.0.get());
+                        txs.push(tx);
+                        return;
+                    }
                     runs.push(Run::FilteredAnn {
                         partition,
-                        embedding,
-                        filter: Filter {
-                            restrictions,
-                            allow_filtering: filter.allow_filtering,
-                        },
-                        limit,
-                        tx,
+                        queries: embedding.as_slice().to_vec(),
+                        filters: vec![filter],
+                        limits: vec![limit.0.get()],
+                        txs: vec![tx],
                     });
                 }
             }

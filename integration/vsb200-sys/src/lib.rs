@@ -200,6 +200,19 @@ unsafe extern "C" {
         distances: *mut f32,
         counts: *mut u32,
     ) -> vsb_status;
+    pub fn vsb_search_filtered_multi(
+        index: *mut vsb_index,
+        queries: *const f32,
+        q: u64,
+        k: u32,
+        allow_bitmaps: *const u32,
+        n_filters: u32,
+        bitmap_bits: u64,
+        filter_of_query: *const u32,
+        keys: *mut u64,
+        distances: *mut f32,
+        counts: *mut u32,
+    ) -> vsb_status;
     pub fn vsb_search_dev(
         index: *mut vsb_index,
         d_queries: *const f32,

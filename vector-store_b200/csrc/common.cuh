@@ -61,6 +61,13 @@ __device__ __forceinline__ bool bit_test(const uint32_t* bm, uint32_t i) {
     return (bm[i >> 5] >> (i & 31)) & 1u;
 }
 
+// Filtered search: the bitmaps of a call lie back to back, ceil(bits / 32) words each; query q tests bitmap
+// allow_of_q[q] (a null index array means bitmap 0 for every query)
+__device__ __forceinline__ const uint32_t* query_allow(const uint32_t* allow, uint64_t bits, const uint32_t* allow_of_q,
+                                                       uint32_t q) {
+    return allow_of_q == nullptr ? allow : allow + (size_t)allow_of_q[q] * (size_t)((bits + 31) / 32);
+}
+
 // ---- warp helpers ------------------------------------------------------------------------------
 __device__ __forceinline__ float butterfly_sum(float v) {
     v = __fadd_rn(v, __shfl_xor_sync(kFullMask, v, 16));

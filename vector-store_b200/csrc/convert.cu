@@ -157,6 +157,41 @@ void launch_gather_u64(const uint64_t* in, const uint32_t* slots, uint32_t n, ui
     g_kernel_launches += 1;
 }
 
+__global__ void gather_u32_kernel(const uint32_t* __restrict__ in, const uint32_t* __restrict__ slots, uint32_t n,
+                                  uint32_t* __restrict__ out) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) out[i] = in[slots[i]];
+}
+
+void launch_gather_u32(const uint32_t* in, const uint32_t* slots, uint32_t n, uint32_t* out, cudaStream_t stream) {
+    if (n == 0) return;
+    gather_u32_kernel<<<(n + 255) / 256, 256, 0, stream>>>(in, slots, n, out);
+    g_kernel_launches += 1;
+}
+
+// one thread per result entry; thread 0 of a row also moves its count
+__global__ void scatter_topk_kernel(const uint64_t* __restrict__ keys, const float* __restrict__ dists,
+                                    const uint32_t* __restrict__ counts, const uint32_t* __restrict__ map, uint32_t n,
+                                    uint32_t k, uint64_t* __restrict__ out_keys, float* __restrict__ out_dists,
+                                    uint32_t* __restrict__ out_counts) {
+    const uint64_t e = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= (uint64_t)n * k) return;
+    const uint32_t i = (uint32_t)(e / k), j = (uint32_t)(e % k);
+    const uint64_t dst = (uint64_t)map[i] * k + j;
+    out_keys[dst] = keys[e];
+    out_dists[dst] = dists[e];
+    if (j == 0 && counts != nullptr && out_counts != nullptr) out_counts[map[i]] = counts[i];
+}
+
+void launch_scatter_topk(const uint64_t* keys, const float* dists, const uint32_t* counts, const uint32_t* map, uint32_t n,
+                         uint32_t k, uint64_t* out_keys, float* out_dists, uint32_t* out_counts, cudaStream_t stream) {
+    if (n == 0) return;
+    const uint64_t total = (uint64_t)n * k;
+    scatter_topk_kernel<<<(unsigned)((total + 255) / 256), 256, 0, stream>>>(keys, dists, counts, map, n, k, out_keys,
+                                                                            out_dists, out_counts);
+    g_kernel_launches += 1;
+}
+
 void launch_convert_rows(int storage, const float* in, uint32_t n_rows, uint32_t dim, uint8_t* out,
                          uint32_t row_bytes, float* sq, float* nrm, cudaStream_t stream) {
     if (n_rows == 0) return;

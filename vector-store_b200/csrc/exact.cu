@@ -110,6 +110,7 @@ struct K1Args {
     const uint64_t* keys;
     const uint32_t* allow;
     uint64_t allow_bits;
+    const uint32_t* allow_of_q;  // [nq] bitmap index per query (nullable: bitmap 0)
     uint32_t kp, n_splits, rows_per_split, n_slabs;
     uint64_t* part;
 };
@@ -234,7 +235,8 @@ __global__ void __launch_bounds__(K1_THREADS, 2) exact_candidates_kernel(K1Args 
                     if (a.deny != nullptr && bit_test(a.deny, n)) ok = false;
                     if (ok && a.allow != nullptr) {
                         const uint64_t rid = a.keys[n] & kRowMask48;
-                        ok = rid < a.allow_bits && bit_test(a.allow, (uint32_t)rid);
+                        ok = rid < a.allow_bits && bit_test(query_allow(a.allow, a.allow_bits, a.allow_of_q, q0 + row),
+                                                            (uint32_t)rid);
                     }
                     if (!ok) {
                         pending &= ~bit;
@@ -497,6 +499,7 @@ struct ScanArgs {
     const uint64_t* keys;
     const uint32_t* allow;
     uint64_t allow_bits;
+    const uint32_t* allow_of_q;  // [nq] bitmap index per query (nullable: bitmap 0)
     uint32_t kf, n_splits, rows_per_split;
     uint64_t* part;  // [nq][n_splits * SCAN_WARPS][kf]
 };
@@ -517,16 +520,30 @@ __global__ void __launch_bounds__(SCAN_WARPS * 32) exact_scan_kernel(ScanArgs a)
     float qn[SCAN_QB];
 #pragma unroll
     for (int j = 0; j < SCAN_QB; ++j) qn[j] = j < nv ? a.q_nrm[q0 + j] : 0.0f;
+    // word offset of each query's own bitmap (in shared memory: registers are what this kernel is short of)
+    __shared__ size_t q_allow_off[SCAN_QB];
+    if (threadIdx.x < SCAN_QB)
+        q_allow_off[threadIdx.x] = a.allow_of_q != nullptr && (int)threadIdx.x < nv
+                                       ? (size_t)a.allow_of_q[q0 + threadIdx.x] * (size_t)((a.allow_bits + 31) / 32) : 0;
+    __syncthreads();
 
     for (uint32_t r0 = lo + warp * 32; r0 < hi; r0 += 32 * SCAN_WARPS) {
         const uint32_t row = r0 + lane;
-        bool ok = row < hi;
-        if (ok && a.deny != nullptr && bit_test(a.deny, row)) ok = false;
-        if (ok && a.allow != nullptr) {
-            const uint64_t rid = a.keys[row] & kRowMask48;
-            ok = rid < a.allow_bits && bit_test(a.allow, (uint32_t)rid);
+        // bit j: the row is admissible for query j of the block; a row is evaluated if any query admits it
+        uint32_t adm = 0;
+        if (row < hi && !(a.deny != nullptr && bit_test(a.deny, row))) {
+            if (a.allow == nullptr) {
+                adm = (1u << nv) - 1;
+            } else {
+                const uint64_t rid = a.keys[row] & kRowMask48;
+                if (rid < a.allow_bits) {
+#pragma unroll
+                    for (int j = 0; j < SCAN_QB; ++j)
+                        if (j < nv && bit_test(a.allow + q_allow_off[j], (uint32_t)rid)) adm |= 1u << j;
+                }
+            }
         }
-        uint32_t mask = __ballot_sync(kFullMask, ok);
+        uint32_t mask = __ballot_sync(kFullMask, adm != 0);
         uint64_t res[SCAN_QB];
 #pragma unroll
         for (int j = 0; j < SCAN_QB; ++j) res[j] = kInvalidPacked;
@@ -565,8 +582,8 @@ __global__ void __launch_bounds__(SCAN_WARPS * 32) exact_scan_kernel(ScanArgs a)
                     }
                     const float d0 = finish_distance<ST, METRIC>(f0, i0, qn[j], xn0);
                     const float d1 = finish_distance<ST, METRIC>(f1, i1, qn[j], xn1);
-                    if (lane == c0) res[j] = pack_ds(d0, s0);
-                    if (lane == c1) res[j] = pack_ds(d1, s1);
+                    if (lane == c0 && (adm >> j & 1u)) res[j] = pack_ds(d0, s0);
+                    if (lane == c1 && (adm >> j & 1u)) res[j] = pack_ds(d1, s1);
                 }
             }
         }
@@ -661,7 +678,7 @@ void launch_exact_candidates(const ExactParams& p, cudaStream_t stream) {
     a.q_rows = p.q.rows; a.q_sq = p.q.sq; a.q_nrm = p.q.nrm; a.nq = p.q.n; a.q_row_bytes = p.q.row_bytes;
     a.x_rows = p.x.rows; a.x_sq = p.x.sq; a.x_nrm = p.x.nrm; a.x_row_bytes = p.x.row_bytes;
     a.x_lo = p.x_lo; a.x_hi = p.x_hi;
-    a.deny = p.deny; a.keys = p.keys; a.allow = p.allow; a.allow_bits = p.allow_bits;
+    a.deny = p.deny; a.keys = p.keys; a.allow = p.allow; a.allow_bits = p.allow_bits; a.allow_of_q = p.allow_of_q;
     a.kp = p.kp; a.n_splits = p.n_splits;
     const uint32_t rows = p.x_hi - p.x_lo;
     uint32_t rps = (rows + p.n_splits - 1) / p.n_splits;
@@ -693,7 +710,7 @@ void launch_exact_scan(const ExactParams& p, uint32_t k, cudaStream_t stream) {
     ScanArgs a;
     a.q_rows = p.q.rows; a.q_nrm = p.q.nrm; a.nq = p.q.n; a.q_row_bytes = p.q.row_bytes;
     a.x_rows = p.x.rows; a.x_nrm = p.x.nrm; a.x_row_bytes = p.x.row_bytes; a.x_lo = p.x_lo; a.x_hi = p.x_hi;
-    a.deny = p.deny; a.keys = p.keys; a.allow = p.allow; a.allow_bits = p.allow_bits;
+    a.deny = p.deny; a.keys = p.keys; a.allow = p.allow; a.allow_bits = p.allow_bits; a.allow_of_q = p.allow_of_q;
     a.kf = p.kp;  // the caller sets kp = round_up(k (+1 for self), 32): lists hold exactly what K3 needs
     (void)k;
     a.n_splits = p.n_splits;

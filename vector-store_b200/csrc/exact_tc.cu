@@ -70,6 +70,7 @@ struct TcArgs {
     const uint64_t* keys;
     const uint32_t* allow;
     uint64_t allow_bits;
+    const uint32_t* allow_of_q;  // [nq] bitmap index per query (nullable: bitmap 0)
     uint32_t kp, n_splits, rows_per_split;  // n_splits = lists per query = TC_HALVES * gridDim.y
     uint64_t* part;
     int tile_min;  // 1: emit only each tile's best row per query (seed layer), no list maintenance
@@ -456,7 +457,8 @@ __global__ void __launch_bounds__(TC_THREADS, 1)
         float thr = q_valid ? (a.thr_init != nullptr ? a.thr_init[q] : __int_as_float(0x7F800000)) : __int_as_float(0xFF800000);
         int cnt = 0;
         const uint32_t* deny = a.deny;
-        const uint32_t* allow = a.allow;
+        // this thread's query row is tested against its own bitmap
+        const uint32_t* allow = a.allow != nullptr && q_valid ? query_allow(a.allow, a.allow_bits, a.allow_of_q, q) : a.allow;
         const uint64_t* keys = a.keys;
         const uint64_t allow_bits = a.allow_bits;
 
@@ -785,7 +787,7 @@ bool launch_exact_candidates_tc(const ExactParams& p, cudaStream_t stream, bool 
     TcArgs a;
     a.q_sq = p.q.sq; a.q_nrm = p.q.nrm; a.nq = p.q.n;
     a.x_sq = p.x.sq; a.x_nrm = p.x.nrm; a.x_lo = p.x_lo; a.x_hi = p.x_hi; a.row_bytes = p.x.row_bytes;
-    a.deny = p.deny; a.keys = p.keys; a.allow = p.allow; a.allow_bits = p.allow_bits;
+    a.deny = p.deny; a.keys = p.keys; a.allow = p.allow; a.allow_bits = p.allow_bits; a.allow_of_q = p.allow_of_q;
     a.kp = p.kp; a.n_splits = p.n_splits;
     if (p.n_splits % TC_HALVES != 0) return false;  // callers size the lists with exact_tc_pick_splits
     const uint32_t row_splits = p.n_splits / TC_HALVES;

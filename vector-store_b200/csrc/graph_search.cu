@@ -85,6 +85,7 @@ void launch_graph_search(const SearchParams& p, cudaStream_t stream) {
     a.out_stride = p.out_stride ? p.out_stride : p.k;
     a.allow = p.allow;
     a.allow_bits = p.allow_bits;
+    a.allow_of_q = p.allow_of_q;
     a.rk = p.allow != nullptr ? ((p.k + 31) / 32) * 32 : 0;
     a.mma = 0;
     static const uint32_t compact_env = [] {

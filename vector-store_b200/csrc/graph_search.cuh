@@ -48,6 +48,7 @@ struct K4Args {
     unsigned long long* counters;
     const uint32_t* allow;  // filtered ANN: admissibility bitmap over (key & 2^48-1); only the FILTER instantiation reads it
     uint64_t allow_bits;
+    const uint32_t* allow_of_q;  // [nq] bitmap index per query (nullable: bitmap 0)
     uint32_t rk;            // length of the result list of the FILTER instantiation (k rounded up to 32)
     uint32_t mma;           // 1: 16-bit rows are evaluated on the tensor cores (mma.sync), distances are candidate-grade
     uint32_t compact;       // 1: survivors of an iteration are compacted before the sort + merge
@@ -336,8 +337,10 @@ __global__ void __launch_bounds__(K4_WARPS * 32, k4_min_blocks<ST, CPL, MMA>()) 
     float* newd = reinterpret_cast<float*>(newq + qcap);     // [qcap] their raw sums
     uint64_t* rlist = reinterpret_cast<uint64_t*>(newd + qcap);  // [rk] FILTER: best admissible rows seen so far
     uint64_t* stage = rlist + (FILTER ? a.rk : 0);               // [64] candidates of this iteration that can enter the list
+    const uint32_t* allow = nullptr;  // FILTER: this query's own bitmap
     if constexpr (FILTER) {
         for (uint32_t i = lane; i < a.rk; i += 32) rlist[i] = kInvalidPacked;
+        allow = query_allow(a.allow, a.allow_bits, a.allow_of_q, q);
     }
     const LessBySlot less;
     const bool is_l2 = a.metric == VSB_METRIC_L2SQ;
@@ -426,7 +429,7 @@ __global__ void __launch_bounds__(K4_WARPS * 32, k4_min_blocks<ST, CPL, MMA>()) 
                 uint64_t adm = kInvalidPacked;
                 if (res != kInvalidPacked) {
                     const uint64_t row_id = a.keys[packed_lo(res)] & kRowMask48;
-                    if (row_id < a.allow_bits && (a.allow[row_id >> 5] >> (row_id & 31) & 1u)) adm = res;
+                    if (row_id < a.allow_bits && (allow[row_id >> 5] >> (row_id & 31) & 1u)) adm = res;
                 }
                 if (__ballot_sync(kFullMask, adm < rlist[a.rk - 1]) != 0) {
                     adm = warp_sort32(adm, lane, less);

@@ -756,15 +756,15 @@ vsb_status vsb_get_options(vsb_index* ix, vsb_options* out) {
 vsb_status vsb_search(vsb_index* ix, const float* queries, uint64_t q, uint32_t k, uint64_t* keys, float* distances,
                       uint32_t* counts) {
     if (!ix) return fail(VSB_EINVAL, "null index");
-    if (ix->sharded) return vsbi::sharded_search_host(ix, queries, q, k, keys, distances, counts, false, nullptr, 0);
-    return ix->search_host(queries, q, k, keys, distances, counts, false, nullptr, 0);
+    if (ix->sharded) return vsbi::sharded_search_host(ix, queries, q, k, keys, distances, counts, false);
+    return ix->search_host(queries, q, k, keys, distances, counts, false);
 }
 
 vsb_status vsb_search_exact(vsb_index* ix, const float* queries, uint64_t q, uint32_t k, uint64_t* keys,
                             float* distances, uint32_t* counts) {
     if (!ix) return fail(VSB_EINVAL, "null index");
-    if (ix->sharded) return vsbi::sharded_search_host(ix, queries, q, k, keys, distances, counts, true, nullptr, 0);
-    return ix->search_host(queries, q, k, keys, distances, counts, true, nullptr, 0);
+    if (ix->sharded) return vsbi::sharded_search_host(ix, queries, q, k, keys, distances, counts, true);
+    return ix->search_host(queries, q, k, keys, distances, counts, true);
 }
 
 vsb_status vsb_search_filtered(vsb_index* ix, const float* queries, uint64_t q, uint32_t k,
@@ -772,9 +772,32 @@ vsb_status vsb_search_filtered(vsb_index* ix, const float* queries, uint64_t q, 
                                uint32_t* counts) {
     if (!ix) return fail(VSB_EINVAL, "null index");
     if (!allow_bitmap) return fail(VSB_EINVAL, "null bitmap");
-    if (ix->sharded)
-        return vsbi::sharded_search_host(ix, queries, q, k, keys, distances, counts, false, allow_bitmap, bitmap_bits);
-    return ix->search_host(queries, q, k, keys, distances, counts, false, allow_bitmap, bitmap_bits);
+    vsbi::HostFilters hf;
+    hf.bitmaps = allow_bitmap;
+    hf.n = 1;
+    hf.bits = bitmap_bits;
+    if (ix->sharded) return vsbi::sharded_search_host(ix, queries, q, k, keys, distances, counts, false, hf);
+    return ix->search_host(queries, q, k, keys, distances, counts, false, hf);
+}
+
+vsb_status vsb_search_filtered_multi(vsb_index* ix, const float* queries, uint64_t q, uint32_t k,
+                                     const uint32_t* allow_bitmaps, uint32_t n_filters, uint64_t bitmap_bits,
+                                     const uint32_t* filter_of_query, uint64_t* keys, float* distances, uint32_t* counts) {
+    if (!ix) return fail(VSB_EINVAL, "null index");
+    if (!queries || !allow_bitmaps || !filter_of_query || !keys || !distances) return fail(VSB_EINVAL, "null argument");
+    if (n_filters == 0 || n_filters > q)
+        return fail(VSB_EINVAL, "n_filters = %u must be in [1, q = %llu]", n_filters, (unsigned long long)q);
+    for (uint64_t i = 0; i < q; ++i)
+        if (filter_of_query[i] >= n_filters)
+            return fail(VSB_EINVAL, "filter_of_query[%llu] = %u >= n_filters = %u", (unsigned long long)i, filter_of_query[i],
+                        n_filters);
+    vsbi::HostFilters hf;
+    hf.bitmaps = allow_bitmaps;
+    hf.n = n_filters;
+    hf.bits = bitmap_bits;
+    hf.of_query = filter_of_query;
+    if (ix->sharded) return vsbi::sharded_search_host(ix, queries, q, k, keys, distances, counts, false, hf);
+    return ix->search_host(queries, q, k, keys, distances, counts, false, hf);
 }
 
 vsb_status vsb_search_dev(vsb_index* ix, const float* d_queries, uint64_t q, uint32_t k, uint64_t* d_keys,
@@ -783,8 +806,7 @@ vsb_status vsb_search_dev(vsb_index* ix, const float* d_queries, uint64_t q, uin
     if (ix->sharded)
         return vsbi::sharded_search_dev(ix, d_queries, q, k, d_keys, d_distances, d_counts, static_cast<cudaStream_t>(stream), exact != 0);
     std::lock_guard<std::mutex> g(ix->search_mu);
-    return ix->search_dev(d_queries, q, k, d_keys, d_distances, d_counts, static_cast<cudaStream_t>(stream), exact != 0,
-                          nullptr, 0, 0);
+    return ix->search_dev(d_queries, q, k, d_keys, d_distances, d_counts, static_cast<cudaStream_t>(stream), exact != 0);
 }
 
 vsb_status vsb_merge_topk_dev(const uint64_t* d_keys, const float* d_distances, uint32_t parts, uint64_t q, uint32_t k,

@@ -115,7 +115,7 @@ vsb_status vsb_index::build() {
                 shq.sq = shx.sq + b0;
                 shq.nrm = shx.nrm + b0;
             }
-            ST(exact_block(w, ms, q, x, 0, n, nullptr, st.keys.as<uint64_t>(), nullptr, 0, kin, nullptr, nullptr, nullptr,
+            ST(exact_block(w, ms, q, x, 0, n, nullptr, st.keys.as<uint64_t>(), nullptr, 0, nullptr, kin, nullptr, nullptr, nullptr,
                            knn.as<uint64_t>() + (size_t)b0 * kin, (int64_t)b0, mstream, true, use_shadow ? &shq : nullptr,
                            use_shadow ? &shx : nullptr));
         }

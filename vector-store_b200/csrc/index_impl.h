@@ -255,17 +255,39 @@ struct View {
 struct Scratch {
     DevBuf q_in, q_rows, q_sq, q_nrm, q16_rows, q16_sq, q16_nrm, q8_rows, q8_sq, q8_nrm;
     DevBuf part, seed_part, tmp_keys, tmp_dists, rr_packed, counters, allow;
-    DevBuf cert_state, fb_map, fb_rows, fb_sq, fb_nrm;  // certified exact search
+    DevBuf cert_state, fb_map, fb_rows, fb_sq, fb_nrm, fb_fidx;  // certified exact search
+    // filtered searches whose bitmaps take different routes: each route's queries, bitmap indices and results
+    DevBuf rt_map, rt_rows, rt_sq, rt_nrm, rt_fidx, rt_keys, rt_dists, rt_counts;
     DevBuf thr_part, thr, thr_cnt;                       // sampled list bounds of the all-pairs build (exact_block)
     PinBuf pin;                                          // pinned staging of this caller class's read-backs
     size_t bytes() const {
         const DevBuf* all[] = {&q_in, &q_rows, &q_sq, &q_nrm, &q16_rows, &q16_sq, &q16_nrm, &q8_rows, &q8_sq, &q8_nrm, &part,
                                &seed_part, &tmp_keys, &tmp_dists, &rr_packed, &counters, &allow, &cert_state, &fb_map,
-                               &fb_rows, &fb_sq, &fb_nrm, &thr_part, &thr, &thr_cnt};
+                               &fb_rows, &fb_sq, &fb_nrm, &fb_fidx, &rt_map, &rt_rows, &rt_sq, &rt_nrm, &rt_fidx,
+                               &rt_keys, &rt_dists, &rt_counts, &thr_part, &thr, &thr_cnt};
         size_t s = 0;
         for (auto* b : all) s += b->bytes;
         return s;
     }
+};
+
+// A filtered call as the caller hands it over: n bitmaps over (key & 2^48-1) back to back in host memory,
+// ceil(bits / 32) words each; query i is filtered by bitmap of_query[i] (null: bitmap 0 for every query).
+struct HostFilters {
+    const uint32_t* bitmaps = nullptr;  // null: unfiltered search
+    uint32_t n = 0;
+    uint64_t bits = 0;
+    const uint32_t* of_query = nullptr;
+};
+
+// The same call once the bitmaps are on the device: what search_dev needs to route and run it.
+struct Filters {
+    const uint32_t* d_allow = nullptr;  // [n][ceil(bits / 32)] (null: unfiltered search)
+    uint64_t bits = 0;
+    uint32_t n = 0;
+    const uint32_t* d_fidx = nullptr;  // [nq] bitmap index per query (null: bitmap 0 for every query)
+    const uint32_t* h_fidx = nullptr;  // host copy of d_fidx (route selection); null exactly when d_fidx is
+    const uint64_t* pop = nullptr;     // host [n]: admissible rows per bitmap (route selection)
 };
 
 struct Sharded;  // sharded.cu: the multi-device router behind the same handle type
@@ -393,7 +415,8 @@ struct vsb_index {
     // search building blocks: run on stream `s` with scratch `sc` against view `v`
     vsb_status exact_block(const vsbi::View& v, vsbi::Scratch& sc, const vsb::RowsView& q, const vsb::RowsView& x,
                            uint32_t x_lo, uint32_t x_hi, const uint32_t* deny_bm, const uint64_t* key_arr,
-                           const uint32_t* allow_bm, uint64_t allow_bits, uint32_t k, uint64_t* out_keys,
+                           const uint32_t* allow_bm, uint64_t allow_bits, const uint32_t* allow_of_q, uint32_t k,
+                           uint64_t* out_keys,
                            float* out_dists, uint32_t* out_counts, uint64_t* out_packed, int64_t self_base,
                            cudaStream_t s, bool approx_ok, const vsb::RowsView* shadow_q = nullptr,
                            const vsb::RowsView* shadow_x = nullptr);
@@ -403,16 +426,21 @@ struct vsb_index {
         bool native = false; // ignore the traversal copies
         const uint32_t* allow = nullptr;  // filtered ANN: bitmap over (key & 2^48-1)
         uint64_t allow_bits = 0;
+        const uint32_t* allow_of_q = nullptr;  // [nb] bitmap index per query (null: bitmap 0)
     };
     vsb_status graph_block(const vsbi::View& v, vsbi::Scratch& sc, const GraphRun& run, const vsb::RowsView& qv,
                            uint32_t nb, uint32_t k, uint64_t* g_keys, float* g_dists, uint32_t* counts_out,
                            uint64_t* packed_out, const vsb::RowsView* q16_in, cudaStream_t s, long long self_base,
                            bool timed_phases, uint64_t* evals_out = nullptr, uint64_t* parents_out = nullptr);
+    // one chunk of converted queries on one route: the graph (with the brute-force tail and the K8 merge) or the
+    // exact scan; allow_bm != null filters it (per query through allow_of_q)
+    vsb_status search_block(const vsbi::View& v, vsbi::Scratch& sc, const vsb::RowsView& qv, uint32_t nb, uint32_t k,
+                            uint64_t* o_keys, float* o_dists, uint32_t* o_counts, cudaStream_t s, bool graph,
+                            const uint32_t* allow_bm, uint64_t allow_bits, const uint32_t* allow_of_q);
     vsb_status search_dev(const float* d_q, uint64_t nq, uint32_t k, uint64_t* d_keys, float* d_dists,
-                          uint32_t* d_counts, cudaStream_t s, bool exact, const uint32_t* d_allow,
-                          uint64_t allow_bits, uint64_t allow_popcount);
+                          uint32_t* d_counts, cudaStream_t s, bool exact, const vsbi::Filters& f = vsbi::Filters());
     vsb_status search_host(const float* queries, uint64_t nq, uint32_t k, uint64_t* keys_out, float* dists_out,
-                           uint32_t* counts_out, bool exact, const uint32_t* allow_bitmap, uint64_t allow_bits);
+                           uint32_t* counts_out, bool exact, const vsbi::HostFilters& hf = vsbi::HostFilters());
 };
 
 namespace vsbi {

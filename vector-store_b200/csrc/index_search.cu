@@ -17,7 +17,7 @@ using vsbi::View;
 // exact top-k of the queries `q` against rows [x_lo, x_hi) of `x` (K1 + K3)
 vsb_status vsb_index::exact_block(const View& v, Scratch& sc, const vsb::RowsView& q, const vsb::RowsView& x, uint32_t x_lo,
                                   uint32_t x_hi, const uint32_t* deny_bm, const uint64_t* key_arr, const uint32_t* allow_bm,
-                                  uint64_t allow_bits, uint32_t k, uint64_t* out_keys, float* out_dists,
+                                  uint64_t allow_bits, const uint32_t* allow_of_q, uint32_t k, uint64_t* out_keys, float* out_dists,
                                   uint32_t* out_counts, uint64_t* out_packed, int64_t self_base, cudaStream_t s,
                                   bool approx_ok, const vsb::RowsView* shadow_q, const vsb::RowsView* shadow_x) {
     (void)v;
@@ -32,6 +32,7 @@ vsb_status vsb_index::exact_block(const View& v, Scratch& sc, const vsb::RowsVie
     p.keys = key_arr;
     p.allow = allow_bm;
     p.allow_bits = allow_bits;
+    p.allow_of_q = allow_of_q;
     const uint32_t extra = std::max<uint32_t>(16, k / 4) + (self_base >= 0 ? 1 : 0);
     p.kp = round_up(k + extra, 32);
     if (p.kp > 256) return fail(VSB_EINVAL, "k=%u too large for the exact path (max 200)", k);
@@ -136,7 +137,8 @@ vsb_status vsb_index::exact_block(const View& v, Scratch& sc, const vsb::RowsVie
     cert.sum = (float)dim * 0x1p-23f;
     cert.rel = (tc && storage == VSB_F32) ? rel_tf32 : rel_fp32;
 
-    // flagged queries of one stage -> compact map (indices into the caller's query block) + gathered rows
+    // flagged queries of one stage -> compact map (indices into the caller's query block) + gathered rows, and the
+    // gathered bitmap index of each query (a filtered call whose queries carry their own bitmaps)
     std::vector<uint32_t> map, flags;
     auto collect = [&](uint32_t n_stage, const std::vector<uint32_t>* prev) -> vsb_status {
         flags.resize(n_stage);
@@ -158,6 +160,10 @@ vsb_status vsb_index::exact_block(const View& v, Scratch& sc, const vsb::RowsVie
         CU(cudaMemcpyAsync(sc.fb_map.p, map.data(), (size_t)nf * 4, cudaMemcpyHostToDevice, s));
         vsb::launch_gather_rows(q.rows, q.row_bytes, q.sq, q.nrm, sc.fb_map.as<uint32_t>(), nf, sc.fb_rows.as<uint8_t>(),
                                 sc.fb_sq.as<float>(), sc.fb_nrm.as<float>(), s);
+        if (allow_of_q != nullptr) {
+            CU(sc.fb_fidx.ensure((size_t)nf * 4));
+            vsb::launch_gather_u32(allow_of_q, sc.fb_map.as<uint32_t>(), nf, sc.fb_fidx.as<uint32_t>(), s);
+        }
         CU(cudaStreamSynchronize(s));  // `map` is pageable and is rebuilt by the next stage
         return VSB_OK;
     };
@@ -184,6 +190,7 @@ vsb_status vsb_index::exact_block(const View& v, Scratch& sc, const vsb::RowsVie
     pf.q.sq = sc.fb_sq.as<float>();
     pf.q.nrm = sc.fb_nrm.as<float>();
     pf.q.n = (uint32_t)map.size();
+    if (allow_of_q != nullptr) pf.allow_of_q = sc.fb_fidx.as<uint32_t>();
     if (tc && storage == VSB_F32) {
         // second stage: full fp32 products on the SIMT tiles, same certificate with the fp32 bound
         pf.kp = kp_simt;
@@ -366,6 +373,7 @@ vsb_status vsb_index::graph_block(const View& v, Scratch& sc, const GraphRun& ru
     gp.self_base = self_base;
     gp.allow = run.allow;
     gp.allow_bits = run.allow_bits;
+    gp.allow_of_q = run.allow_of_q;
     gp.mma = mma;
     uint32_t kr = 0;
     if (packed_out != nullptr) {
@@ -431,10 +439,78 @@ vsb_status vsb_index::graph_block(const View& v, Scratch& sc, const GraphRun& ru
     return VSB_OK;
 }
 
+vsb_status vsb_index::search_block(const View& v, Scratch& sc, const vsb::RowsView& qv, uint32_t nb, uint32_t k,
+                                    uint64_t* o_keys, float* o_dists, uint32_t* o_counts, cudaStream_t s, bool graph,
+                                    const uint32_t* allow_bm, uint64_t allow_bits, const uint32_t* allow_of_q) {
+    const vsbi::Store& st = *v.st;
+    const vsb::RowsView x = rows_view(v);
+    const uint32_t* deny_bm = v.any_tombstone ? st.deny.as<uint32_t>() : nullptr;
+    const bool use_graph = graph && v.n_graphed > 0 && k <= 1024;
+    const uint32_t tail_lo = use_graph ? v.n_graphed : 0, tail_hi = v.n_slots;
+    const bool have_tail = tail_hi > tail_lo;
+    // the brute-force tail contributes at most its 200 best rows to an ANN answer (list length of K1)
+    const uint32_t k_tail = use_graph ? std::min<uint32_t>(k, 200) : k;
+    uint64_t* g_keys = o_keys;
+    float* g_dists = o_dists;
+    uint64_t* t_keys = o_keys;
+    float* t_dists = o_dists;
+    if (use_graph && have_tail) {
+        CU(sc.tmp_keys.ensure((size_t)2 * nb * k * 8));
+        CU(sc.tmp_dists.ensure((size_t)2 * nb * k * 4));
+        g_keys = sc.tmp_keys.as<uint64_t>();
+        g_dists = sc.tmp_dists.as<float>();
+        t_keys = g_keys + (size_t)nb * k;
+        t_dists = g_dists + (size_t)nb * k;
+    }
+    if (use_graph) {
+        GraphRun run;
+        run.itopk = itopk;
+        run.max_iters = max_iters;
+        run.n_seeds = n_seeds;
+        run.search_width = search_width;
+        run.count = instrumented;
+        run.native = native_traversal;
+        run.allow = allow_bm;
+        run.allow_bits = allow_bits;
+        run.allow_of_q = allow_of_q;
+        ST(graph_block(v, sc, run, qv, nb, k, g_keys, g_dists, have_tail ? nullptr : o_counts, nullptr, nullptr, s, -1, true));
+    }
+    if (have_tail) {
+        t_begin(PH_EXACT, s);
+        vsb_status est;
+        if (k_tail == k) {
+            est = exact_block(v, sc, qv, x, tail_lo, tail_hi, deny_bm, st.keys.as<uint64_t>(), allow_bm, allow_bits, allow_of_q,
+                              k, t_keys, t_dists, use_graph ? nullptr : o_counts, nullptr, -1, s,
+                              /*approx_ok=*/use_graph);  // the ANN tail needs no certificate (no host sync)
+        } else {
+            // k > 200 with a tail: the tail's best 200 rows, laid out with stride k so that K8 can merge them
+            vsb::launch_fill_empty(t_keys, t_dists, nullptr, nb, k, s);
+            vsbi::DevBuf& tk = sc.fb_rows;  // scratch that the ANN path does not otherwise touch
+            CU(tk.ensure((size_t)nb * k_tail * 12));
+            uint64_t* ck = tk.as<uint64_t>();
+            float* cd = reinterpret_cast<float*>(ck + (size_t)nb * k_tail);
+            est = exact_block(v, sc, qv, x, tail_lo, tail_hi, deny_bm, st.keys.as<uint64_t>(), allow_bm, allow_bits, allow_of_q,
+                              k_tail, ck, cd, nullptr, nullptr, -1, s, true);
+            if (est == VSB_OK) {
+                CU(cudaMemcpy2DAsync(t_keys, (size_t)k * 8, ck, (size_t)k_tail * 8, (size_t)k_tail * 8, nb, cudaMemcpyDeviceToDevice, s));
+                CU(cudaMemcpy2DAsync(t_dists, (size_t)k * 4, cd, (size_t)k_tail * 4, (size_t)k_tail * 4, nb, cudaMemcpyDeviceToDevice, s));
+            }
+        }
+        t_end(s);
+        ST(est);
+    }
+    if (use_graph && have_tail) {
+        t_begin(PH_MERGE, s);
+        vsb::launch_merge_topk(g_keys, g_dists, 2, nb, k, o_keys, o_dists, o_counts, s);
+        t_end(s);
+        CU(cudaGetLastError());
+    }
+    return VSB_OK;
+}
+
 // search_mu held by the caller
 vsb_status vsb_index::search_dev(const float* d_q, uint64_t nq, uint32_t k, uint64_t* d_keys, float* d_dists,
-                                 uint32_t* d_counts, cudaStream_t s, bool exact, const uint32_t* d_allow,
-                                 uint64_t allow_bits, uint64_t allow_popcount) {
+                                 uint32_t* d_counts, cudaStream_t s, bool exact, const vsbi::Filters& f) {
     if (nq == 0) return VSB_OK;
     if (k == 0) return fail(VSB_EINVAL, "k must be > 0");
     if (d_q == nullptr || d_keys == nullptr || d_dists == nullptr) return fail(VSB_EINVAL, "null buffer");
@@ -444,11 +520,13 @@ vsb_status vsb_index::search_dev(const float* d_q, uint64_t nq, uint32_t k, uint
     const View v = snapshot();
     ST(begin_search(s));
     Scratch& sc = ss;
-    // filtered search: graph traversal with the bitmap unless too few rows are admissible (then the exact scan wins)
-    bool filtered_graph = false;
-    if (d_allow != nullptr && !exact && v.n_graphed > 0 && k <= 256) {
+    // filtered search, per bitmap: graph traversal with the bitmap unless too few rows are admissible (then the exact
+    // scan wins).  Queries whose bitmaps take different routes are split by route below.
+    std::vector<uint8_t> graph_of_filter(f.d_allow != nullptr ? f.n : 0, 0);
+    if (f.d_allow != nullptr && !exact && v.n_graphed > 0 && k <= 256) {
         const uint64_t live_rows = live_atomic.load();
-        filtered_graph = allow_popcount * 100 >= (uint64_t)filter_min_pct * std::max<uint64_t>(live_rows, 1) && filter_min_pct <= 100;
+        for (uint32_t i = 0; i < f.n; ++i)
+            graph_of_filter[i] = f.pop[i] * 100 >= (uint64_t)filter_min_pct * std::max<uint64_t>(live_rows, 1) && filter_min_pct <= 100;
     }
     const uint64_t QCHUNK = 65536;
     for (uint64_t q0 = 0; q0 < nq; q0 += QCHUNK) {
@@ -461,7 +539,6 @@ vsb_status vsb_index::search_dev(const float* d_q, uint64_t nq, uint32_t k, uint
             CU(cudaGetLastError());
             continue;
         }
-        const vsbi::Store& st = *v.st;
         CU(sc.q_rows.ensure((size_t)nb * row_bytes));
         CU(sc.q_sq.ensure((size_t)nb * 4));
         CU(sc.q_nrm.ensure((size_t)nb * 4));
@@ -476,67 +553,51 @@ vsb_status vsb_index::search_dev(const float* d_q, uint64_t nq, uint32_t k, uint
         qv.nrm = sc.q_nrm.as<float>();
         qv.row_bytes = row_bytes;
         qv.n = nb;
-        const vsb::RowsView x = rows_view(v);
-        const uint32_t* deny_bm = v.any_tombstone ? st.deny.as<uint32_t>() : nullptr;
-        const bool use_graph = !exact && (d_allow == nullptr || filtered_graph) && v.n_graphed > 0 && k <= 1024;
-        const uint32_t tail_lo = use_graph ? v.n_graphed : 0, tail_hi = v.n_slots;
-        const bool have_tail = tail_hi > tail_lo;
-        // the brute-force tail contributes at most its 200 best rows to an ANN answer (list length of K1)
-        const uint32_t k_tail = use_graph ? std::min<uint32_t>(k, 200) : k;
-        uint64_t* g_keys = o_keys;
-        float* g_dists = o_dists;
-        uint64_t* t_keys = o_keys;
-        float* t_dists = o_dists;
-        if (use_graph && have_tail) {
-            CU(sc.tmp_keys.ensure((size_t)2 * nb * k * 8));
-            CU(sc.tmp_dists.ensure((size_t)2 * nb * k * 4));
-            g_keys = sc.tmp_keys.as<uint64_t>();
-            g_dists = sc.tmp_dists.as<float>();
-            t_keys = g_keys + (size_t)nb * k;
-            t_dists = g_dists + (size_t)nb * k;
+        if (f.d_allow == nullptr) {
+            ST(search_block(v, sc, qv, nb, k, o_keys, o_dists, o_counts, s, !exact, nullptr, 0, nullptr));
+            continue;
         }
-        if (use_graph) {
-            GraphRun run;
-            run.itopk = itopk;
-            run.max_iters = max_iters;
-            run.n_seeds = n_seeds;
-            run.search_width = search_width;
-            run.count = instrumented;
-            run.native = native_traversal;
-            if (filtered_graph) {
-                run.allow = d_allow;
-                run.allow_bits = allow_bits;
+        const uint32_t* c_fidx = f.d_fidx ? f.d_fidx + q0 : nullptr;  // this chunk's bitmap indices
+        // route of each query of the chunk: by_route[1] = graph, by_route[0] = exact scan
+        std::vector<uint32_t> by_route[2];
+        for (uint32_t i = 0; i < nb; ++i) by_route[graph_of_filter[f.h_fidx ? f.h_fidx[q0 + i] : 0]].push_back(i);
+        if (by_route[0].empty() || by_route[1].empty()) {
+            ST(search_block(v, sc, qv, nb, k, o_keys, o_dists, o_counts, s, by_route[0].empty(), f.d_allow, f.bits, c_fidx));
+            continue;
+        }
+        // mixed routes: each route runs on a compact block of its own queries (rows and bitmap indices gathered like
+        // the certificate fallback's), and its [n][k] results are scattered back to the caller's rows
+        const uint32_t n_max = (uint32_t)std::max(by_route[0].size(), by_route[1].size());
+        CU(sc.rt_map.ensure((size_t)nb * 4));
+        CU(sc.rt_rows.ensure((size_t)n_max * row_bytes));
+        CU(sc.rt_sq.ensure((size_t)n_max * 4));
+        CU(sc.rt_nrm.ensure((size_t)n_max * 4));
+        CU(sc.rt_fidx.ensure((size_t)n_max * 4));
+        CU(sc.rt_keys.ensure((size_t)n_max * k * 8));
+        CU(sc.rt_dists.ensure((size_t)n_max * k * 4));
+        CU(sc.rt_counts.ensure((size_t)n_max * 4));
+        uint32_t* d_map[2] = {sc.rt_map.as<uint32_t>(), sc.rt_map.as<uint32_t>() + by_route[0].size()};
+        CU(cudaMemcpyAsync(d_map[0], by_route[0].data(), by_route[0].size() * 4, cudaMemcpyHostToDevice, s));
+        CU(cudaMemcpyAsync(d_map[1], by_route[1].data(), by_route[1].size() * 4, cudaMemcpyHostToDevice, s));
+        for (int r = 1; r >= 0; --r) {
+            const uint32_t n = (uint32_t)by_route[r].size();
+            vsb::launch_gather_rows(qv.rows, row_bytes, qv.sq, qv.nrm, d_map[r], n, sc.rt_rows.as<uint8_t>(),
+                                    sc.rt_sq.as<float>(), sc.rt_nrm.as<float>(), s);
+            const uint32_t* r_fidx = nullptr;
+            if (c_fidx != nullptr) {
+                vsb::launch_gather_u32(c_fidx, d_map[r], n, sc.rt_fidx.as<uint32_t>(), s);
+                r_fidx = sc.rt_fidx.as<uint32_t>();
             }
-            ST(graph_block(v, sc, run, qv, nb, k, g_keys, g_dists, have_tail ? nullptr : o_counts, nullptr, nullptr, s, -1, true));
-        }
-        if (have_tail) {
-            t_begin(PH_EXACT, s);
-            vsb_status est;
-            if (k_tail == k) {
-                est = exact_block(v, sc, qv, x, tail_lo, tail_hi, deny_bm, st.keys.as<uint64_t>(), d_allow, allow_bits, k, t_keys,
-                                  t_dists, use_graph ? nullptr : o_counts, nullptr, -1, s,
-                                  /*approx_ok=*/use_graph);  // the ANN tail needs no certificate (no host sync)
-            } else {
-                // k > 200 with a tail: the tail's best 200 rows, laid out with stride k so that K8 can merge them
-                vsb::launch_fill_empty(t_keys, t_dists, nullptr, nb, k, s);
-                vsbi::DevBuf& tk = sc.fb_rows;  // scratch that the ANN path does not otherwise touch
-                CU(tk.ensure((size_t)nb * k_tail * 12));
-                uint64_t* ck = tk.as<uint64_t>();
-                float* cd = reinterpret_cast<float*>(ck + (size_t)nb * k_tail);
-                est = exact_block(v, sc, qv, x, tail_lo, tail_hi, deny_bm, st.keys.as<uint64_t>(), d_allow, allow_bits, k_tail, ck,
-                                  cd, nullptr, nullptr, -1, s, true);
-                if (est == VSB_OK) {
-                    CU(cudaMemcpy2DAsync(t_keys, (size_t)k * 8, ck, (size_t)k_tail * 8, (size_t)k_tail * 8, nb, cudaMemcpyDeviceToDevice, s));
-                    CU(cudaMemcpy2DAsync(t_dists, (size_t)k * 4, cd, (size_t)k_tail * 4, (size_t)k_tail * 4, nb, cudaMemcpyDeviceToDevice, s));
-                }
-            }
-            t_end(s);
-            ST(est);
-        }
-        if (use_graph && have_tail) {
-            t_begin(PH_MERGE, s);
-            vsb::launch_merge_topk(g_keys, g_dists, 2, nb, k, o_keys, o_dists, o_counts, s);
-            t_end(s);
+            CU(cudaGetLastError());
+            vsb::RowsView rv = qv;
+            rv.rows = sc.rt_rows.as<uint8_t>();
+            rv.sq = sc.rt_sq.as<float>();
+            rv.nrm = sc.rt_nrm.as<float>();
+            rv.n = n;
+            ST(search_block(v, sc, rv, n, k, sc.rt_keys.as<uint64_t>(), sc.rt_dists.as<float>(), sc.rt_counts.as<uint32_t>(),
+                            s, r == 1, f.d_allow, f.bits, r_fidx));
+            vsb::launch_scatter_topk(sc.rt_keys.as<uint64_t>(), sc.rt_dists.as<float>(), sc.rt_counts.as<uint32_t>(), d_map[r],
+                                     n, k, o_keys, o_dists, o_counts, s);
             CU(cudaGetLastError());
         }
     }
@@ -544,8 +605,6 @@ vsb_status vsb_index::search_dev(const float* d_q, uint64_t nq, uint32_t k, uint
     return VSB_OK;
 }
 
-static uint64_t popcount_words(const uint32_t* w, size_t n_words, uint64_t bits);
-// (defined below search_host's slot path, which needs it)
 static uint64_t popcount_words(const uint32_t* w, size_t n_words, uint64_t bits) {
     uint64_t c = 0;
     const size_t full = (size_t)(bits / 32);
@@ -554,15 +613,36 @@ static uint64_t popcount_words(const uint32_t* w, size_t n_words, uint64_t bits)
     return c;
 }
 
+// Uploads the bitmaps of a filtered call (one copy of the whole block) on `s`, points `f` at them and counts each
+// bitmap's admissible rows for the route selection; the per-query indices are the caller's to upload (d_fidx).
+static vsb_status upload_filters(vsbi::Scratch& sc, const vsbi::HostFilters& hf, cudaStream_t s, std::vector<uint64_t>& pop,
+                                 vsbi::Filters& f) {
+    if (hf.bitmaps == nullptr) return VSB_OK;
+    const size_t words = (size_t)((hf.bits + 31) / 32);
+    CU(sc.allow.ensure(std::max<size_t>((size_t)hf.n * words * 4, 16)));
+    CU(cudaMemcpyAsync(sc.allow.p, hf.bitmaps, (size_t)hf.n * words * 4, cudaMemcpyHostToDevice, s));
+    pop.resize(hf.n);
+    for (uint32_t i = 0; i < hf.n; ++i) pop[i] = popcount_words(hf.bitmaps + (size_t)i * words, words, hf.bits);
+    f.d_allow = sc.allow.as<uint32_t>();
+    f.bits = hf.bits;
+    f.n = hf.n;
+    f.h_fidx = hf.of_query;
+    f.pop = pop.data();
+    return VSB_OK;
+}
+
 vsb_status vsb_index::search_host(const float* queries, uint64_t nq, uint32_t k, uint64_t* keys_out,
-                                  float* dists_out, uint32_t* counts_out, bool exact, const uint32_t* allow_bitmap,
-                                  uint64_t allow_bits) {
+                                  float* dists_out, uint32_t* counts_out, bool exact, const vsbi::HostFilters& hf) {
     if (nq == 0) return VSB_OK;
     if (k == 0) return fail(VSB_EINVAL, "k must be > 0");
     if (queries == nullptr || keys_out == nullptr || dists_out == nullptr) return fail(VSB_EINVAL, "null buffer");
     const size_t in_bytes = (size_t)nq * dim * 4;
     const size_t keys_bytes = (size_t)nq * k * 8, dists_bytes = (size_t)nq * k * 4, counts_bytes = (size_t)nq * 4;
+    // per-query bitmap indices travel with the queries
+    const size_t fidx_bytes = hf.of_query != nullptr ? (size_t)nq * 4 : 0;
     auto al = [](size_t v) { return (v + 255) / 256 * 256; };
+    std::vector<uint64_t> pop;
+    vsbi::Filters f;
     if (nq >= 1024) {
         // Large batches are PIPELINED across concurrent callers (the reference serves ann requests from a worker
         // pool, worker.rs:44-118): each call takes one of two staging slots, uploads its queries on the slot's copy
@@ -591,27 +671,22 @@ vsb_status vsb_index::search_host(const float* queries, uint64_t nq, uint32_t k,
             CU(cudaEventCreateWithFlags(&sl.ev_in, cudaEventDisableTiming));
             CU(cudaEventCreateWithFlags(&sl.ev_done, cudaEventDisableTiming));
         }
-        CU(sl.buf.ensure(al(in_bytes) + al(keys_bytes) + al(dists_bytes) + al(counts_bytes)));
+        CU(sl.buf.ensure(al(in_bytes) + al(keys_bytes) + al(dists_bytes) + al(counts_bytes) + al(fidx_bytes)));
         uint8_t* base = sl.buf.as<uint8_t>();
         float* dq = reinterpret_cast<float*>(base);
         uint64_t* dk = reinterpret_cast<uint64_t*>(base + al(in_bytes));
         float* dd = reinterpret_cast<float*>(base + al(in_bytes) + al(keys_bytes));
         uint32_t* dc = reinterpret_cast<uint32_t*>(base + al(in_bytes) + al(keys_bytes) + al(dists_bytes));
+        uint32_t* dfi = reinterpret_cast<uint32_t*>(base + al(in_bytes) + al(keys_bytes) + al(dists_bytes) + al(counts_bytes));
         CU(cudaMemcpyAsync(dq, queries, in_bytes, cudaMemcpyHostToDevice, sl.cs));
+        if (fidx_bytes) CU(cudaMemcpyAsync(dfi, hf.of_query, fidx_bytes, cudaMemcpyHostToDevice, sl.cs));
         CU(cudaEventRecord(sl.ev_in, sl.cs));
         {
             std::lock_guard<std::mutex> g(search_mu);
-            const uint32_t* d_allow = nullptr;
-            uint64_t allow_pop = 0;
-            if (allow_bitmap != nullptr) {
-                const size_t words = (size_t)((allow_bits + 31) / 32);
-                CU(ss.allow.ensure(std::max<size_t>(words * 4, 16)));
-                CU(cudaMemcpyAsync(ss.allow.p, allow_bitmap, words * 4, cudaMemcpyHostToDevice, stream));
-                d_allow = ss.allow.as<uint32_t>();
-                allow_pop = popcount_words(allow_bitmap, words, allow_bits);
-            }
+            ST(upload_filters(ss, hf, stream, pop, f));
+            if (fidx_bytes) f.d_fidx = dfi;
             CU(cudaStreamWaitEvent(stream, sl.ev_in, 0));
-            ST(search_dev(dq, nq, k, dk, dd, dc, stream, exact, d_allow, allow_bits, allow_pop));
+            ST(search_dev(dq, nq, k, dk, dd, dc, stream, exact, f));
             CU(cudaEventRecord(sl.ev_done, stream));
         }
         CU(cudaStreamWaitEvent(sl.cs, sl.ev_done, 0));
@@ -628,23 +703,20 @@ vsb_status vsb_index::search_host(const float* queries, uint64_t nq, uint32_t k,
     CU(cudaSetDevice(device));
     ST(begin_search(stream));
     vsbi::DevBuf& d_in = ss.q_in;
-    CU(d_in.ensure(al(in_bytes) + al(keys_bytes) + al(dists_bytes) + al(counts_bytes)));
+    CU(d_in.ensure(al(in_bytes) + al(keys_bytes) + al(dists_bytes) + al(counts_bytes) + al(fidx_bytes)));
     uint8_t* base = d_in.as<uint8_t>();
     float* dq = reinterpret_cast<float*>(base);
     uint64_t* dk = reinterpret_cast<uint64_t*>(base + al(in_bytes));
     float* dd = reinterpret_cast<float*>(base + al(in_bytes) + al(keys_bytes));
     uint32_t* dc = reinterpret_cast<uint32_t*>(base + al(in_bytes) + al(keys_bytes) + al(dists_bytes));
+    uint32_t* dfi = reinterpret_cast<uint32_t*>(base + al(in_bytes) + al(keys_bytes) + al(dists_bytes) + al(counts_bytes));
     CU(cudaMemcpyAsync(dq, queries, in_bytes, cudaMemcpyHostToDevice, stream));
-    const uint32_t* d_allow = nullptr;
-    uint64_t allow_pop = 0;
-    if (allow_bitmap != nullptr) {
-        const size_t words = (size_t)((allow_bits + 31) / 32);
-        CU(ss.allow.ensure(std::max<size_t>(words * 4, 16)));
-        CU(cudaMemcpyAsync(ss.allow.p, allow_bitmap, words * 4, cudaMemcpyHostToDevice, stream));
-        d_allow = ss.allow.as<uint32_t>();
-        allow_pop = popcount_words(allow_bitmap, words, allow_bits);
+    if (fidx_bytes) {
+        CU(cudaMemcpyAsync(dfi, hf.of_query, fidx_bytes, cudaMemcpyHostToDevice, stream));
+        f.d_fidx = dfi;
     }
-    ST(search_dev(dq, nq, k, dk, dd, dc, stream, exact, d_allow, allow_bits, allow_pop));
+    ST(upload_filters(ss, hf, stream, pop, f));
+    ST(search_dev(dq, nq, k, dk, dd, dc, stream, exact, f));
     vsbi::HostReadback rb(ss.pin, stream);
     CU(rb.reserve(al(keys_bytes) + al(dists_bytes) + al(counts_bytes)));
     CU(rb.copy(keys_out, dk, keys_bytes));

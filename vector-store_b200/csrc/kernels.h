@@ -30,6 +30,10 @@ void launch_gather_rows(const uint8_t* rows, uint32_t row_bytes, const float* sq
                         cudaStream_t stream);
 
 void launch_gather_u64(const uint64_t* in, const uint32_t* slots, uint32_t n, uint64_t* out, cudaStream_t stream);
+void launch_gather_u32(const uint32_t* in, const uint32_t* slots, uint32_t n, uint32_t* out, cudaStream_t stream);
+// result row i of [n][k] (keys, dists, counts) goes to row map[i] of the output (counts / out_counts nullable)
+void launch_scatter_topk(const uint64_t* keys, const float* dists, const uint32_t* counts, const uint32_t* map, uint32_t n,
+                         uint32_t k, uint64_t* out_keys, float* out_dists, uint32_t* out_counts, cudaStream_t stream);
 
 // K1 + K3 (exact.cu) ----------------------------------------------------------------------------
 struct ExactParams {
@@ -41,6 +45,9 @@ struct ExactParams {
     const uint64_t* keys = nullptr;   // u64 key per row of x (tie-break + output)
     const uint32_t* allow = nullptr;  // N1: bitmap over (key & 2^48-1) (nullable)
     uint64_t allow_bits = 0;
+    // [q.n] index of each query's bitmap: query i tests allow + allow_of_q[i] * ceil(allow_bits / 32)
+    // (nullable: every query uses the first bitmap)
+    const uint32_t* allow_of_q = nullptr;
     uint32_t kp = 32;                 // candidate list length, multiple of 32, <= 256
     uint32_t n_splits = 1;
     uint64_t* part = nullptr;         // scratch [q.n][n_splits][kp]
@@ -149,6 +156,7 @@ struct SearchParams {
     // result list (a second list next to the traversal list)
     const uint32_t* allow = nullptr;
     uint64_t allow_bits = 0;
+    const uint32_t* allow_of_q = nullptr;  // per-query bitmap index, as in ExactParams (nullable)
     // 16-bit float rows, warp-per-query kernel only: evaluate the rows on the tensor cores (mma.sync, candidate-grade
     // distances — the caller re-ranks the rows it returns).  graph_search_uses_mma() tells which launches honour it.
     bool mma = false;

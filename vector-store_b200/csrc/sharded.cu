@@ -42,7 +42,7 @@ struct Sharded {
     DevBuf g_keys, g_dists, out_buf, q0;
     PinBuf pin;  // pinned staging of the merged results for pageable callers
     // per shard
-    std::vector<DevBuf> qbuf, allow;
+    std::vector<DevBuf> qbuf, allow, fidx;
     std::vector<cudaEvent_t> done_ev;
 
     uint32_t G() const { return (uint32_t)shards.size(); }
@@ -154,6 +154,7 @@ vsb_status create_sharded(const vsb_options* o, vsb_index** out) {
     ix->graph_stride = S.shards[0]->graph_stride;
     S.qbuf.resize(G);
     S.allow.resize(G);
+    S.fidx.resize(G);
     S.done_ev.resize(G, nullptr);
     cudaSetDevice(dev0);
     int prio_lo = 0, prio_hi = 0;
@@ -195,6 +196,7 @@ void destroy_sharded(vsb_index* ix) {
         if (i < S.done_ev.size() && S.done_ev[i]) cudaEventDestroy(S.done_ev[i]);
         if (i < S.qbuf.size()) S.qbuf[i].release();
         if (i < S.allow.size()) S.allow[i].release();
+        if (i < S.fidx.size()) S.fidx[i].release();
     }
     cudaSetDevice(ix->device);
     cudaDeviceSynchronize();
@@ -391,10 +393,11 @@ vsb_status sharded_get_build_stats(vsb_index* ix, vsb_build_stats* out) {
 }
 
 // Common body: queries are in `d_q` on device 0, valid once `ready` has fired; results land in o_* on device 0,
-// ordered on `s0`.  d_allow_host: optional host bitmap (uploaded to every shard).
+// ordered on `s0`.  hf: optional host bitmaps and per-query bitmap indices (uploaded to every shard); pop: admissible
+// rows of each bitmap, split evenly over the shards for the route selection.
 static vsb_status fan_out(vsb_index* ix, const float* d_q, cudaEvent_t ready, uint64_t nq, uint32_t k, uint64_t* o_keys,
-                          float* o_dists, uint32_t* o_counts, cudaStream_t s0, bool exact, const uint32_t* allow_host,
-                          uint64_t allow_bits, uint64_t allow_pop) {
+                          float* o_dists, uint32_t* o_counts, cudaStream_t s0, bool exact, const HostFilters& hf,
+                          const std::vector<uint64_t>& pop) {
     Sharded& S = *ix->sharded;
     const uint32_t G = S.G();
     const int dev0 = S.devices[0];
@@ -405,7 +408,9 @@ static vsb_status fan_out(vsb_index* ix, const float* d_q, cudaEvent_t ready, ui
     uint64_t* gk = S.g_keys.as<uint64_t>();
     float* gd = S.g_dists.as<float>();
     const size_t q_bytes = (size_t)nq * ix->dim * 4;
-    const size_t allow_words = allow_host ? (size_t)((allow_bits + 31) / 32) : 0;
+    const size_t allow_words = hf.bitmaps ? (size_t)((hf.bits + 31) / 32) * hf.n : 0;
+    std::vector<uint64_t> shard_pop(pop.size());
+    for (size_t f = 0; f < pop.size(); ++f) shard_pop[f] = pop[f] / G;
     ST(S.for_each([&](uint32_t i) -> vsb_status {
         vsb_index* sh = S.shards[i];
         CU(cudaSetDevice(S.devices[i]));
@@ -418,15 +423,23 @@ static vsb_status fan_out(vsb_index* ix, const float* d_q, cudaEvent_t ready, ui
             CU(cudaMemcpyPeerAsync(S.qbuf[i].p, S.devices[i], d_q, dev0, q_bytes, si));  // NVLink, device to device
             q_local = S.qbuf[i].as<float>();
         }
-        const uint32_t* d_allow = nullptr;
-        if (allow_host) {
+        Filters f;
+        if (hf.bitmaps) {
             CU(S.allow[i].ensure(std::max<size_t>(allow_words * 4, 16)));
-            CU(cudaMemcpyAsync(S.allow[i].p, allow_host, allow_words * 4, cudaMemcpyHostToDevice, si));
-            d_allow = S.allow[i].as<uint32_t>();
+            CU(cudaMemcpyAsync(S.allow[i].p, hf.bitmaps, allow_words * 4, cudaMemcpyHostToDevice, si));
+            f.d_allow = S.allow[i].as<uint32_t>();
+            f.bits = hf.bits;
+            f.n = hf.n;
+            f.pop = shard_pop.data();
+            if (hf.of_query) {
+                CU(S.fidx[i].ensure((size_t)nq * 4));
+                CU(cudaMemcpyAsync(S.fidx[i].p, hf.of_query, (size_t)nq * 4, cudaMemcpyHostToDevice, si));
+                f.d_fidx = S.fidx[i].as<uint32_t>();
+                f.h_fidx = hf.of_query;
+            }
         }
         // the shard's last kernel stores into device 0's gather buffer (peer-mapped): part i of [G][nq][k]
-        ST(sh->search_dev(q_local, nq, k, gk + (size_t)i * nq * k, gd + (size_t)i * nq * k, nullptr, si, exact, d_allow,
-                          allow_bits, allow_pop / G));
+        ST(sh->search_dev(q_local, nq, k, gk + (size_t)i * nq * k, gd + (size_t)i * nq * k, nullptr, si, exact, f));
         CU(cudaEventRecord(S.done_ev[i], si));
         return VSB_OK;
     }));
@@ -446,11 +459,11 @@ vsb_status sharded_search_dev(vsb_index* ix, const float* d_queries, uint64_t nq
     std::lock_guard<std::mutex> g(S.search);
     CU(cudaSetDevice(S.devices[0]));
     CU(cudaEventRecord(S.q_ready, stream));
-    return fan_out(ix, d_queries, S.q_ready, nq, k, d_keys, d_dists, d_counts, stream, exact, nullptr, 0, 0);
+    return fan_out(ix, d_queries, S.q_ready, nq, k, d_keys, d_dists, d_counts, stream, exact, HostFilters(), {});
 }
 
 vsb_status sharded_search_host(vsb_index* ix, const float* queries, uint64_t nq, uint32_t k, uint64_t* keys, float* dists,
-                               uint32_t* counts, bool exact, const uint32_t* allow_bitmap, uint64_t allow_bits) {
+                               uint32_t* counts, bool exact, const HostFilters& hf) {
     if (nq == 0) return VSB_OK;
     if (k == 0) return fail(VSB_EINVAL, "k must be > 0");
     if (!queries || !keys || !dists) return fail(VSB_EINVAL, "null buffer");
@@ -467,12 +480,11 @@ vsb_status sharded_search_host(vsb_index* ix, const float* queries, uint64_t nq,
     uint32_t* oc = reinterpret_cast<uint32_t*>(S.out_buf.as<uint8_t>() + al(kb) + al(db));
     CU(cudaMemcpyAsync(S.q0.p, queries, q_bytes, cudaMemcpyHostToDevice, S.stream0));
     CU(cudaEventRecord(S.q_ready, S.stream0));
-    uint64_t pop = 0;
-    if (allow_bitmap) {
-        const size_t words = (size_t)((allow_bits + 31) / 32);
-        for (size_t i = 0; i < words; ++i) pop += (uint64_t)__builtin_popcount(allow_bitmap[i]);
-    }
-    ST(fan_out(ix, S.q0.as<float>(), S.q_ready, nq, k, ok, od, oc, S.stream0, exact, allow_bitmap, allow_bits, pop));
+    std::vector<uint64_t> pop(hf.bitmaps ? hf.n : 0, 0);
+    const size_t words = (size_t)((hf.bits + 31) / 32);
+    for (size_t f = 0; f < pop.size(); ++f)
+        for (size_t i = 0; i < words; ++i) pop[f] += (uint64_t)__builtin_popcount(hf.bitmaps[f * words + i]);
+    ST(fan_out(ix, S.q0.as<float>(), S.q_ready, nq, k, ok, od, oc, S.stream0, exact, hf, pop));
     vsbi::HostReadback rb(S.pin, S.stream0);  // pageable destinations are staged (index_impl.h)
     CU(rb.reserve(al(kb) + al(db) + al(cb)));
     CU(rb.copy(keys, ok, kb));

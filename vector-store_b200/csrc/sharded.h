@@ -21,8 +21,7 @@ vsb_status sharded_set_kernel_timing(vsb_index* ix, int on);
 vsb_status sharded_get_stats(vsb_index* ix, vsb_stats* out);
 vsb_status sharded_get_build_stats(vsb_index* ix, vsb_build_stats* out);
 vsb_status sharded_search_host(vsb_index* ix, const float* queries, uint64_t nq, uint32_t k, uint64_t* keys,
-                               float* dists, uint32_t* counts, bool exact, const uint32_t* allow_bitmap,
-                               uint64_t allow_bits);
+                               float* dists, uint32_t* counts, bool exact, const HostFilters& hf = HostFilters());
 vsb_status sharded_search_dev(vsb_index* ix, const float* d_queries, uint64_t nq, uint32_t k, uint64_t* d_keys,
                               float* d_dists, uint32_t* d_counts, cudaStream_t stream, bool exact);
 vsb_status sharded_save(vsb_index* ix, const char* path);

@@ -237,6 +237,39 @@ class IndexActor:
         dists = np.array([h[1] for h in hits], dtype=np.float32)
         return self._to_hits(keys, dists, len(hits))
 
+    def filtered_ann_batch(self, embeddings, limit: int, predicates, max_row_id: int,
+                           partition_id: int = GLOBAL_PARTITION):
+        """A run of FilteredAnn requests on one partition in one call, as the Rust backend coalesces them:
+        predicates[i] filters embeddings[i]; each predicate becomes a bitmap over the row ids, identical bitmaps are
+        sent once, and every request gets what `filtered_ann` would return for it.  A None predicate is a plain Ann."""
+        e = np.asarray(embeddings, dtype=np.float32)
+        self._validate(e)
+        n = e.shape[0]
+        if len(predicates) != n:
+            raise ValueError("one predicate per embedding")
+        p = self.partitions.get(partition_id)
+        if p is None:
+            return [([], []) for _ in range(n)]
+        out = [None] * n
+        plain = [i for i in range(n) if predicates[i] is None]
+        for i in plain:
+            out[i] = self.ann(e[i], limit, partition_id)
+        filtered = [i for i in range(n) if predicates[i] is not None]
+        if filtered:
+            bits = max_row_id + 1
+            rows = np.arange(bits)
+            masks, index_of, fq = [], {}, []
+            for i in filtered:
+                m = np.fromiter((bool(predicates[i](int(r))) for r in rows), dtype=bool, count=bits)
+                j = index_of.setdefault(m.tobytes(), len(masks))
+                if j == len(masks):
+                    masks.append(m)
+                fq.append(j)
+            keys, dists, counts = p.idx.search_filtered_multi(e[filtered], limit, np.stack(masks), fq)
+            for r, i in enumerate(filtered):
+                out[i] = self._to_hits(keys[r], dists[r], counts[r])
+        return out
+
     def count(self) -> int:
         return self.size
 

@@ -208,6 +208,28 @@ class GpuIndex:
                                             _ptr(counts)))
         return keys, dists, counts
 
+    def search_filtered_multi(self, queries, k: int, masks, filter_of_query):
+        """Batched filtered search with one filter per query: masks is an [n_filters][bits] bool array (row i of a
+        mask admits the row whose id, key & 2^48-1, is i) and query j is filtered by masks[filter_of_query[j]]."""
+        q = np.ascontiguousarray(queries, dtype=np.float32)
+        self._check_dim(q)
+        m = np.asarray(masks, dtype=bool)
+        if m.ndim != 2:
+            raise ValueError("masks must be [n_filters][bits]")
+        bm = np.packbits(m, axis=1, bitorder="little")
+        bm = np.concatenate([bm, np.zeros((m.shape[0], (-bm.shape[1]) % 4), np.uint8)], axis=1)
+        bm = np.ascontiguousarray(bm).view(np.uint32)
+        fq = np.ascontiguousarray(filter_of_query, dtype=np.uint32)
+        n = q.shape[0]
+        if fq.shape != (n,):
+            raise ValueError("filter_of_query must hold one index per query")
+        keys = np.empty((n, k), dtype=np.uint64)
+        dists = np.empty((n, k), dtype=np.float32)
+        counts = np.empty(n, dtype=np.uint32)
+        check(self._lib.vsb_search_filtered_multi(self._h, _ptr(q), n, k, _ptr(bm), m.shape[0], m.shape[1], _ptr(fq),
+                                                  _ptr(keys), _ptr(dists), _ptr(counts)))
+        return keys, dists, counts
+
     def search_raw(self, q_ptr: int, n: int, k: int, keys_ptr: int, dists_ptr: int, counts_ptr: int,
                    exact: bool = False) -> None:
         """Host-pointer call without NumPy marshalling (bench e2e leg uses pinned torch buffers)."""
