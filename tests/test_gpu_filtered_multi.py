@@ -279,6 +279,44 @@ def test_sharded_handle_matches_single_device_on_the_exact_route():
     check_exact_per_query(x, keys, q, k, O.COS, O.F32, masks, fq, *out[0])
 
 
+def test_sharded_handle_routes_by_admissible_rows_below_bitmap_bits():
+    """Bits at and past bitmap_bits admit nothing and do not count when a filter picks its route: a bitmap just
+    under the exact-scan threshold, with stray bits in its last word, takes the exact route on a sharded handle as it
+    does on a single device."""
+    import torch
+    g = min(torch.cuda.device_count(), 8)
+    if g < 2:
+        pytest.skip("needs two or more GPUs")
+    n, dim, k, pct = 4000, 64, 10, 1
+    bits = 3617                                  # bits % 32 == 1: the last word holds one row and 31 stray bits
+    x = embedding_like(n, dim, n_clusters=16)
+    q = embedding_like(16, dim, seed=77, n_clusters=16)
+    keys = np.arange(n, dtype=np.uint64)
+    rng = np.random.default_rng(8)
+    ids = rng.choice(bits, 20, replace=False)    # 20 admissible rows: 0.5 %; 51 (1.3 %) with the stray bits
+    mask = np.zeros(n, bool)
+    mask[ids] = True
+    bm = np.zeros((bits + 31) // 32, np.uint32)
+    np.bitwise_or.at(bm, ids >> 5, (np.uint32(1) << (ids & 31).astype(np.uint32)))
+    bm[-1] |= np.uint32(0xFFFFFFFE)              # rows bits .. bits + 30 exist but lie past bitmap_bits
+    v = V()
+    out = []
+    for devices in (None, list(range(g))):
+        idx = v.GpuIndex(dim, v.Metric.Cos, v.Scalar.F32, devices=devices)
+        idx.set_search_params(min_graph_size=256, filter_exact_below_pct=pct)
+        idx.reserve(n)
+        idx.add_batch(keys, x)
+        idx.build()
+        assert idx.stats()["n_graphed"] == n
+        out.append([idx.filtered_search_bitmap(q[i], k, bm, bits) for i in range(len(q))])
+        idx.close()
+    assert out[1] == out[0]
+    ok, od, oc, _ = O.exact_topk(x, q, k, O.COS, O.F32, keys=keys, alive=mask.astype(np.uint8))
+    for i in range(len(q)):
+        assert [r[0] for r in out[0][i]] == [int(c) for c in ok[i][:oc[i]]]
+        assert [r[1] for r in out[0][i]] == [float(d) for d in od[i][:oc[i]]]
+
+
 # ---- actor mirror ---------------------------------------------------------------------------------------------------
 def test_actor_filtered_ann_batch_equals_one_call_per_query():
     v = V()

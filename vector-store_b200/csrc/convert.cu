@@ -210,13 +210,12 @@ void launch_convert_rows_i8s(const float* in, uint32_t n_rows, uint32_t dim, uin
     g_kernel_launches += 1;
 }
 
-void launch_gather_rows(const uint8_t* rows, uint32_t row_bytes, const float* sq, const float* nrm,
-                        const uint32_t* slots, uint32_t n, uint8_t* out_rows, float* out_sq, float* out_nrm,
-                        cudaStream_t stream) {
+void launch_gather_rows(const RowsView& src, const uint32_t* slots, uint32_t n, uint8_t* out_rows, float* out_sq,
+                        float* out_nrm, cudaStream_t stream) {
     if (n == 0) return;
     const int warps = 8;
-    gather_rows_kernel<<<(n + warps - 1) / warps, warps * 32, 0, stream>>>(rows, row_bytes, sq, nrm, slots, n,
-                                                                          out_rows, out_sq, out_nrm);
+    gather_rows_kernel<<<(n + warps - 1) / warps, warps * 32, 0, stream>>>(src.rows, src.row_bytes, src.sq, src.nrm, slots,
+                                                                          n, out_rows, out_sq, out_nrm);
     g_kernel_launches += 1;
 }
 

@@ -678,7 +678,7 @@ void launch_exact_candidates(const ExactParams& p, cudaStream_t stream) {
     a.q_rows = p.q.rows; a.q_sq = p.q.sq; a.q_nrm = p.q.nrm; a.nq = p.q.n; a.q_row_bytes = p.q.row_bytes;
     a.x_rows = p.x.rows; a.x_sq = p.x.sq; a.x_nrm = p.x.nrm; a.x_row_bytes = p.x.row_bytes;
     a.x_lo = p.x_lo; a.x_hi = p.x_hi;
-    a.deny = p.deny; a.keys = p.keys; a.allow = p.allow; a.allow_bits = p.allow_bits; a.allow_of_q = p.allow_of_q;
+    a.deny = p.deny; a.keys = p.keys; a.allow = p.allow.bm; a.allow_bits = p.allow.bits; a.allow_of_q = p.allow.of_q;
     a.kp = p.kp; a.n_splits = p.n_splits;
     const uint32_t rows = p.x_hi - p.x_lo;
     uint32_t rps = (rows + p.n_splits - 1) / p.n_splits;
@@ -710,7 +710,7 @@ void launch_exact_scan(const ExactParams& p, uint32_t k, cudaStream_t stream) {
     ScanArgs a;
     a.q_rows = p.q.rows; a.q_nrm = p.q.nrm; a.nq = p.q.n; a.q_row_bytes = p.q.row_bytes;
     a.x_rows = p.x.rows; a.x_nrm = p.x.nrm; a.x_row_bytes = p.x.row_bytes; a.x_lo = p.x_lo; a.x_hi = p.x_hi;
-    a.deny = p.deny; a.keys = p.keys; a.allow = p.allow; a.allow_bits = p.allow_bits; a.allow_of_q = p.allow_of_q;
+    a.deny = p.deny; a.keys = p.keys; a.allow = p.allow.bm; a.allow_bits = p.allow.bits; a.allow_of_q = p.allow.of_q;
     a.kf = p.kp;  // the caller sets kp = round_up(k (+1 for self), 32): lists hold exactly what K3 needs
     (void)k;
     a.n_splits = p.n_splits;

@@ -787,7 +787,7 @@ bool launch_exact_candidates_tc(const ExactParams& p, cudaStream_t stream, bool 
     TcArgs a;
     a.q_sq = p.q.sq; a.q_nrm = p.q.nrm; a.nq = p.q.n;
     a.x_sq = p.x.sq; a.x_nrm = p.x.nrm; a.x_lo = p.x_lo; a.x_hi = p.x_hi; a.row_bytes = p.x.row_bytes;
-    a.deny = p.deny; a.keys = p.keys; a.allow = p.allow; a.allow_bits = p.allow_bits; a.allow_of_q = p.allow_of_q;
+    a.deny = p.deny; a.keys = p.keys; a.allow = p.allow.bm; a.allow_bits = p.allow.bits; a.allow_of_q = p.allow.of_q;
     a.kp = p.kp; a.n_splits = p.n_splits;
     if (p.n_splits % TC_HALVES != 0) return false;  // callers size the lists with exact_tc_pick_splits
     const uint32_t row_splits = p.n_splits / TC_HALVES;

@@ -83,10 +83,10 @@ void launch_graph_search(const SearchParams& p, cudaStream_t stream) {
     a.metric = p.metric;
     a.out_keys = p.out_keys; a.out_dists = p.out_dists; a.out_counts = p.out_counts; a.out_packed = p.out_packed; a.self_base = p.self_base; a.counters = p.counters;
     a.out_stride = p.out_stride ? p.out_stride : p.k;
-    a.allow = p.allow;
-    a.allow_bits = p.allow_bits;
-    a.allow_of_q = p.allow_of_q;
-    a.rk = p.allow != nullptr ? ((p.k + 31) / 32) * 32 : 0;
+    a.allow = p.allow.bm;
+    a.allow_bits = p.allow.bits;
+    a.allow_of_q = p.allow.of_q;
+    a.rk = p.allow.bm != nullptr ? ((p.k + 31) / 32) * 32 : 0;
     a.mma = 0;
     static const uint32_t compact_env = [] {
         const char* e = getenv("VSB_K4_COMPACT");
@@ -100,7 +100,7 @@ void launch_graph_search(const SearchParams& p, cudaStream_t stream) {
     a.l2pf = l2pf_env;
     const int cpl = pick_cpl((int)(p.x.row_bytes / 16));
     // filtered ANN always runs the warp-per-query kernel (the second list lives there)
-    if (p.q.n <= graph_search_small_batch() && p.allow == nullptr) {
+    if (p.q.n <= graph_search_small_batch() && p.allow.bm == nullptr) {
         // CTA-per-query kernel: 8 warps and up to 8 parents per iteration for one query
         a.search_width = a.search_width < 4 ? 8 : (a.search_width > 8 ? 8 : a.search_width);
         a.max_iters = p.max_iters ? p.max_iters : (2 * a.itopk) / a.search_width + 8;
@@ -118,7 +118,7 @@ void launch_graph_search(const SearchParams& p, cudaStream_t stream) {
         return;
     }
     dim3 grid((p.q.n + K4_WARPS - 1) / K4_WARPS);
-    a.mma = (p.mma && p.allow == nullptr && (p.storage == VSB_ST_BF16 || p.storage == VSB_ST_F16)) ? 1u : 0u;
+    a.mma = (p.mma && p.allow.bm == nullptr && (p.storage == VSB_ST_BF16 || p.storage == VSB_ST_F16)) ? 1u : 0u;
     const size_t smem = (size_t)K4_WARPS * ((size_t)a.itopk * 8 + ((size_t)2 << bits) + (size_t)a.queue_cap * 8 + (size_t)a.rk * 8 + 64 * 8);
     switch (p.storage) {
         case VSB_ST_F32: launch_k4_f32(a, cpl, grid, smem, stream); break;

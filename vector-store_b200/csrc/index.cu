@@ -148,36 +148,16 @@ size_t vsb_index::hbm_bytes() {
     return s;
 }
 
-vsb::RowsView vsb_index::rows_view(const vsbi::View& v) const {
-    vsb::RowsView r;
-    r.rows = v.st->rows.as<uint8_t>();
-    r.sq = v.st->sq.as<float>();
-    r.nrm = v.st->nrm.as<float>();
-    r.row_bytes = row_bytes;
-    r.n = v.n_slots;
-    return r;
-}
-
 // ---- mutators (mut_mu held by the caller) -----------------------------------------------------------------------
 vsb_status vsb_index::new_store(uint64_t cap, std::shared_ptr<vsbi::Store>& out) {
     auto st = std::make_shared<vsbi::Store>();
     const uint64_t words = (cap + 31) / 32;
     st->capacity = cap;
-    CU(st->rows.alloc((size_t)cap * row_bytes));
-    CU(st->sq.alloc((size_t)cap * 4));
-    CU(st->nrm.alloc((size_t)cap * 4));
+    CU(st->rows.alloc(cap, row_bytes));
     CU(st->keys.alloc((size_t)cap * 8));
     CU(st->deny.alloc((size_t)words * 4));
-    if (trav16) {
-        CU(st->rows16.alloc((size_t)cap * row_bytes16));
-        CU(st->sq16.alloc((size_t)cap * 4));
-        CU(st->nrm16.alloc((size_t)cap * 4));
-    }
-    if (trav8) {
-        CU(st->rows8.alloc((size_t)cap * row_bytes8));
-        CU(st->sq8.alloc((size_t)cap * 4));
-        CU(st->nrm8.alloc((size_t)cap * 4));
-    }
+    if (trav16) CU(st->bf16.alloc(cap, row_bytes16));
+    if (trav8) CU(st->i8.alloc(cap, row_bytes8));
     CU(cudaMemsetAsync(st->deny.p, 0, (size_t)words * 4, mstream));
     out = std::move(st);
     return VSB_OK;
@@ -201,21 +181,15 @@ vsb_status vsb_index::reserve(uint64_t cap) {
         auto cp = [&](const DevBuf& dst, const DevBuf& src, size_t bytes) {
             return cudaMemcpyAsync(dst.p, src.p, bytes, cudaMemcpyDeviceToDevice, mstream);
         };
-        CU(cp(ns->rows, o.rows, n * row_bytes));
-        CU(cp(ns->sq, o.sq, n * 4));
-        CU(cp(ns->nrm, o.nrm, n * 4));
+        for (auto b : vsbi::kStoreRows) {
+            const vsbi::RowBuf &from = o.*b, &to = (*ns).*b;
+            if (from.row_bytes == 0) continue;
+            CU(cp(to.rows, from.rows, n * from.row_bytes));
+            CU(cp(to.sq, from.sq, n * 4));
+            CU(cp(to.nrm, from.nrm, n * 4));
+        }
         CU(cp(ns->keys, o.keys, n * 8));
         CU(cp(ns->deny, o.deny, ((n + 31) / 32) * 4));
-        if (trav16) {
-            CU(cp(ns->rows16, o.rows16, n * row_bytes16));
-            CU(cp(ns->sq16, o.sq16, n * 4));
-            CU(cp(ns->nrm16, o.nrm16, n * 4));
-        }
-        if (trav8) {
-            CU(cp(ns->rows8, o.rows8, n * row_bytes8));
-            CU(cp(ns->sq8, o.sq8, n * 4));
-            CU(cp(ns->nrm8, o.nrm8, n * 4));
-        }
     }
     CU(cudaStreamSynchronize(mstream));
     w.st = ns;
@@ -297,20 +271,10 @@ vsb_status vsb_index::add(const uint64_t* k, const float* r, uint64_t n, int32_t
             d_src = ms.q_in.as<float>();
         }
         const uint32_t s0 = w.n_slots + (uint32_t)b;
-        vsb::launch_convert_rows(storage, d_src, (uint32_t)nb, dim, st.rows.as<uint8_t>() + (size_t)s0 * row_bytes,
-                                 row_bytes, st.sq.as<float>() + s0, st.nrm.as<float>() + s0, mstream);
+        vsb::launch_convert_rows(storage, d_src, (uint32_t)nb, dim, st.rows.rows.as<uint8_t>() + (size_t)s0 * row_bytes,
+                                 row_bytes, st.rows.sq.as<float>() + s0, st.rows.nrm.as<float>() + s0, mstream);
         CU(cudaGetLastError());
-        if (trav16) {
-            vsb::launch_convert_rows(VSB_BF16, d_src, (uint32_t)nb, dim,
-                                     st.rows16.as<uint8_t>() + (size_t)s0 * row_bytes16, row_bytes16, st.sq16.as<float>() + s0,
-                                     st.nrm16.as<float>() + s0, mstream);
-            CU(cudaGetLastError());
-        }
-        if (trav8) {
-            vsb::launch_convert_rows_i8s(d_src, (uint32_t)nb, dim, dim, st.rows8.as<uint8_t>() + (size_t)s0 * row_bytes8,
-                                         row_bytes8, st.sq8.as<float>() + s0, st.nrm8.as<float>() + s0, mstream);
-            CU(cudaGetLastError());
-        }
+        ST(derive_traversal(st, d_src, dim, s0, (uint32_t)nb));
         CU(cudaMemcpyAsync(st.keys.as<uint64_t>() + s0, src_keys + b, nb * 8, cudaMemcpyHostToDevice, mstream));
         CU(cudaStreamSynchronize(mstream));  // q_in is reused by the next chunk
     }
@@ -325,6 +289,20 @@ vsb_status vsb_index::add(const uint64_t* k, const float* r, uint64_t n, int32_t
     if (w.n_graphed > 0 && stream_threshold > 0 && w.n_slots - w.n_graphed >= stream_threshold) {
         ST(stream_insert());
         publish();
+    }
+    return VSB_OK;
+}
+
+vsb_status vsb_index::derive_traversal(vsbi::Store& st, const float* src, uint32_t in_stride, uint32_t s0, uint32_t n) {
+    if (trav16) {
+        vsb::launch_convert_rows(VSB_BF16, src, n, in_stride, st.bf16.rows.as<uint8_t>() + (size_t)s0 * row_bytes16, row_bytes16,
+                                 st.bf16.sq.as<float>() + s0, st.bf16.nrm.as<float>() + s0, mstream);
+        CU(cudaGetLastError());
+    }
+    if (trav8) {
+        vsb::launch_convert_rows_i8s(src, n, dim, in_stride, st.i8.rows.as<uint8_t>() + (size_t)s0 * row_bytes8, row_bytes8,
+                                     st.i8.sq.as<float>() + s0, st.i8.nrm.as<float>() + s0, mstream);
+        CU(cudaGetLastError());
     }
     return VSB_OK;
 }
@@ -387,16 +365,9 @@ vsb_status vsb_index::compact(bool keep_graph) {
     DevBuf d_slots, d_map;
     CU(d_slots.alloc(std::max<size_t>((size_t)m * 4, 16)));
     CU(cudaMemcpyAsync(d_slots.p, live_slots.data(), (size_t)m * 4, cudaMemcpyHostToDevice, mstream));
-    vsb::launch_gather_rows(o.rows.as<uint8_t>(), row_bytes, o.sq.as<float>(), o.nrm.as<float>(), d_slots.as<uint32_t>(), m,
-                            ns->rows.as<uint8_t>(), ns->sq.as<float>(), ns->nrm.as<float>(), mstream);
+    for (auto b : vsbi::kStoreRows)
+        if ((o.*b).row_bytes) vsbi::gather_rows((o.*b).view(n_old), d_slots.as<uint32_t>(), m, (*ns).*b, mstream);
     vsb::launch_gather_u64(o.keys.as<uint64_t>(), d_slots.as<uint32_t>(), m, ns->keys.as<uint64_t>(), mstream);
-    if (trav16)
-        vsb::launch_gather_rows(o.rows16.as<uint8_t>(), row_bytes16, o.sq16.as<float>(), o.nrm16.as<float>(),
-                                d_slots.as<uint32_t>(), m, ns->rows16.as<uint8_t>(), ns->sq16.as<float>(),
-                                ns->nrm16.as<float>(), mstream);
-    if (trav8)
-        vsb::launch_gather_rows(o.rows8.as<uint8_t>(), row_bytes8, o.sq8.as<float>(), o.nrm8.as<float>(), d_slots.as<uint32_t>(),
-                                m, ns->rows8.as<uint8_t>(), ns->sq8.as<float>(), ns->nrm8.as<float>(), mstream);
     CU(cudaGetLastError());
     std::vector<uint32_t> old2new((size_t)n_old, vsb::kInvalidSlot);
     for (uint32_t i = 0; i < m; ++i) old2new[live_slots[i]] = i;

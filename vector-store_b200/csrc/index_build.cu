@@ -67,33 +67,21 @@ vsb_status vsb_index::build() {
     const uint32_t kin = std::min<uint32_t>(k_init, 128);
     DevBuf knn;
     CU(knn.alloc((size_t)n * kin * 8));
-    const vsb::RowsView x = rows_view(w);
     const vsbi::Store& st = *w.st;
     // f32 storage: the all-pairs candidate stage runs on a bf16 copy (kNN lists only need candidate-grade
     // distances; K3 re-evaluates the survivors on the f32 rows in the canonical order)
-    DevBuf sh_rows, sh_sq, sh_nrm;
+    vsbi::RowBuf sh;
     vsb::RowsView shx;
     const bool use_shadow = storage == VSB_F32 && tc_enabled && n >= tc_min_rows;
     if (use_shadow) {
         if (trav16) {  // the traversal copy IS that shadow
-            shx.rows = st.rows16.as<uint8_t>();
-            shx.sq = st.sq16.as<float>();
-            shx.nrm = st.nrm16.as<float>();
-            shx.row_bytes = row_bytes16;
-            shx.n = n;
+            shx = st.bf16.view(n);
         } else {
-            const uint32_t dim_pad = row_bytes / 4;
-            shx.row_bytes = ((dim_pad * 2 + 15) / 16) * 16;
-            shx.n = n;
-            CU(sh_rows.alloc((size_t)n * shx.row_bytes));
-            CU(sh_sq.alloc((size_t)n * 4));
-            CU(sh_nrm.alloc((size_t)n * 4));
-            vsb::launch_convert_rows(VSB_BF16, reinterpret_cast<const float*>(x.rows), n, dim_pad, sh_rows.as<uint8_t>(),
-                                     shx.row_bytes, sh_sq.as<float>(), sh_nrm.as<float>(), mstream);
+            CU(sh.alloc(n, row_bytes16));
+            vsb::launch_convert_rows(VSB_BF16, st.rows.rows.as<float>(), n, row_bytes / 4, sh.rows.as<uint8_t>(), row_bytes16,
+                                     sh.sq.as<float>(), sh.nrm.as<float>(), mstream);
             CU(cudaGetLastError());
-            shx.rows = sh_rows.as<uint8_t>();
-            shx.sq = sh_sq.as<float>();
-            shx.nrm = sh_nrm.as<float>();
+            shx = sh.view(n);
         }
     }
     {
@@ -102,31 +90,21 @@ vsb_status vsb_index::build() {
         // query blocks of one 128-row tensor-core tile per SM: a block is exactly one wave of K1-TC CTAs
         const uint32_t QB = std::max<uint32_t>(16384, (uint32_t)sm_count * 128);
         for (uint32_t b0 = 0; b0 < n; b0 += QB) {
-            vsb::RowsView q;
-            q.n = std::min(QB, n - b0);
-            q.rows = x.rows + (size_t)b0 * row_bytes;
-            q.sq = x.sq + b0;
-            q.nrm = x.nrm + b0;
-            q.row_bytes = row_bytes;
-            vsb::RowsView shq = shx;
-            if (use_shadow) {
-                shq.n = q.n;
-                shq.rows = shx.rows + (size_t)b0 * shx.row_bytes;
-                shq.sq = shx.sq + b0;
-                shq.nrm = shx.nrm + b0;
-            }
-            ST(exact_block(w, ms, q, x, 0, n, nullptr, st.keys.as<uint64_t>(), nullptr, 0, nullptr, kin, nullptr, nullptr, nullptr,
-                           knn.as<uint64_t>() + (size_t)b0 * kin, (int64_t)b0, mstream, true, use_shadow ? &shq : nullptr,
-                           use_shadow ? &shx : nullptr));
+            const uint32_t nb = std::min(QB, n - b0);
+            const vsb::RowsView shq = use_shadow ? shx.slice(b0, nb) : vsb::RowsView{};
+            vsbi::TopK out;
+            out.packed = knn.as<uint64_t>() + (size_t)b0 * kin;
+            out.self_base = b0;
+            // no tombstones here (compacted above), no filter
+            ST(exact_block(ms, exact_in(w, st.rows.view(nb, b0), 0, n, vsb::Allow{}), kin, out, mstream, true,
+                           use_shadow ? &shq : nullptr, use_shadow ? &shx : nullptr));
         }
         bstats.allpairs_ns = t.stop();
         bstats.allpairs_rows = n;
         bstats.allpairs_flops = 2ull * n * n * dim;
         nvtxRangePop();
     }
-    sh_rows.release();
-    sh_sq.release();
-    sh_nrm.release();
+    sh.release();
     ST(graph_from_knn(knn.as<uint64_t>(), n, kin, nullptr));
     knn.release();
     // the reachability pass (extra seeds for lost components) runs on the FINAL graph only
@@ -194,28 +172,18 @@ vsb_status vsb_index::refine_graph() {
     run.max_iters = 0;
     run.n_seeds = 32;
     run.search_width = build_search_width;  // 2 parents per iteration: ~10 % more evaluations, but twice the rows in flight per warp
+    run.evals = &bstats.refine_evals;
+    run.parents = &bstats.refine_parents;
     {
         EvTimer t(mstream);
         const uint32_t QB = 16384;
         for (uint32_t b0 = 0; b0 < n; b0 += QB) {
             const uint32_t nb = std::min(QB, n - b0);
-            vsb::RowsView qv;
-            qv.rows = st.rows.as<uint8_t>() + (size_t)b0 * row_bytes;
-            qv.sq = st.sq.as<float>() + b0;
-            qv.nrm = st.nrm.as<float>() + b0;
-            qv.row_bytes = row_bytes;
-            qv.n = nb;
-            vsb::RowsView q16;
-            if (trav16) {
-                q16.rows = st.rows16.as<uint8_t>() + (size_t)b0 * row_bytes16;
-                q16.sq = st.sq16.as<float>() + b0;
-                q16.nrm = st.nrm16.as<float>() + b0;
-                q16.row_bytes = row_bytes16;
-                q16.n = nb;
-            }
-            ST(graph_block(w, ms, run, qv, nb, kin, nullptr, nullptr, nullptr, knn.as<uint64_t>() + (size_t)b0 * kin,
-                           trav16 ? &q16 : nullptr, mstream, (long long)b0, false, &bstats.refine_evals,
-                           &bstats.refine_parents));
+            const vsb::RowsView q16 = trav16 ? st.bf16.view(nb, b0) : vsb::RowsView{};
+            vsbi::TopK out;
+            out.packed = knn.as<uint64_t>() + (size_t)b0 * kin;
+            out.self_base = b0;
+            ST(graph_block(w, ms, run, st.rows.view(nb, b0), kin, out, trav16 ? &q16 : nullptr, mstream));
         }
         bstats.refine_ns += t.stop();
         bstats.refine_rows += n;
@@ -230,7 +198,6 @@ vsb_status vsb_index::refine_graph() {
 vsb_status vsb_index::sample_seeds(uint32_t n, bool ensure_reach) {
     nvtxRangePushA("build.seeds");
     EvTimer t(mstream);
-    const vsb::RowsView x = rows_view(w);
     const vsbi::Store& st = *w.st;
     uint64_t live_below = 0;
     for (uint32_t wd = 0; wd < (n + 31) / 32; ++wd) live_below += __builtin_popcount(~h_deny[wd]);
@@ -282,10 +249,7 @@ vsb_status vsb_index::sample_seeds(uint32_t n, bool ensure_reach) {
                 for (int i = 0; i < 4; ++i)
                     vsb::launch_reach_step(w.gr->g.as<uint32_t>(), n, graph_stride, degree, state, flag, mstream);
                 uint32_t changed = 0;
-                vsbi::HostReadback rb(ms.pin, mstream);
-                CU(rb.reserve(4));
-                CU(rb.copy(&changed, flag, 4));
-                CU(rb.finish());
+                CU(vsbi::HostReadback::read(ms.pin, mstream, &changed, flag, 4));
                 if (!changed) break;
             }
             return VSB_OK;
@@ -297,12 +261,7 @@ vsb_status vsb_index::sample_seeds(uint32_t n, bool ensure_reach) {
         while (extra_seeds < reach_budget) {
             const uint32_t room = std::min<uint32_t>(kPromote, reach_budget - extra_seeds);
             vsb::launch_collect_unreached(state, deny_bm, n, room, found, mstream);
-            {
-                vsbi::HostReadback rb(ms.pin, mstream);
-                CU(rb.reserve((size_t)(1 + room) * 4));
-                CU(rb.copy(h_found.data(), found, (size_t)(1 + room) * 4));
-                CU(rb.finish());
-            }
+            CU(vsbi::HostReadback::read(ms.pin, mstream, h_found.data(), found, (size_t)(1 + room) * 4));
             const uint32_t cnt = std::min(h_found[0], room);
             if (cnt == 0) break;
             for (uint32_t i = 0; i < cnt; ++i) h_seeds.push_back(h_found[1 + i]);
@@ -316,21 +275,14 @@ vsb_status vsb_index::sample_seeds(uint32_t n, bool ensure_reach) {
         CU(sd->slots.alloc((size_t)std::max<uint32_t>(S, 1) * 4));
     }
     sd->extra = extra_seeds;
-    CU(sd->rows.alloc((size_t)S * row_bytes));
-    CU(sd->sq.alloc((size_t)S * 4));
-    CU(sd->nrm.alloc((size_t)S * 4));
+    CU(sd->rows.alloc(S, row_bytes));
     CU(cudaMemcpyAsync(sd->slots.p, h_seeds.data(), (size_t)S * 4, cudaMemcpyHostToDevice, mstream));
-    vsb::launch_gather_rows(x.rows, row_bytes, x.sq, x.nrm, sd->slots.as<uint32_t>(), S, sd->rows.as<uint8_t>(),
-                            sd->sq.as<float>(), sd->nrm.as<float>(), mstream);
+    vsbi::gather_rows(st.rows.view(w.n_slots), sd->slots.as<uint32_t>(), S, sd->rows, mstream);
     CU(cudaGetLastError());
     if (storage == VSB_F32) {
-        const uint32_t dim_pad = row_bytes / 4;
-        const uint32_t rb16 = ((dim_pad * 2 + 15) / 16) * 16;
-        CU(sd->rows16.alloc((size_t)S * rb16));
-        CU(sd->sq16.alloc((size_t)S * 4));
-        CU(sd->nrm16.alloc((size_t)S * 4));
-        vsb::launch_convert_rows(VSB_BF16, sd->rows.as<float>(), S, dim_pad, sd->rows16.as<uint8_t>(), rb16,
-                                 sd->sq16.as<float>(), sd->nrm16.as<float>(), mstream);
+        CU(sd->bf16.alloc(S, row_bytes16));
+        vsb::launch_convert_rows(VSB_BF16, sd->rows.rows.as<float>(), S, row_bytes / 4, sd->bf16.rows.as<uint8_t>(), row_bytes16,
+                                 sd->bf16.sq.as<float>(), sd->bf16.nrm.as<float>(), mstream);
         CU(cudaGetLastError());
     }
     CU(cudaStreamSynchronize(mstream));
@@ -369,6 +321,8 @@ vsb_status vsb_index::stream_insert() {
     run.max_iters = 0;
     run.n_seeds = 32;
     run.search_width = build_search_width;
+    run.evals = &bstats.stream_evals;
+    run.parents = &bstats.stream_parents;
     DevBuf cand, link_scratch;
     const uint32_t QB = 8192;
     CU(cand.alloc((size_t)QB * C * 8));
@@ -381,22 +335,10 @@ vsb_status vsb_index::stream_insert() {
         if (w.sd && w.n_graphed >= 2 * std::max<uint32_t>(w.sd->sampled_rows, 1024)) ST(sample_seeds(w.n_graphed, false));
         const uint32_t t0 = w.n_graphed;
         const uint32_t nb = std::min(QB, w.n_slots - t0);
-        vsb::RowsView qv;
-        qv.rows = st.rows.as<uint8_t>() + (size_t)t0 * row_bytes;
-        qv.sq = st.sq.as<float>() + t0;
-        qv.nrm = st.nrm.as<float>() + t0;
-        qv.row_bytes = row_bytes;
-        qv.n = nb;
-        vsb::RowsView q16;
-        if (trav16) {
-            q16.rows = st.rows16.as<uint8_t>() + (size_t)t0 * row_bytes16;
-            q16.sq = st.sq16.as<float>() + t0;
-            q16.nrm = st.nrm16.as<float>() + t0;
-            q16.row_bytes = row_bytes16;
-            q16.n = nb;
-        }
-        ST(graph_block(w, ms, run, qv, nb, C, nullptr, nullptr, nullptr, cand.as<uint64_t>(), trav16 ? &q16 : nullptr, mstream,
-                       -1, false, &bstats.stream_evals, &bstats.stream_parents));
+        const vsb::RowsView q16 = trav16 ? st.bf16.view(nb, t0) : vsb::RowsView{};
+        vsbi::TopK out;
+        out.packed = cand.as<uint64_t>();
+        ST(graph_block(w, ms, run, st.rows.view(nb, t0), C, out, trav16 ? &q16 : nullptr, mstream));
         CU(vsb::launch_stream_link(cand.as<uint64_t>(), nb, C, t0, R, w.gr->g.as<uint32_t>(), graph_stride, link_scratch.p,
                                    link_bytes, mstream));
         w.n_graphed = t0 + nb;  // later batches may link to these rows (stream order)

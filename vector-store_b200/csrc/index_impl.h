@@ -146,6 +146,43 @@ struct DevBuf {
 
 inline uint32_t round_up(uint32_t v, uint32_t m) { return (v + m - 1) / m * m; }
 
+// A block of rows in one storage format: [n][row_bytes] bytes plus the canonical sum of squares and norm of each row.
+struct RowBuf {
+    DevBuf rows, sq, nrm;
+    uint32_t row_bytes = 0;  // 0: no rows (a traversal copy the index does not keep)
+    // exact size (contents undefined)
+    cudaError_t alloc(size_t n, uint32_t rb) {
+        row_bytes = rb;
+        cudaError_t e = rows.alloc(n * rb);
+        if (e == cudaSuccess) e = sq.alloc(n * 4);
+        if (e == cudaSuccess) e = nrm.alloc(n * 4);
+        return e;
+    }
+    // grow-only scratch (contents not preserved; see DevBuf::ensure)
+    cudaError_t ensure(size_t n, uint32_t rb) {
+        row_bytes = rb;
+        cudaError_t e = rows.ensure(n * rb);
+        if (e == cudaSuccess) e = sq.ensure(n * 4);
+        if (e == cudaSuccess) e = nrm.ensure(n * 4);
+        return e;
+    }
+    // rows [first, first + n)
+    vsb::RowsView view(uint32_t n, uint32_t first = 0) const {
+        return vsb::RowsView{rows.as<uint8_t>(), sq.as<float>(), nrm.as<float>(), row_bytes, n}.slice(first, n);
+    }
+    size_t bytes() const { return rows.bytes + sq.bytes + nrm.bytes; }
+    void release() {
+        rows.release();
+        sq.release();
+        nrm.release();
+    }
+};
+
+// dst row i = src row slots[i], for i < n
+inline void gather_rows(const vsb::RowsView& src, const uint32_t* slots, uint32_t n, RowBuf& dst, cudaStream_t s) {
+    vsb::launch_gather_rows(src, slots, n, dst.rows.as<uint8_t>(), dst.sq.as<float>(), dst.nrm.as<float>(), s);
+}
+
 // Device -> host copies never go straight into PAGEABLE memory: for such a destination cudaMemcpyAsync waits INSIDE the
 // call — holding the context lock — until the stream has reached the copy, and every other thread's CUDA call queues up
 // behind it.  Measured in config C5: while a refinement pass read back its 16-byte work counters after each K4 launch,
@@ -216,19 +253,41 @@ class HostReadback {
         used = 0;
         return cudaSuccess;
     }
+    // one device -> host copy on `s`, waited for
+    static cudaError_t read(PinBuf& pin, cudaStream_t s, void* dst, const void* src_dev, size_t bytes) {
+        HostReadback rb(pin, s);
+        cudaError_t e = rb.reserve(bytes);
+        if (e == cudaSuccess) e = rb.copy(dst, src_dev, bytes);
+        return e == cudaSuccess ? rb.finish() : e;
+    }
+};
+
+// The device block of a search with host buffers: queries (q_bytes, 0 when they are staged elsewhere), then the
+// keys, dists and counts of nq x k results and, if asked for, nq bitmap indices; each part starts on 256 bytes.
+struct Staging {
+    float* q = nullptr;
+    uint64_t* keys = nullptr;
+    float* dists = nullptr;
+    uint32_t* counts = nullptr;
+    uint32_t* fidx = nullptr;
+    size_t keys_bytes = 0, dists_bytes = 0, counts_bytes = 0;
+    cudaError_t carve(DevBuf& buf, size_t q_bytes, uint64_t nq, uint32_t k, bool with_fidx);
+    // copies the results to the host buffers (counts_out nullable) on `s` and waits for them
+    cudaError_t read(PinBuf& pin, cudaStream_t s, uint64_t* keys_out, float* dists_out, uint32_t* counts_out) const;
 };
 
 // capacity-sized per-row arrays; reserve / compaction build a NEW store and publish it
 struct Store {
     uint64_t capacity = 0;
-    DevBuf rows, sq, nrm, keys, deny;
-    DevBuf rows16, sq16, nrm16;  // VSB_FLAG_BF16_TRAVERSAL: bf16 copy of the rows for K4
-    DevBuf rows8, sq8, nrm8;     // VSB_FLAG_I8_TRAVERSAL: scaled-int8 copy
-    size_t bytes() const {
-        return rows.bytes + sq.bytes + nrm.bytes + keys.bytes + deny.bytes + rows16.bytes + sq16.bytes + nrm16.bytes +
-               rows8.bytes + sq8.bytes + nrm8.bytes;
-    }
+    RowBuf rows;  // the stored rows
+    RowBuf bf16;  // VSB_FLAG_BF16_TRAVERSAL: bf16 copy of the rows for K4
+    RowBuf i8;    // VSB_FLAG_I8_TRAVERSAL: scaled-int8 copy
+    DevBuf keys, deny;
+    size_t bytes() const { return rows.bytes() + bf16.bytes() + i8.bytes() + keys.bytes + deny.bytes; }
 };
+// every row block of a store: the stored rows and the traversal copies (row_bytes == 0 where the index has none)
+using StoreRows = RowBuf Store::*;
+inline constexpr StoreRows kStoreRows[] = {&Store::rows, &Store::bf16, &Store::i8};
 
 struct Graph {
     DevBuf g;  // [cap_rows][stride] u32
@@ -236,11 +295,12 @@ struct Graph {
 };
 
 struct Seeds {
-    DevBuf rows, sq, nrm, slots;
-    DevBuf rows16, sq16, nrm16;  // bf16 shadow of the seed block (f32 storage only)
+    RowBuf rows;
+    RowBuf bf16;  // bf16 shadow of the seed block (f32 storage only)
+    DevBuf slots;
     uint32_t n = 0, extra = 0;
     uint32_t sampled_rows = 0;  // rows the sample was drawn from (the streaming insert re-samples when the graph has doubled)
-    size_t bytes() const { return rows.bytes + sq.bytes + nrm.bytes + slots.bytes + rows16.bytes + sq16.bytes + nrm16.bytes; }
+    size_t bytes() const { return rows.bytes() + bf16.bytes() + slots.bytes; }
 };
 
 struct View {
@@ -253,19 +313,20 @@ struct View {
 
 // per-caller-class scratch: one set for searches (under search_mu), one for mutators (under mut_mu)
 struct Scratch {
-    DevBuf q_in, q_rows, q_sq, q_nrm, q16_rows, q16_sq, q16_nrm, q8_rows, q8_sq, q8_nrm;
+    DevBuf q_in;
+    RowBuf q, q16, q8;  // converted queries, their bf16 and int8 shadows
     DevBuf part, seed_part, tmp_keys, tmp_dists, rr_packed, counters, allow;
-    DevBuf cert_state, fb_map, fb_rows, fb_sq, fb_nrm, fb_fidx;  // certified exact search
+    DevBuf cert_state, fb_map, fb_fidx;  // certified exact search
+    RowBuf fb;
     // filtered searches whose bitmaps take different routes: each route's queries, bitmap indices and results
-    DevBuf rt_map, rt_rows, rt_sq, rt_nrm, rt_fidx, rt_keys, rt_dists, rt_counts;
+    DevBuf rt_map, rt_fidx, rt_keys, rt_dists, rt_counts;
+    RowBuf rt;
     DevBuf thr_part, thr, thr_cnt;                       // sampled list bounds of the all-pairs build (exact_block)
     PinBuf pin;                                          // pinned staging of this caller class's read-backs
     size_t bytes() const {
-        const DevBuf* all[] = {&q_in, &q_rows, &q_sq, &q_nrm, &q16_rows, &q16_sq, &q16_nrm, &q8_rows, &q8_sq, &q8_nrm, &part,
-                               &seed_part, &tmp_keys, &tmp_dists, &rr_packed, &counters, &allow, &cert_state, &fb_map,
-                               &fb_rows, &fb_sq, &fb_nrm, &fb_fidx, &rt_map, &rt_rows, &rt_sq, &rt_nrm, &rt_fidx,
-                               &rt_keys, &rt_dists, &rt_counts, &thr_part, &thr, &thr_cnt};
-        size_t s = 0;
+        const DevBuf* all[] = {&q_in, &part, &seed_part, &tmp_keys, &tmp_dists, &rr_packed, &counters, &allow, &cert_state,
+                               &fb_map, &fb_fidx, &rt_map, &rt_fidx, &rt_keys, &rt_dists, &rt_counts, &thr_part, &thr, &thr_cnt};
+        size_t s = q.bytes() + q16.bytes() + q8.bytes() + fb.bytes() + rt.bytes();
         for (auto* b : all) s += b->bytes;
         return s;
     }
@@ -282,12 +343,25 @@ struct HostFilters {
 
 // The same call once the bitmaps are on the device: what search_dev needs to route and run it.
 struct Filters {
-    const uint32_t* d_allow = nullptr;  // [n][ceil(bits / 32)] (null: unfiltered search)
-    uint64_t bits = 0;
-    uint32_t n = 0;
-    const uint32_t* d_fidx = nullptr;  // [nq] bitmap index per query (null: bitmap 0 for every query)
-    const uint32_t* h_fidx = nullptr;  // host copy of d_fidx (route selection); null exactly when d_fidx is
+    vsb::Allow allow;                  // allow.bm null: unfiltered search
+    uint32_t n = 0;                    // bitmaps
+    const uint32_t* h_fidx = nullptr;  // host copy of allow.of_q (route selection); null exactly when allow.of_q is
     const uint64_t* pop = nullptr;     // host [n]: admissible rows per bitmap (route selection)
+};
+// index_search.cu: admissible rows of each bitmap (bits at and past hf.bits admit nothing and are not counted)
+std::vector<uint64_t> filter_population(const HostFilters& hf);
+// uploads the bitmaps into sc.allow on `s` and points f at them; d_fidx: the per-query indices, already on the device
+vsb_status upload_filters(Scratch& sc, const HostFilters& hf, const uint64_t* pop, const uint32_t* d_fidx, cudaStream_t s,
+                          Filters& f);
+
+// where a search block writes its top-k: the user-facing keys / dists / counts (each nullable) or the packed
+// (ord(dist) << 32 | slot) lists the build uses; self_base >= 0: query i is row self_base + i and skips itself
+struct TopK {
+    uint64_t* keys = nullptr;
+    float* dists = nullptr;
+    uint32_t* counts = nullptr;
+    uint64_t* packed = nullptr;
+    int64_t self_base = -1;
 };
 
 struct Sharded;  // sharded.cu: the multi-device router behind the same handle type
@@ -398,12 +472,13 @@ struct vsb_index {
     }
 
     size_t hbm_bytes();
-    vsb::RowsView rows_view(const vsbi::View& v) const;
 
     vsb_status new_store(uint64_t cap, std::shared_ptr<vsbi::Store>& out);
     vsb_status reserve(uint64_t cap);
     vsb_status add(const uint64_t* k, const float* r, uint64_t n, int32_t* row_status, uint64_t* n_added,
                    bool rows_on_device = false);
+    // the traversal copies of store rows [s0, s0 + n) from f32 rows `src` (in_stride floats apart)
+    vsb_status derive_traversal(vsbi::Store& st, const float* src, uint32_t in_stride, uint32_t s0, uint32_t n);
     vsb_status remove(const uint64_t* k, uint64_t n, uint64_t* removed);
     vsb_status compact(bool keep_graph);
     vsb_status build();
@@ -413,30 +488,28 @@ struct vsb_index {
     vsb_status sample_seeds(uint32_t n_rows, bool ensure_reach = true);
 
     // search building blocks: run on stream `s` with scratch `sc` against view `v`
-    vsb_status exact_block(const vsbi::View& v, vsbi::Scratch& sc, const vsb::RowsView& q, const vsb::RowsView& x,
-                           uint32_t x_lo, uint32_t x_hi, const uint32_t* deny_bm, const uint64_t* key_arr,
-                           const uint32_t* allow_bm, uint64_t allow_bits, const uint32_t* allow_of_q, uint32_t k,
-                           uint64_t* out_keys,
-                           float* out_dists, uint32_t* out_counts, uint64_t* out_packed, int64_t self_base,
-                           cudaStream_t s, bool approx_ok, const vsb::RowsView* shadow_q = nullptr,
-                           const vsb::RowsView* shadow_x = nullptr);
+    // the fixed inputs of an exact search of `q` over rows [x_lo, x_hi) of the view's store
+    vsb::ExactParams exact_in(const vsbi::View& v, const vsb::RowsView& q, uint32_t x_lo, uint32_t x_hi,
+                              const vsb::Allow& allow) const;
+    // exact top-k (K1 + K3) of `in`; shadow_q / shadow_x: bf16 copies for the candidate stage of an approx_ok block
+    vsb_status exact_block(vsbi::Scratch& sc, const vsb::ExactParams& in, uint32_t k, const vsbi::TopK& out, cudaStream_t s,
+                           bool approx_ok, const vsb::RowsView* shadow_q = nullptr, const vsb::RowsView* shadow_x = nullptr);
     struct GraphRun {
         uint32_t itopk = 64, max_iters = 0, n_seeds = 32, search_width = 1;
         bool count = false;  // instrumented launch (E / P counters)
         bool native = false; // ignore the traversal copies
-        const uint32_t* allow = nullptr;  // filtered ANN: bitmap over (key & 2^48-1)
-        uint64_t allow_bits = 0;
-        const uint32_t* allow_of_q = nullptr;  // [nb] bitmap index per query (null: bitmap 0)
+        bool timed = false;  // phase timing of the search path (t_begin / t_end)
+        vsb::Allow allow;    // filtered ANN
+        uint64_t* evals = nullptr;    // nullable: += distance evaluations
+        uint64_t* parents = nullptr;  // nullable: += parent expansions
     };
-    vsb_status graph_block(const vsbi::View& v, vsbi::Scratch& sc, const GraphRun& run, const vsb::RowsView& qv,
-                           uint32_t nb, uint32_t k, uint64_t* g_keys, float* g_dists, uint32_t* counts_out,
-                           uint64_t* packed_out, const vsb::RowsView* q16_in, cudaStream_t s, long long self_base,
-                           bool timed_phases, uint64_t* evals_out = nullptr, uint64_t* parents_out = nullptr);
+    // q16_in: bf16 copy of the queries if the caller already has one (corpus rows), else built here when needed
+    vsb_status graph_block(const vsbi::View& v, vsbi::Scratch& sc, const GraphRun& run, const vsb::RowsView& qv, uint32_t k,
+                           const vsbi::TopK& out, const vsb::RowsView* q16_in, cudaStream_t s);
     // one chunk of converted queries on one route: the graph (with the brute-force tail and the K8 merge) or the
-    // exact scan; allow_bm != null filters it (per query through allow_of_q)
-    vsb_status search_block(const vsbi::View& v, vsbi::Scratch& sc, const vsb::RowsView& qv, uint32_t nb, uint32_t k,
-                            uint64_t* o_keys, float* o_dists, uint32_t* o_counts, cudaStream_t s, bool graph,
-                            const uint32_t* allow_bm, uint64_t allow_bits, const uint32_t* allow_of_q);
+    // exact scan; allow filters it
+    vsb_status search_block(const vsbi::View& v, vsbi::Scratch& sc, const vsb::RowsView& qv, uint32_t k, const vsbi::TopK& out,
+                            cudaStream_t s, bool graph, const vsb::Allow& allow);
     vsb_status search_dev(const float* d_q, uint64_t nq, uint32_t k, uint64_t* d_keys, float* d_dists,
                           uint32_t* d_counts, cudaStream_t s, bool exact, const vsbi::Filters& f = vsbi::Filters());
     vsb_status search_host(const float* queries, uint64_t nq, uint32_t k, uint64_t* keys_out, float* dists_out,

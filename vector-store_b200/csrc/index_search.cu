@@ -9,30 +9,46 @@
 
 #include "index_impl.h"
 
+using vsbi::DevBuf;
 using vsbi::fail;
 using vsbi::round_up;
 using vsbi::Scratch;
+using vsbi::TopK;
 using vsbi::View;
 
-// exact top-k of the queries `q` against rows [x_lo, x_hi) of `x` (K1 + K3)
-vsb_status vsb_index::exact_block(const View& v, Scratch& sc, const vsb::RowsView& q, const vsb::RowsView& x, uint32_t x_lo,
-                                  uint32_t x_hi, const uint32_t* deny_bm, const uint64_t* key_arr, const uint32_t* allow_bm,
-                                  uint64_t allow_bits, const uint32_t* allow_of_q, uint32_t k, uint64_t* out_keys, float* out_dists,
-                                  uint32_t* out_counts, uint64_t* out_packed, int64_t self_base, cudaStream_t s,
-                                  bool approx_ok, const vsb::RowsView* shadow_q, const vsb::RowsView* shadow_x) {
-    (void)v;
+// the filter of queries map[0..n) of a block: their bitmap indices gathered into `fidx`
+static vsb_status gather_allow(const vsb::Allow& a, const uint32_t* map, uint32_t n, DevBuf& fidx, cudaStream_t s,
+                               vsb::Allow& out) {
+    out = a;
+    if (a.of_q == nullptr) return VSB_OK;
+    CU(fidx.ensure((size_t)n * 4));
+    vsb::launch_gather_u32(a.of_q, map, n, fidx.as<uint32_t>(), s);
+    out.of_q = fidx.as<uint32_t>();
+    return VSB_OK;
+}
+
+vsb::ExactParams vsb_index::exact_in(const View& v, const vsb::RowsView& q, uint32_t x_lo, uint32_t x_hi,
+                                     const vsb::Allow& allow) const {
     vsb::ExactParams p;
     p.storage = storage;
     p.metric = metric;
     p.q = q;
-    p.x = x;
+    p.x = v.st->rows.view(v.n_slots);
     p.x_lo = x_lo;
     p.x_hi = x_hi;
-    p.deny = deny_bm;
-    p.keys = key_arr;
-    p.allow = allow_bm;
-    p.allow_bits = allow_bits;
-    p.allow_of_q = allow_of_q;
+    p.deny = v.any_tombstone ? v.st->deny.as<uint32_t>() : nullptr;
+    p.keys = v.st->keys.as<uint64_t>();
+    p.allow = allow;
+    return p;
+}
+
+// exact top-k of the queries in.q against rows [in.x_lo, in.x_hi) of in.x (K1 + K3)
+vsb_status vsb_index::exact_block(Scratch& sc, const vsb::ExactParams& in, uint32_t k, const TopK& out, cudaStream_t s,
+                                  bool approx_ok, const vsb::RowsView* shadow_q, const vsb::RowsView* shadow_x) {
+    vsb::ExactParams p = in;
+    const vsb::RowsView& q = in.q;
+    const uint32_t x_lo = in.x_lo, x_hi = in.x_hi;
+    const int64_t self_base = out.self_base;
     const uint32_t extra = std::max<uint32_t>(16, k / 4) + (self_base >= 0 ? 1 : 0);
     p.kp = round_up(k + extra, 32);
     if (p.kp > 256) return fail(VSB_EINVAL, "k=%u too large for the exact path (max 200)", k);
@@ -65,7 +81,7 @@ vsb_status vsb_index::exact_block(const View& v, Scratch& sc, const vsb::RowsVie
         // without it (rows stored in the order of their clusters would do that).
         const uint32_t rows = x_hi - x_lo;
         const bool sampled = sampled_bounds && approx_ok && !certify && self_base >= 0 && rows >= 65536 && p.kp >= 64 &&
-                             p.n_splits == vsb::exact_tc_halves() && allow_bm == nullptr;
+                             p.n_splits == vsb::exact_tc_halves() && p.allow.bm == nullptr;
         if (sampled) {
             const uint32_t sample_tiles = 32, halves = vsb::exact_tc_halves();
             vsb::ExactParams ps = pc;
@@ -88,12 +104,7 @@ vsb_status vsb_index::exact_block(const View& v, Scratch& sc, const vsb::RowsVie
                 vsb::launch_tc_count_short(p.part, q.n, p.n_splits, p.kp, k + (self_base >= 0 ? 1u : 0u),
                                            sc.thr_cnt.as<uint32_t>(), s);
                 uint32_t n_short = 0;
-                {
-                    vsbi::HostReadback rb(sc.pin, s);
-                    CU(rb.reserve(4));
-                    CU(rb.copy(&n_short, sc.thr_cnt.p, 4));
-                    CU(rb.finish());
-                }
+                CU(vsbi::HostReadback::read(sc.pin, s, &n_short, sc.thr_cnt.p, 4));
                 if ((uint64_t)n_short * 50 > q.n) {
                     pc.thr_init = nullptr;
                     tc = vsb::launch_exact_candidates_tc(pc, s);
@@ -114,7 +125,7 @@ vsb_status vsb_index::exact_block(const View& v, Scratch& sc, const vsb::RowsVie
     }
     CU(cudaGetLastError());
     if (!certify) {
-        vsb::launch_exact_rerank(p, k, out_keys, out_dists, out_counts, out_packed, self_base, s);
+        vsb::launch_exact_rerank(p, k, out.keys, out.dists, out.counts, out.packed, self_base, s);
         CU(cudaGetLastError());
         return VSB_OK;
     }
@@ -124,7 +135,7 @@ vsb_status vsb_index::exact_block(const View& v, Scratch& sc, const vsb::RowsVie
     float* d_xmax = sc.cert_state.as<float>();
     uint32_t* d_count = sc.cert_state.as<uint32_t>() + 1;
     uint32_t* d_flags = sc.cert_state.as<uint32_t>() + 2;
-    vsb::launch_max_norm(x.nrm, x_lo, x_hi, d_xmax, s);
+    vsb::launch_max_norm(in.x.nrm, x_lo, x_hi, d_xmax, s);
     vsb::ExactCert cert;
     cert.x_nrm_max = d_xmax;
     cert.flags = d_flags;
@@ -139,58 +150,36 @@ vsb_status vsb_index::exact_block(const View& v, Scratch& sc, const vsb::RowsVie
 
     // flagged queries of one stage -> compact map (indices into the caller's query block) + gathered rows, and the
     // gathered bitmap index of each query (a filtered call whose queries carry their own bitmaps)
+    vsb::ExactParams pf = p;
     std::vector<uint32_t> map, flags;
     auto collect = [&](uint32_t n_stage, const std::vector<uint32_t>* prev) -> vsb_status {
         flags.resize(n_stage);
-        {
-            vsbi::HostReadback rb(sc.pin, s);
-            CU(rb.reserve((size_t)n_stage * 4));
-            CU(rb.copy(flags.data(), d_flags, (size_t)n_stage * 4));
-            CU(rb.finish());
-        }
+        CU(vsbi::HostReadback::read(sc.pin, s, flags.data(), d_flags, (size_t)n_stage * 4));
         std::vector<uint32_t> next;
         for (uint32_t i = 0; i < n_stage; ++i)
             if (flags[i]) next.push_back(prev ? (*prev)[i] : i);
         map.swap(next);
         const uint32_t nf = (uint32_t)map.size();
         CU(sc.fb_map.ensure((size_t)nf * 4));
-        CU(sc.fb_rows.ensure((size_t)nf * q.row_bytes));
-        CU(sc.fb_sq.ensure((size_t)nf * 4));
-        CU(sc.fb_nrm.ensure((size_t)nf * 4));
+        CU(sc.fb.ensure(nf, q.row_bytes));
         CU(cudaMemcpyAsync(sc.fb_map.p, map.data(), (size_t)nf * 4, cudaMemcpyHostToDevice, s));
-        vsb::launch_gather_rows(q.rows, q.row_bytes, q.sq, q.nrm, sc.fb_map.as<uint32_t>(), nf, sc.fb_rows.as<uint8_t>(),
-                                sc.fb_sq.as<float>(), sc.fb_nrm.as<float>(), s);
-        if (allow_of_q != nullptr) {
-            CU(sc.fb_fidx.ensure((size_t)nf * 4));
-            vsb::launch_gather_u32(allow_of_q, sc.fb_map.as<uint32_t>(), nf, sc.fb_fidx.as<uint32_t>(), s);
-        }
+        vsbi::gather_rows(q, sc.fb_map.as<uint32_t>(), nf, sc.fb, s);
+        ST(gather_allow(p.allow, sc.fb_map.as<uint32_t>(), nf, sc.fb_fidx, s, pf.allow));
+        pf.q = sc.fb.view(nf);
         CU(cudaStreamSynchronize(s));  // `map` is pageable and is rebuilt by the next stage
-        return VSB_OK;
-    };
-    auto read_count = [&](uint32_t* out) -> vsb_status {
-        vsbi::HostReadback rb(sc.pin, s);
-        CU(rb.reserve(4));
-        CU(rb.copy(out, d_count, 4));
-        CU(rb.finish());
         return VSB_OK;
     };
 
     CU(cudaMemsetAsync(d_count, 0, 4, s));
-    vsb::launch_exact_rerank(p, k, out_keys, out_dists, out_counts, out_packed, self_base, s, &cert);
+    vsb::launch_exact_rerank(p, k, out.keys, out.dists, out.counts, out.packed, self_base, s, &cert);
     CU(cudaGetLastError());
     uint32_t n_flagged = 0;
-    ST(read_count(&n_flagged));
+    CU(vsbi::HostReadback::read(sc.pin, s, &n_flagged, d_count, 4));
     cert_ok += q.n - n_flagged;
     cert_fallback += n_flagged;
     if (n_flagged == 0) return VSB_OK;
     ST(collect(q.n, nullptr));
 
-    vsb::ExactParams pf = p;
-    pf.q.rows = sc.fb_rows.as<uint8_t>();
-    pf.q.sq = sc.fb_sq.as<float>();
-    pf.q.nrm = sc.fb_nrm.as<float>();
-    pf.q.n = (uint32_t)map.size();
-    if (allow_of_q != nullptr) pf.allow_of_q = sc.fb_fidx.as<uint32_t>();
     if (tc && storage == VSB_F32) {
         // second stage: full fp32 products on the SIMT tiles, same certificate with the fp32 bound
         pf.kp = kp_simt;
@@ -201,14 +190,13 @@ vsb_status vsb_index::exact_block(const View& v, Scratch& sc, const vsb::RowsVie
         CU(cudaGetLastError());
         cert.rel = rel_fp32;
         CU(cudaMemsetAsync(d_count, 0, 4, s));
-        vsb::launch_exact_rerank(pf, k, out_keys, out_dists, out_counts, out_packed, self_base, s, &cert,
+        vsb::launch_exact_rerank(pf, k, out.keys, out.dists, out.counts, out.packed, self_base, s, &cert,
                                  sc.fb_map.as<uint32_t>());
         CU(cudaGetLastError());
-        ST(read_count(&n_flagged));
+        CU(vsbi::HostReadback::read(sc.pin, s, &n_flagged, d_count, 4));
         if (n_flagged == 0) return VSB_OK;
         const std::vector<uint32_t> prev = map;
         ST(collect(pf.q.n, &prev));
-        pf.q.n = (uint32_t)map.size();
     }
 
     // last stage: canonical scan of the whole block for what is left
@@ -222,23 +210,22 @@ vsb_status vsb_index::exact_block(const View& v, Scratch& sc, const vsb::RowsVie
     vsb::launch_exact_scan(pf, k, s);
     CU(cudaGetLastError());
     pf.n_splits = lists;
-    vsb::launch_exact_rerank(pf, k, out_keys, out_dists, out_counts, out_packed, self_base, s, nullptr,
+    vsb::launch_exact_rerank(pf, k, out.keys, out.dists, out.counts, out.packed, self_base, s, nullptr,
                              sc.fb_map.as<uint32_t>());
     CU(cudaGetLastError());
     return VSB_OK;
 }
 
-// Seeds + K4 (+ K3 re-rank on the bf16-traversal path) for `nb` converted queries `qv`.
-//   g_keys/g_dists/counts_out : user-facing top-k (nullable when packed_out is used)
-//   packed_out                : raw K4 list (packed ord(dist)<<32|slot, [nb][k]) — used by the streaming insert
-//   q16_in                    : bf16 copy of the queries if the caller already has one (corpus rows), else built here
-vsb_status vsb_index::graph_block(const View& v, Scratch& sc, const GraphRun& run, const vsb::RowsView& qv, uint32_t nb,
-                                  uint32_t k, uint64_t* g_keys, float* g_dists, uint32_t* counts_out, uint64_t* packed_out,
-                                  const vsb::RowsView* q16_in, cudaStream_t s, long long self_base, bool tp,
-                                  uint64_t* evals_out, uint64_t* parents_out) {
+// Seeds + K4 (+ K3 re-rank on the bf16-traversal path) for the converted queries `qv`.  out.packed: the raw K4 list
+// ([n][k], used by the streaming insert and the refinement) instead of the user-facing top-k.
+vsb_status vsb_index::graph_block(const View& v, Scratch& sc, const GraphRun& run, const vsb::RowsView& qv, uint32_t k,
+                                  const TopK& out, const vsb::RowsView* q16_in, cudaStream_t s) {
     const vsbi::Store& st = *v.st;
     const vsbi::Seeds& sd = *v.sd;
-    const vsb::RowsView x = rows_view(v);
+    const vsb::RowsView x = st.rows.view(v.n_slots);
+    const uint32_t nb = qv.n;
+    const bool tp = run.timed;
+    uint64_t* packed_out = out.packed;
     const uint32_t* deny_bm = v.any_tombstone ? st.deny.as<uint32_t>() : nullptr;
     // the traversal copies serve searches; `native` (a runtime override, searches only) walks the stored rows instead
     const bool t16 = trav16 && !(run.native && packed_out == nullptr);
@@ -247,7 +234,7 @@ vsb_status vsb_index::graph_block(const View& v, Scratch& sc, const GraphRun& ru
     // order, exactly like the results of the bf16 / int8 traversal copies (the build only needs the ranking)
     const int trav_storage = t16 ? (int)VSB_BF16 : storage;
     const bool use8_early = trav8 && t16 && packed_out == nullptr;
-    const bool mma = !use8_early && vsb::graph_search_uses_mma(trav_storage, nb, run.allow != nullptr, std::max(run.itopk, k));
+    const bool mma = !use8_early && vsb::graph_search_uses_mma(trav_storage, nb, run.allow.bm != nullptr, std::max(run.itopk, k));
     const bool rerank = (t16 || mma) && packed_out == nullptr;
     // ---- bf16 shadow of the queries (f32 storage: tensor-core seed layer and/or bf16 traversal) ----
     bool seed_tc = tc_enabled && vsb::exact_tc_supported(storage, metric) && nb >= 16;
@@ -255,28 +242,18 @@ vsb_status vsb_index::graph_block(const View& v, Scratch& sc, const GraphRun& ru
     if (q16_in != nullptr) {
         q16v = *q16_in;
     } else if (storage == VSB_F32 && (seed_tc || t16)) {
-        CU(sc.q16_rows.ensure((size_t)nb * row_bytes16));
-        CU(sc.q16_sq.ensure((size_t)nb * 4));
-        CU(sc.q16_nrm.ensure((size_t)nb * 4));
-        vsb::launch_convert_rows(VSB_BF16, reinterpret_cast<const float*>(qv.rows), nb, row_bytes / 4, sc.q16_rows.as<uint8_t>(),
-                                 row_bytes16, sc.q16_sq.as<float>(), sc.q16_nrm.as<float>(), s);
+        CU(sc.q16.ensure(nb, row_bytes16));
+        vsb::launch_convert_rows(VSB_BF16, reinterpret_cast<const float*>(qv.rows), nb, row_bytes / 4, sc.q16.rows.as<uint8_t>(),
+                                 row_bytes16, sc.q16.sq.as<float>(), sc.q16.nrm.as<float>(), s);
         CU(cudaGetLastError());
-        q16v.rows = sc.q16_rows.as<uint8_t>();
-        q16v.sq = sc.q16_sq.as<float>();
-        q16v.nrm = sc.q16_nrm.as<float>();
-        q16v.row_bytes = row_bytes16;
-        q16v.n = nb;
+        q16v = sc.q16.view(nb);
     }
     // ---- seed layer: distances to the contiguous entry-point sample ----
     vsb::ExactParams sp;
     sp.storage = storage;
     sp.metric = metric;
     sp.q = qv;
-    sp.x.rows = sd.rows.as<uint8_t>();
-    sp.x.sq = sd.sq.as<float>();
-    sp.x.nrm = sd.nrm.as<float>();
-    sp.x.row_bytes = row_bytes;
-    sp.x.n = sd.n;
+    sp.x = sd.rows.view(sd.n);
     sp.x_lo = 0;
     sp.x_hi = sd.n;
     sp.keys = nullptr;  // ties fall back to the seed index (LessByKey with null keys)
@@ -289,10 +266,7 @@ vsb_status vsb_index::graph_block(const View& v, Scratch& sc, const GraphRun& ru
         if (storage == VSB_F32) {
             sp.storage = VSB_BF16;
             sp.q = q16v;
-            sp.x.rows = sd.rows16.as<uint8_t>();
-            sp.x.sq = sd.sq16.as<float>();
-            sp.x.nrm = sd.nrm16.as<float>();
-            sp.x.row_bytes = row_bytes16;
+            sp.x = sd.bf16.view(sd.n);
         }
     } else {
         sp.n_splits = vsb::exact_pick_splits(nb, sd.n, sm_count);
@@ -327,31 +301,16 @@ vsb_status vsb_index::graph_block(const View& v, Scratch& sc, const GraphRun& ru
     gp.storage = t16 ? VSB_BF16 : storage;
     gp.metric = metric;
     gp.q = t16 ? q16v : qv;
-    gp.x = x;
-    if (t16) {
-        gp.x.rows = st.rows16.as<uint8_t>();
-        gp.x.sq = st.sq16.as<float>();
-        gp.x.nrm = st.nrm16.as<float>();
-        gp.x.row_bytes = row_bytes16;
-    }
+    gp.x = t16 ? st.bf16.view(v.n_slots) : x;
     const bool use8 = trav8 && rerank;  // searches only: the build keeps the bf16 traversal
     if (use8) {
-        CU(sc.q8_rows.ensure((size_t)nb * row_bytes8));
-        CU(sc.q8_sq.ensure((size_t)nb * 4));
-        CU(sc.q8_nrm.ensure((size_t)nb * 4));
-        vsb::launch_convert_rows_i8s(reinterpret_cast<const float*>(qv.rows), nb, dim, row_bytes / 4, sc.q8_rows.as<uint8_t>(),
-                                     row_bytes8, sc.q8_sq.as<float>(), sc.q8_nrm.as<float>(), s);
+        CU(sc.q8.ensure(nb, row_bytes8));
+        vsb::launch_convert_rows_i8s(reinterpret_cast<const float*>(qv.rows), nb, dim, row_bytes / 4, sc.q8.rows.as<uint8_t>(),
+                                     row_bytes8, sc.q8.sq.as<float>(), sc.q8.nrm.as<float>(), s);
         CU(cudaGetLastError());
         gp.storage = VSB_I8;
-        gp.q.rows = sc.q8_rows.as<uint8_t>();
-        gp.q.sq = sc.q8_sq.as<float>();
-        gp.q.nrm = sc.q8_nrm.as<float>();
-        gp.q.row_bytes = row_bytes8;
-        gp.q.n = nb;
-        gp.x.rows = st.rows8.as<uint8_t>();
-        gp.x.sq = st.sq8.as<float>();
-        gp.x.nrm = st.nrm8.as<float>();
-        gp.x.row_bytes = row_bytes8;
+        gp.q = sc.q8.view(nb);
+        gp.x = st.i8.view(v.n_slots);
     }
     gp.graph = v.gr->g.as<uint32_t>();
     gp.graph_stride = graph_stride;
@@ -367,13 +326,11 @@ vsb_status vsb_index::graph_block(const View& v, Scratch& sc, const GraphRun& ru
     gp.max_iters = run.max_iters;
     gp.search_width = run.search_width;
     gp.k = k;
-    gp.out_keys = g_keys;
-    gp.out_dists = g_dists;
-    gp.out_counts = counts_out;
-    gp.self_base = self_base;
+    gp.out_keys = out.keys;
+    gp.out_dists = out.dists;
+    gp.out_counts = out.counts;
+    gp.self_base = out.self_base;
     gp.allow = run.allow;
-    gp.allow_bits = run.allow_bits;
-    gp.allow_of_q = run.allow_of_q;
     gp.mma = mma;
     uint32_t kr = 0;
     if (packed_out != nullptr) {
@@ -395,7 +352,7 @@ vsb_status vsb_index::graph_block(const View& v, Scratch& sc, const GraphRun& ru
         gp.out_packed = sc.rr_packed.as<uint64_t>();
         gp.out_counts = nullptr;
     }
-    const bool count = run.count || evals_out != nullptr;
+    const bool count = run.count || run.evals != nullptr;
     if (count) {
         CU(sc.counters.ensure(16));
         CU(cudaMemsetAsync(sc.counters.p, 0, 16, s));
@@ -416,20 +373,15 @@ vsb_status vsb_index::graph_block(const View& v, Scratch& sc, const GraphRun& ru
         rp.kp = kr;
         rp.n_splits = 1;
         if (tp) t_begin(PH_EXACT, s);
-        vsb::launch_exact_rerank(rp, k, g_keys, g_dists, counts_out, nullptr, -1, s);
+        vsb::launch_exact_rerank(rp, k, out.keys, out.dists, out.counts, nullptr, -1, s);
         if (tp) t_end(s);
         CU(cudaGetLastError());
     }
     if (count) {
         unsigned long long h[2];
-        {
-            vsbi::HostReadback rb(sc.pin, s);  // pinned staging: see index_impl.h (a pageable read-back stalls every search)
-            CU(rb.reserve(16));
-            CU(rb.copy(h, sc.counters.p, 16));
-            CU(rb.finish());
-        }
-        if (evals_out) *evals_out += h[0];
-        if (parents_out) *parents_out += h[1];
+        CU(vsbi::HostReadback::read(sc.pin, s, h, sc.counters.p, 16));
+        if (run.evals) *run.evals += h[0];
+        if (run.parents) *run.parents += h[1];
         if (run.count) {
             last_evals = h[0];
             last_parents = h[1];
@@ -439,12 +391,12 @@ vsb_status vsb_index::graph_block(const View& v, Scratch& sc, const GraphRun& ru
     return VSB_OK;
 }
 
-vsb_status vsb_index::search_block(const View& v, Scratch& sc, const vsb::RowsView& qv, uint32_t nb, uint32_t k,
-                                    uint64_t* o_keys, float* o_dists, uint32_t* o_counts, cudaStream_t s, bool graph,
-                                    const uint32_t* allow_bm, uint64_t allow_bits, const uint32_t* allow_of_q) {
-    const vsbi::Store& st = *v.st;
-    const vsb::RowsView x = rows_view(v);
-    const uint32_t* deny_bm = v.any_tombstone ? st.deny.as<uint32_t>() : nullptr;
+vsb_status vsb_index::search_block(const View& v, Scratch& sc, const vsb::RowsView& qv, uint32_t k, const TopK& out,
+                                    cudaStream_t s, bool graph, const vsb::Allow& allow) {
+    const uint32_t nb = qv.n;
+    uint64_t* o_keys = out.keys;
+    float* o_dists = out.dists;
+    uint32_t* o_counts = out.counts;
     const bool use_graph = graph && v.n_graphed > 0 && k <= 1024;
     const uint32_t tail_lo = use_graph ? v.n_graphed : 0, tail_hi = v.n_slots;
     const bool have_tail = tail_hi > tail_lo;
@@ -470,30 +422,36 @@ vsb_status vsb_index::search_block(const View& v, Scratch& sc, const vsb::RowsVi
         run.search_width = search_width;
         run.count = instrumented;
         run.native = native_traversal;
-        run.allow = allow_bm;
-        run.allow_bits = allow_bits;
-        run.allow_of_q = allow_of_q;
-        ST(graph_block(v, sc, run, qv, nb, k, g_keys, g_dists, have_tail ? nullptr : o_counts, nullptr, nullptr, s, -1, true));
+        run.timed = true;
+        run.allow = allow;
+        TopK g;
+        g.keys = g_keys;
+        g.dists = g_dists;
+        g.counts = have_tail ? nullptr : o_counts;
+        ST(graph_block(v, sc, run, qv, k, g, nullptr, s));
     }
     if (have_tail) {
         t_begin(PH_EXACT, s);
+        const vsb::ExactParams tail = exact_in(v, qv, tail_lo, tail_hi, allow);
         vsb_status est;
         if (k_tail == k) {
-            est = exact_block(v, sc, qv, x, tail_lo, tail_hi, deny_bm, st.keys.as<uint64_t>(), allow_bm, allow_bits, allow_of_q,
-                              k, t_keys, t_dists, use_graph ? nullptr : o_counts, nullptr, -1, s,
-                              /*approx_ok=*/use_graph);  // the ANN tail needs no certificate (no host sync)
+            TopK t;
+            t.keys = t_keys;
+            t.dists = t_dists;
+            t.counts = use_graph ? nullptr : o_counts;
+            est = exact_block(sc, tail, k, t, s, /*approx_ok=*/use_graph);  // the ANN tail needs no certificate (no host sync)
         } else {
             // k > 200 with a tail: the tail's best 200 rows, laid out with stride k so that K8 can merge them
             vsb::launch_fill_empty(t_keys, t_dists, nullptr, nb, k, s);
-            vsbi::DevBuf& tk = sc.fb_rows;  // scratch that the ANN path does not otherwise touch
+            DevBuf& tk = sc.fb.rows;  // scratch that the ANN path does not otherwise touch
             CU(tk.ensure((size_t)nb * k_tail * 12));
-            uint64_t* ck = tk.as<uint64_t>();
-            float* cd = reinterpret_cast<float*>(ck + (size_t)nb * k_tail);
-            est = exact_block(v, sc, qv, x, tail_lo, tail_hi, deny_bm, st.keys.as<uint64_t>(), allow_bm, allow_bits, allow_of_q,
-                              k_tail, ck, cd, nullptr, nullptr, -1, s, true);
+            TopK c;
+            c.keys = tk.as<uint64_t>();
+            c.dists = reinterpret_cast<float*>(c.keys + (size_t)nb * k_tail);
+            est = exact_block(sc, tail, k_tail, c, s, true);
             if (est == VSB_OK) {
-                CU(cudaMemcpy2DAsync(t_keys, (size_t)k * 8, ck, (size_t)k_tail * 8, (size_t)k_tail * 8, nb, cudaMemcpyDeviceToDevice, s));
-                CU(cudaMemcpy2DAsync(t_dists, (size_t)k * 4, cd, (size_t)k_tail * 4, (size_t)k_tail * 4, nb, cudaMemcpyDeviceToDevice, s));
+                CU(cudaMemcpy2DAsync(t_keys, (size_t)k * 8, c.keys, (size_t)k_tail * 8, (size_t)k_tail * 8, nb, cudaMemcpyDeviceToDevice, s));
+                CU(cudaMemcpy2DAsync(t_dists, (size_t)k * 4, c.dists, (size_t)k_tail * 4, (size_t)k_tail * 4, nb, cudaMemcpyDeviceToDevice, s));
             }
         }
         t_end(s);
@@ -520,10 +478,11 @@ vsb_status vsb_index::search_dev(const float* d_q, uint64_t nq, uint32_t k, uint
     const View v = snapshot();
     ST(begin_search(s));
     Scratch& sc = ss;
+    const bool filtered = f.allow.bm != nullptr;
     // filtered search, per bitmap: graph traversal with the bitmap unless too few rows are admissible (then the exact
     // scan wins).  Queries whose bitmaps take different routes are split by route below.
-    std::vector<uint8_t> graph_of_filter(f.d_allow != nullptr ? f.n : 0, 0);
-    if (f.d_allow != nullptr && !exact && v.n_graphed > 0 && k <= 256) {
+    std::vector<uint8_t> graph_of_filter(filtered ? f.n : 0, 0);
+    if (filtered && !exact && v.n_graphed > 0 && k <= 256) {
         const uint64_t live_rows = live_atomic.load();
         for (uint32_t i = 0; i < f.n; ++i)
             graph_of_filter[i] = f.pop[i] * 100 >= (uint64_t)filter_min_pct * std::max<uint64_t>(live_rows, 1) && filter_min_pct <= 100;
@@ -531,73 +490,58 @@ vsb_status vsb_index::search_dev(const float* d_q, uint64_t nq, uint32_t k, uint
     const uint64_t QCHUNK = 65536;
     for (uint64_t q0 = 0; q0 < nq; q0 += QCHUNK) {
         const uint32_t nb = (uint32_t)std::min<uint64_t>(QCHUNK, nq - q0);
-        uint64_t* o_keys = d_keys + q0 * k;
-        float* o_dists = d_dists + q0 * k;
-        uint32_t* o_counts = d_counts ? d_counts + q0 : nullptr;
+        TopK o;
+        o.keys = d_keys + q0 * k;
+        o.dists = d_dists + q0 * k;
+        o.counts = d_counts ? d_counts + q0 : nullptr;
         if (v.n_slots == 0) {
-            vsb::launch_fill_empty(o_keys, o_dists, o_counts, nb, k, s);
+            vsb::launch_fill_empty(o.keys, o.dists, o.counts, nb, k, s);
             CU(cudaGetLastError());
             continue;
         }
-        CU(sc.q_rows.ensure((size_t)nb * row_bytes));
-        CU(sc.q_sq.ensure((size_t)nb * 4));
-        CU(sc.q_nrm.ensure((size_t)nb * 4));
+        CU(sc.q.ensure(nb, row_bytes));
         t_begin(PH_CONVERT, s);
-        vsb::launch_convert_rows(storage, d_q + q0 * dim, nb, dim, sc.q_rows.as<uint8_t>(), row_bytes, sc.q_sq.as<float>(),
-                                 sc.q_nrm.as<float>(), s);
+        vsb::launch_convert_rows(storage, d_q + q0 * dim, nb, dim, sc.q.rows.as<uint8_t>(), row_bytes, sc.q.sq.as<float>(),
+                                 sc.q.nrm.as<float>(), s);
         t_end(s);
         CU(cudaGetLastError());
-        vsb::RowsView qv;
-        qv.rows = sc.q_rows.as<uint8_t>();
-        qv.sq = sc.q_sq.as<float>();
-        qv.nrm = sc.q_nrm.as<float>();
-        qv.row_bytes = row_bytes;
-        qv.n = nb;
-        if (f.d_allow == nullptr) {
-            ST(search_block(v, sc, qv, nb, k, o_keys, o_dists, o_counts, s, !exact, nullptr, 0, nullptr));
+        const vsb::RowsView qv = sc.q.view(nb);
+        if (!filtered) {
+            ST(search_block(v, sc, qv, k, o, s, !exact, vsb::Allow{}));
             continue;
         }
-        const uint32_t* c_fidx = f.d_fidx ? f.d_fidx + q0 : nullptr;  // this chunk's bitmap indices
+        const vsb::Allow c_allow = f.allow.from(q0);  // this chunk's bitmap indices
         // route of each query of the chunk: by_route[1] = graph, by_route[0] = exact scan
         std::vector<uint32_t> by_route[2];
         for (uint32_t i = 0; i < nb; ++i) by_route[graph_of_filter[f.h_fidx ? f.h_fidx[q0 + i] : 0]].push_back(i);
         if (by_route[0].empty() || by_route[1].empty()) {
-            ST(search_block(v, sc, qv, nb, k, o_keys, o_dists, o_counts, s, by_route[0].empty(), f.d_allow, f.bits, c_fidx));
+            ST(search_block(v, sc, qv, k, o, s, by_route[0].empty(), c_allow));
             continue;
         }
         // mixed routes: each route runs on a compact block of its own queries (rows and bitmap indices gathered like
         // the certificate fallback's), and its [n][k] results are scattered back to the caller's rows
         const uint32_t n_max = (uint32_t)std::max(by_route[0].size(), by_route[1].size());
         CU(sc.rt_map.ensure((size_t)nb * 4));
-        CU(sc.rt_rows.ensure((size_t)n_max * row_bytes));
-        CU(sc.rt_sq.ensure((size_t)n_max * 4));
-        CU(sc.rt_nrm.ensure((size_t)n_max * 4));
+        CU(sc.rt.ensure(n_max, row_bytes));
         CU(sc.rt_fidx.ensure((size_t)n_max * 4));
         CU(sc.rt_keys.ensure((size_t)n_max * k * 8));
         CU(sc.rt_dists.ensure((size_t)n_max * k * 4));
         CU(sc.rt_counts.ensure((size_t)n_max * 4));
+        TopK r_out;
+        r_out.keys = sc.rt_keys.as<uint64_t>();
+        r_out.dists = sc.rt_dists.as<float>();
+        r_out.counts = sc.rt_counts.as<uint32_t>();
         uint32_t* d_map[2] = {sc.rt_map.as<uint32_t>(), sc.rt_map.as<uint32_t>() + by_route[0].size()};
         CU(cudaMemcpyAsync(d_map[0], by_route[0].data(), by_route[0].size() * 4, cudaMemcpyHostToDevice, s));
         CU(cudaMemcpyAsync(d_map[1], by_route[1].data(), by_route[1].size() * 4, cudaMemcpyHostToDevice, s));
         for (int r = 1; r >= 0; --r) {
             const uint32_t n = (uint32_t)by_route[r].size();
-            vsb::launch_gather_rows(qv.rows, row_bytes, qv.sq, qv.nrm, d_map[r], n, sc.rt_rows.as<uint8_t>(),
-                                    sc.rt_sq.as<float>(), sc.rt_nrm.as<float>(), s);
-            const uint32_t* r_fidx = nullptr;
-            if (c_fidx != nullptr) {
-                vsb::launch_gather_u32(c_fidx, d_map[r], n, sc.rt_fidx.as<uint32_t>(), s);
-                r_fidx = sc.rt_fidx.as<uint32_t>();
-            }
+            vsbi::gather_rows(qv, d_map[r], n, sc.rt, s);
+            vsb::Allow r_allow;
+            ST(gather_allow(c_allow, d_map[r], n, sc.rt_fidx, s, r_allow));
             CU(cudaGetLastError());
-            vsb::RowsView rv = qv;
-            rv.rows = sc.rt_rows.as<uint8_t>();
-            rv.sq = sc.rt_sq.as<float>();
-            rv.nrm = sc.rt_nrm.as<float>();
-            rv.n = n;
-            ST(search_block(v, sc, rv, n, k, sc.rt_keys.as<uint64_t>(), sc.rt_dists.as<float>(), sc.rt_counts.as<uint32_t>(),
-                            s, r == 1, f.d_allow, f.bits, r_fidx));
-            vsb::launch_scatter_topk(sc.rt_keys.as<uint64_t>(), sc.rt_dists.as<float>(), sc.rt_counts.as<uint32_t>(), d_map[r],
-                                     n, k, o_keys, o_dists, o_counts, s);
+            ST(search_block(v, sc, sc.rt.view(n), k, r_out, s, r == 1, r_allow));
+            vsb::launch_scatter_topk(r_out.keys, r_out.dists, r_out.counts, d_map[r], n, k, o.keys, o.dists, o.counts, s);
             CU(cudaGetLastError());
         }
     }
@@ -605,31 +549,62 @@ vsb_status vsb_index::search_dev(const float* d_q, uint64_t nq, uint32_t k, uint
     return VSB_OK;
 }
 
-static uint64_t popcount_words(const uint32_t* w, size_t n_words, uint64_t bits) {
-    uint64_t c = 0;
-    const size_t full = (size_t)(bits / 32);
-    for (size_t i = 0; i < full && i < n_words; ++i) c += (uint64_t)__builtin_popcount(w[i]);
-    if (bits % 32 && full < n_words) c += (uint64_t)__builtin_popcount(w[full] & ((1u << (bits % 32)) - 1));
-    return c;
+namespace vsbi {
+
+std::vector<uint64_t> filter_population(const HostFilters& hf) {
+    std::vector<uint64_t> pop(hf.bitmaps ? hf.n : 0, 0);
+    const size_t words = (size_t)((hf.bits + 31) / 32), full = (size_t)(hf.bits / 32);
+    for (size_t f = 0; f < pop.size(); ++f) {
+        const uint32_t* w = hf.bitmaps + f * words;
+        for (size_t i = 0; i < full; ++i) pop[f] += (uint64_t)__builtin_popcount(w[i]);
+        if (hf.bits % 32) pop[f] += (uint64_t)__builtin_popcount(w[full] & ((1u << (hf.bits % 32)) - 1));
+    }
+    return pop;
 }
 
-// Uploads the bitmaps of a filtered call (one copy of the whole block) on `s`, points `f` at them and counts each
-// bitmap's admissible rows for the route selection; the per-query indices are the caller's to upload (d_fidx).
-static vsb_status upload_filters(vsbi::Scratch& sc, const vsbi::HostFilters& hf, cudaStream_t s, std::vector<uint64_t>& pop,
-                                 vsbi::Filters& f) {
+vsb_status upload_filters(Scratch& sc, const HostFilters& hf, const uint64_t* pop, const uint32_t* d_fidx, cudaStream_t s,
+                          Filters& f) {
     if (hf.bitmaps == nullptr) return VSB_OK;
-    const size_t words = (size_t)((hf.bits + 31) / 32);
-    CU(sc.allow.ensure(std::max<size_t>((size_t)hf.n * words * 4, 16)));
-    CU(cudaMemcpyAsync(sc.allow.p, hf.bitmaps, (size_t)hf.n * words * 4, cudaMemcpyHostToDevice, s));
-    pop.resize(hf.n);
-    for (uint32_t i = 0; i < hf.n; ++i) pop[i] = popcount_words(hf.bitmaps + (size_t)i * words, words, hf.bits);
-    f.d_allow = sc.allow.as<uint32_t>();
-    f.bits = hf.bits;
+    const size_t bytes = (size_t)hf.n * ((hf.bits + 31) / 32) * 4;
+    CU(sc.allow.ensure(std::max<size_t>(bytes, 16)));
+    CU(cudaMemcpyAsync(sc.allow.p, hf.bitmaps, bytes, cudaMemcpyHostToDevice, s));
+    f.allow = vsb::Allow{sc.allow.as<uint32_t>(), hf.bits, d_fidx};
     f.n = hf.n;
     f.h_fidx = hf.of_query;
-    f.pop = pop.data();
+    f.pop = pop;
     return VSB_OK;
 }
+
+cudaError_t Staging::carve(DevBuf& buf, size_t q_bytes, uint64_t nq, uint32_t k, bool with_fidx) {
+    auto al = [](size_t v) { return (v + 255) / 256 * 256; };
+    keys_bytes = (size_t)nq * k * 8;
+    dists_bytes = (size_t)nq * k * 4;
+    counts_bytes = (size_t)nq * 4;
+    const size_t fidx_bytes = with_fidx ? (size_t)nq * 4 : 0;
+    const cudaError_t e = buf.ensure(al(q_bytes) + al(keys_bytes) + al(dists_bytes) + al(counts_bytes) + al(fidx_bytes));
+    if (e != cudaSuccess) return e;
+    uint8_t* p = buf.as<uint8_t>();
+    q = q_bytes ? reinterpret_cast<float*>(p) : nullptr;
+    keys = reinterpret_cast<uint64_t*>(p += al(q_bytes));
+    dists = reinterpret_cast<float*>(p += al(keys_bytes));
+    counts = reinterpret_cast<uint32_t*>(p += al(dists_bytes));
+    fidx = with_fidx ? reinterpret_cast<uint32_t*>(p + al(counts_bytes)) : nullptr;
+    return cudaSuccess;
+}
+
+cudaError_t Staging::read(PinBuf& pin, cudaStream_t s, uint64_t* keys_out, float* dists_out, uint32_t* counts_out) const {
+    auto al = [](size_t v) { return (v + 255) / 256 * 256; };
+    HostReadback rb(pin, s);
+    cudaError_t e = cudaSuccess;
+    if (!host_is_pinned(keys_out) || !host_is_pinned(dists_out) || (counts_out && !host_is_pinned(counts_out)))
+        e = rb.reserve(al(keys_bytes) + al(dists_bytes) + al(counts_bytes));
+    if (e == cudaSuccess) e = rb.copy(keys_out, keys, keys_bytes);
+    if (e == cudaSuccess) e = rb.copy(dists_out, dists, dists_bytes);
+    if (e == cudaSuccess && counts_out) e = rb.copy(counts_out, counts, counts_bytes);
+    return e == cudaSuccess ? rb.finish() : e;
+}
+
+}  // namespace vsbi
 
 vsb_status vsb_index::search_host(const float* queries, uint64_t nq, uint32_t k, uint64_t* keys_out,
                                   float* dists_out, uint32_t* counts_out, bool exact, const vsbi::HostFilters& hf) {
@@ -637,12 +612,9 @@ vsb_status vsb_index::search_host(const float* queries, uint64_t nq, uint32_t k,
     if (k == 0) return fail(VSB_EINVAL, "k must be > 0");
     if (queries == nullptr || keys_out == nullptr || dists_out == nullptr) return fail(VSB_EINVAL, "null buffer");
     const size_t in_bytes = (size_t)nq * dim * 4;
-    const size_t keys_bytes = (size_t)nq * k * 8, dists_bytes = (size_t)nq * k * 4, counts_bytes = (size_t)nq * 4;
-    // per-query bitmap indices travel with the queries
-    const size_t fidx_bytes = hf.of_query != nullptr ? (size_t)nq * 4 : 0;
-    auto al = [](size_t v) { return (v + 255) / 256 * 256; };
-    std::vector<uint64_t> pop;
+    const std::vector<uint64_t> pop = vsbi::filter_population(hf);
     vsbi::Filters f;
+    vsbi::Staging st;  // per-query bitmap indices travel with the queries
     if (nq >= 1024) {
         // Large batches are PIPELINED across concurrent callers (the reference serves ann requests from a worker
         // pool, worker.rs:44-118): each call takes one of two staging slots, uploads its queries on the slot's copy
@@ -671,58 +643,30 @@ vsb_status vsb_index::search_host(const float* queries, uint64_t nq, uint32_t k,
             CU(cudaEventCreateWithFlags(&sl.ev_in, cudaEventDisableTiming));
             CU(cudaEventCreateWithFlags(&sl.ev_done, cudaEventDisableTiming));
         }
-        CU(sl.buf.ensure(al(in_bytes) + al(keys_bytes) + al(dists_bytes) + al(counts_bytes) + al(fidx_bytes)));
-        uint8_t* base = sl.buf.as<uint8_t>();
-        float* dq = reinterpret_cast<float*>(base);
-        uint64_t* dk = reinterpret_cast<uint64_t*>(base + al(in_bytes));
-        float* dd = reinterpret_cast<float*>(base + al(in_bytes) + al(keys_bytes));
-        uint32_t* dc = reinterpret_cast<uint32_t*>(base + al(in_bytes) + al(keys_bytes) + al(dists_bytes));
-        uint32_t* dfi = reinterpret_cast<uint32_t*>(base + al(in_bytes) + al(keys_bytes) + al(dists_bytes) + al(counts_bytes));
-        CU(cudaMemcpyAsync(dq, queries, in_bytes, cudaMemcpyHostToDevice, sl.cs));
-        if (fidx_bytes) CU(cudaMemcpyAsync(dfi, hf.of_query, fidx_bytes, cudaMemcpyHostToDevice, sl.cs));
+        CU(st.carve(sl.buf, in_bytes, nq, k, hf.of_query != nullptr));
+        CU(cudaMemcpyAsync(st.q, queries, in_bytes, cudaMemcpyHostToDevice, sl.cs));
+        if (st.fidx) CU(cudaMemcpyAsync(st.fidx, hf.of_query, (size_t)nq * 4, cudaMemcpyHostToDevice, sl.cs));
         CU(cudaEventRecord(sl.ev_in, sl.cs));
         {
             std::lock_guard<std::mutex> g(search_mu);
-            ST(upload_filters(ss, hf, stream, pop, f));
-            if (fidx_bytes) f.d_fidx = dfi;
+            ST(vsbi::upload_filters(ss, hf, pop.data(), st.fidx, stream, f));
             CU(cudaStreamWaitEvent(stream, sl.ev_in, 0));
-            ST(search_dev(dq, nq, k, dk, dd, dc, stream, exact, f));
+            ST(search_dev(st.q, nq, k, st.keys, st.dists, st.counts, stream, exact, f));
             CU(cudaEventRecord(sl.ev_done, stream));
         }
         CU(cudaStreamWaitEvent(sl.cs, sl.ev_done, 0));
-        vsbi::HostReadback rb(sl.pin, sl.cs);
-        if (!vsbi::host_is_pinned(keys_out) || !vsbi::host_is_pinned(dists_out) || (counts_out && !vsbi::host_is_pinned(counts_out)))
-            CU(rb.reserve(al(keys_bytes) + al(dists_bytes) + al(counts_bytes)));
-        CU(rb.copy(keys_out, dk, keys_bytes));
-        CU(rb.copy(dists_out, dd, dists_bytes));
-        if (counts_out) CU(rb.copy(counts_out, dc, counts_bytes));
-        CU(rb.finish());
+        CU(st.read(sl.pin, sl.cs, keys_out, dists_out, counts_out));
         return VSB_OK;
     }
     std::lock_guard<std::mutex> g(search_mu);
     CU(cudaSetDevice(device));
     ST(begin_search(stream));
-    vsbi::DevBuf& d_in = ss.q_in;
-    CU(d_in.ensure(al(in_bytes) + al(keys_bytes) + al(dists_bytes) + al(counts_bytes) + al(fidx_bytes)));
-    uint8_t* base = d_in.as<uint8_t>();
-    float* dq = reinterpret_cast<float*>(base);
-    uint64_t* dk = reinterpret_cast<uint64_t*>(base + al(in_bytes));
-    float* dd = reinterpret_cast<float*>(base + al(in_bytes) + al(keys_bytes));
-    uint32_t* dc = reinterpret_cast<uint32_t*>(base + al(in_bytes) + al(keys_bytes) + al(dists_bytes));
-    uint32_t* dfi = reinterpret_cast<uint32_t*>(base + al(in_bytes) + al(keys_bytes) + al(dists_bytes) + al(counts_bytes));
-    CU(cudaMemcpyAsync(dq, queries, in_bytes, cudaMemcpyHostToDevice, stream));
-    if (fidx_bytes) {
-        CU(cudaMemcpyAsync(dfi, hf.of_query, fidx_bytes, cudaMemcpyHostToDevice, stream));
-        f.d_fidx = dfi;
-    }
-    ST(upload_filters(ss, hf, stream, pop, f));
-    ST(search_dev(dq, nq, k, dk, dd, dc, stream, exact, f));
-    vsbi::HostReadback rb(ss.pin, stream);
-    CU(rb.reserve(al(keys_bytes) + al(dists_bytes) + al(counts_bytes)));
-    CU(rb.copy(keys_out, dk, keys_bytes));
-    CU(rb.copy(dists_out, dd, dists_bytes));
-    if (counts_out) CU(rb.copy(counts_out, dc, counts_bytes));
-    CU(rb.finish());
+    CU(st.carve(ss.q_in, in_bytes, nq, k, hf.of_query != nullptr));
+    CU(cudaMemcpyAsync(st.q, queries, in_bytes, cudaMemcpyHostToDevice, stream));
+    if (st.fidx) CU(cudaMemcpyAsync(st.fidx, hf.of_query, (size_t)nq * 4, cudaMemcpyHostToDevice, stream));
+    ST(vsbi::upload_filters(ss, hf, pop.data(), st.fidx, stream, f));
+    ST(search_dev(st.q, nq, k, st.keys, st.dists, st.counts, stream, exact, f));
+    CU(st.read(ss.pin, stream, keys_out, dists_out, counts_out));
     reap_inflight(true);
     return VSB_OK;
 }

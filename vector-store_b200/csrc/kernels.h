@@ -17,6 +17,20 @@ struct RowsView {
     const float* nrm = nullptr;     // sqrt(sq)
     uint32_t row_bytes = 0;
     uint32_t n = 0;
+    // rows [first, first + count) of this block
+    RowsView slice(uint32_t first, uint32_t count) const {
+        return RowsView{rows + (size_t)first * row_bytes, sq + first, nrm + first, row_bytes, count};
+    }
+};
+
+// A filter: bitmaps over (key & 2^48-1), ceil(bits / 32) words each, back to back; query i tests bitmap of_q[i]
+// (of_q null: every query tests the first bitmap).  bm null: no filter.
+struct Allow {
+    const uint32_t* bm = nullptr;
+    uint64_t bits = 0;
+    const uint32_t* of_q = nullptr;
+    // the same filter for the queries from q0 on
+    Allow from(uint64_t q0) const { return Allow{bm, bits, of_q ? of_q + q0 : nullptr}; }
 };
 
 // K0 ------------------------------------------------------------------------------------------
@@ -25,9 +39,9 @@ void launch_convert_rows(int storage, const float* in, uint32_t n_rows, uint32_t
 // scaled int8 copy for the cosine traversal (per-row scale max|x|/127; nrm = |x| in units of the scale)
 void launch_convert_rows_i8s(const float* in, uint32_t n_rows, uint32_t dim, uint32_t in_stride, uint8_t* out,
                              uint32_t row_bytes, float* sq, float* nrm, cudaStream_t stream);
-void launch_gather_rows(const uint8_t* rows, uint32_t row_bytes, const float* sq, const float* nrm,
-                        const uint32_t* slots, uint32_t n, uint8_t* out_rows, float* out_sq, float* out_nrm,
-                        cudaStream_t stream);
+// row i of the output = row slots[i] of src
+void launch_gather_rows(const RowsView& src, const uint32_t* slots, uint32_t n, uint8_t* out_rows, float* out_sq,
+                        float* out_nrm, cudaStream_t stream);
 
 void launch_gather_u64(const uint64_t* in, const uint32_t* slots, uint32_t n, uint64_t* out, cudaStream_t stream);
 void launch_gather_u32(const uint32_t* in, const uint32_t* slots, uint32_t n, uint32_t* out, cudaStream_t stream);
@@ -43,11 +57,7 @@ struct ExactParams {
     uint32_t x_lo = 0, x_hi = 0;      // row range inside x
     const uint32_t* deny = nullptr;   // tombstone bitmap over rows of x (nullable)
     const uint64_t* keys = nullptr;   // u64 key per row of x (tie-break + output)
-    const uint32_t* allow = nullptr;  // N1: bitmap over (key & 2^48-1) (nullable)
-    uint64_t allow_bits = 0;
-    // [q.n] index of each query's bitmap: query i tests allow + allow_of_q[i] * ceil(allow_bits / 32)
-    // (nullable: every query uses the first bitmap)
-    const uint32_t* allow_of_q = nullptr;
+    Allow allow;                      // N1: filter over (key & 2^48-1), of_q indexed by query of q
     uint32_t kp = 32;                 // candidate list length, multiple of 32, <= 256
     uint32_t n_splits = 1;
     uint64_t* part = nullptr;         // scratch [q.n][n_splits][kp]
@@ -154,9 +164,7 @@ struct SearchParams {
     unsigned long long* counters = nullptr;  // [2]: distance evals, parent expansions (instrumented only)
     // filtered ANN (usearch.rs:224-248): every row is traversed, only rows whose bit (key & 2^48-1) is set enter the
     // result list (a second list next to the traversal list)
-    const uint32_t* allow = nullptr;
-    uint64_t allow_bits = 0;
-    const uint32_t* allow_of_q = nullptr;  // per-query bitmap index, as in ExactParams (nullable)
+    Allow allow;
     // 16-bit float rows, warp-per-query kernel only: evaluate the rows on the tensor cores (mma.sync, candidate-grade
     // distances — the caller re-ranks the rows it returns).  graph_search_uses_mma() tells which launches honour it.
     bool mma = false;

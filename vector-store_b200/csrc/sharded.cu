@@ -42,7 +42,7 @@ struct Sharded {
     DevBuf g_keys, g_dists, out_buf, q0;
     PinBuf pin;  // pinned staging of the merged results for pageable callers
     // per shard
-    std::vector<DevBuf> qbuf, allow, fidx;
+    std::vector<DevBuf> qbuf, fidx;
     std::vector<cudaEvent_t> done_ev;
 
     uint32_t G() const { return (uint32_t)shards.size(); }
@@ -153,7 +153,6 @@ vsb_status create_sharded(const vsb_options* o, vsb_index** out) {
     ix->degree = S.shards[0]->degree;
     ix->graph_stride = S.shards[0]->graph_stride;
     S.qbuf.resize(G);
-    S.allow.resize(G);
     S.fidx.resize(G);
     S.done_ev.resize(G, nullptr);
     cudaSetDevice(dev0);
@@ -195,7 +194,6 @@ void destroy_sharded(vsb_index* ix) {
         cudaDeviceSynchronize();
         if (i < S.done_ev.size() && S.done_ev[i]) cudaEventDestroy(S.done_ev[i]);
         if (i < S.qbuf.size()) S.qbuf[i].release();
-        if (i < S.allow.size()) S.allow[i].release();
         if (i < S.fidx.size()) S.fidx[i].release();
     }
     cudaSetDevice(ix->device);
@@ -408,7 +406,6 @@ static vsb_status fan_out(vsb_index* ix, const float* d_q, cudaEvent_t ready, ui
     uint64_t* gk = S.g_keys.as<uint64_t>();
     float* gd = S.g_dists.as<float>();
     const size_t q_bytes = (size_t)nq * ix->dim * 4;
-    const size_t allow_words = hf.bitmaps ? (size_t)((hf.bits + 31) / 32) * hf.n : 0;
     std::vector<uint64_t> shard_pop(pop.size());
     for (size_t f = 0; f < pop.size(); ++f) shard_pop[f] = pop[f] / G;
     ST(S.for_each([&](uint32_t i) -> vsb_status {
@@ -423,21 +420,13 @@ static vsb_status fan_out(vsb_index* ix, const float* d_q, cudaEvent_t ready, ui
             CU(cudaMemcpyPeerAsync(S.qbuf[i].p, S.devices[i], d_q, dev0, q_bytes, si));  // NVLink, device to device
             q_local = S.qbuf[i].as<float>();
         }
-        Filters f;
-        if (hf.bitmaps) {
-            CU(S.allow[i].ensure(std::max<size_t>(allow_words * 4, 16)));
-            CU(cudaMemcpyAsync(S.allow[i].p, hf.bitmaps, allow_words * 4, cudaMemcpyHostToDevice, si));
-            f.d_allow = S.allow[i].as<uint32_t>();
-            f.bits = hf.bits;
-            f.n = hf.n;
-            f.pop = shard_pop.data();
-            if (hf.of_query) {
-                CU(S.fidx[i].ensure((size_t)nq * 4));
-                CU(cudaMemcpyAsync(S.fidx[i].p, hf.of_query, (size_t)nq * 4, cudaMemcpyHostToDevice, si));
-                f.d_fidx = S.fidx[i].as<uint32_t>();
-                f.h_fidx = hf.of_query;
-            }
+        // the bitmaps go into the shard's own search scratch (its search_mu is held)
+        if (hf.of_query) {
+            CU(S.fidx[i].ensure((size_t)nq * 4));
+            CU(cudaMemcpyAsync(S.fidx[i].p, hf.of_query, (size_t)nq * 4, cudaMemcpyHostToDevice, si));
         }
+        Filters f;
+        ST(upload_filters(sh->ss, hf, shard_pop.data(), hf.of_query ? S.fidx[i].as<uint32_t>() : nullptr, si, f));
         // the shard's last kernel stores into device 0's gather buffer (peer-mapped): part i of [G][nq][k]
         ST(sh->search_dev(q_local, nq, k, gk + (size_t)i * nq * k, gd + (size_t)i * nq * k, nullptr, si, exact, f));
         CU(cudaEventRecord(S.done_ev[i], si));
@@ -471,26 +460,14 @@ vsb_status sharded_search_host(vsb_index* ix, const float* queries, uint64_t nq,
     std::lock_guard<std::mutex> g(S.search);
     CU(cudaSetDevice(S.devices[0]));
     const size_t q_bytes = (size_t)nq * ix->dim * 4;
-    const size_t kb = (size_t)nq * k * 8, db = (size_t)nq * k * 4, cb = (size_t)nq * 4;
-    auto al = [](size_t v) { return (v + 255) / 256 * 256; };
-    CU(S.q0.ensure(q_bytes, true));
-    CU(S.out_buf.ensure(al(kb) + al(db) + al(cb)));
-    uint64_t* ok = S.out_buf.as<uint64_t>();
-    float* od = reinterpret_cast<float*>(S.out_buf.as<uint8_t>() + al(kb));
-    uint32_t* oc = reinterpret_cast<uint32_t*>(S.out_buf.as<uint8_t>() + al(kb) + al(db));
+    CU(S.q0.ensure(q_bytes, true));  // plain memory: the shards read it peer to peer
+    Staging out;
+    CU(out.carve(S.out_buf, 0, nq, k, false));
     CU(cudaMemcpyAsync(S.q0.p, queries, q_bytes, cudaMemcpyHostToDevice, S.stream0));
     CU(cudaEventRecord(S.q_ready, S.stream0));
-    std::vector<uint64_t> pop(hf.bitmaps ? hf.n : 0, 0);
-    const size_t words = (size_t)((hf.bits + 31) / 32);
-    for (size_t f = 0; f < pop.size(); ++f)
-        for (size_t i = 0; i < words; ++i) pop[f] += (uint64_t)__builtin_popcount(hf.bitmaps[f * words + i]);
-    ST(fan_out(ix, S.q0.as<float>(), S.q_ready, nq, k, ok, od, oc, S.stream0, exact, hf, pop));
-    vsbi::HostReadback rb(S.pin, S.stream0);  // pageable destinations are staged (index_impl.h)
-    CU(rb.reserve(al(kb) + al(db) + al(cb)));
-    CU(rb.copy(keys, ok, kb));
-    CU(rb.copy(dists, od, db));
-    if (counts) CU(rb.copy(counts, oc, cb));
-    CU(rb.finish());
+    ST(fan_out(ix, S.q0.as<float>(), S.q_ready, nq, k, out.keys, out.dists, out.counts, S.stream0, exact, hf,
+               filter_population(hf)));
+    CU(out.read(S.pin, S.stream0, keys, dists, counts));
     return VSB_OK;
 }
 

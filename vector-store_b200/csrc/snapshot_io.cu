@@ -75,9 +75,10 @@ vsb_status save_single(vsb_index* ix, const char* path) {
     ok = ok && fwrite(ix->h_deny.data(), 4, (n + 31) / 32, f) == (n + 31) / 32;
     if (n) {
         ok = ok && write_dev(f, v.st->keys.p, n * 8, stage);
-        ok = ok && write_dev(f, v.st->rows.p, n * ix->row_bytes, stage);
-        ok = ok && write_dev(f, v.st->sq.p, n * 4, stage);
-        ok = ok && write_dev(f, v.st->nrm.p, n * 4, stage);
+        const vsbi::RowBuf& rows = v.st->rows;
+        ok = ok && write_dev(f, rows.rows.p, n * ix->row_bytes, stage);
+        ok = ok && write_dev(f, rows.sq.p, n * 4, stage);
+        ok = ok && write_dev(f, rows.nrm.p, n * 4, stage);
     }
     if (v.n_graphed) ok = ok && write_dev(f, v.gr->g.p, (size_t)v.n_graphed * ix->graph_stride * 4, stage);
     ok = (fclose(f) == 0) && ok;
@@ -126,9 +127,9 @@ vsb_status load_single(const char* path, int32_t device, vsb_index** out) {
         if (cudaMemcpy(store.keys.p, h_keys.data(), n * 8, cudaMemcpyHostToDevice) != cudaSuccess ||
             cudaMemcpy(store.deny.p, ix->h_deny.data(), ((n + 31) / 32) * 4, cudaMemcpyHostToDevice) != cudaSuccess)
             return bail(VSB_ECUDA, "upload failed");
-        ok = read_dev(f, store.rows.p, n * ix->row_bytes, stage, no_check);
-        ok = ok && read_dev(f, store.sq.p, n * 4, stage, no_check);
-        ok = ok && read_dev(f, store.nrm.p, n * 4, stage, no_check);
+        ok = read_dev(f, store.rows.rows.p, n * ix->row_bytes, stage, no_check);
+        ok = ok && read_dev(f, store.rows.sq.p, n * 4, stage, no_check);
+        ok = ok && read_dev(f, store.rows.nrm.p, n * 4, stage, no_check);
     }
     if (ok && h.n_graphed) {
         auto gr = std::make_shared<vsbi::Graph>();
@@ -170,15 +171,9 @@ vsb_status load_single(const char* path, int32_t device, vsb_index** out) {
     ix->search_width = std::min<uint32_t>(std::max<uint32_t>(h.search_width, 1), 4);
     ix->stream_threshold = h.stream_threshold;
     ix->churn_since_refine = h.churn_since_refine;
-    if (ix->trav16 && n) {  // the traversal copies are derived data: regenerated instead of stored
-        vsb::launch_convert_rows(VSB_BF16, store.rows.as<float>(), (uint32_t)n, ix->row_bytes / 4, store.rows16.as<uint8_t>(),
-                                 ix->row_bytes16, store.sq16.as<float>(), store.nrm16.as<float>(), ix->mstream);
-    }
-    if (ix->trav8 && n) {
-        vsb::launch_convert_rows_i8s(store.rows.as<float>(), (uint32_t)n, ix->dim, ix->row_bytes / 4, store.rows8.as<uint8_t>(),
-                                     ix->row_bytes8, store.sq8.as<float>(), store.nrm8.as<float>(), ix->mstream);
-    }
-    if (ix->w.n_graphed && ix->sample_seeds(ix->w.n_graphed) != VSB_OK) {
+    // the traversal copies are derived data: regenerated instead of stored
+    if ((n && ix->derive_traversal(store, store.rows.rows.as<float>(), ix->row_bytes / 4, 0, (uint32_t)n) != VSB_OK) ||
+        (ix->w.n_graphed && ix->sample_seeds(ix->w.n_graphed) != VSB_OK)) {
         destroy_single(ix);
         return VSB_ECUDA;
     }
