@@ -27,7 +27,6 @@
 
 #include <algorithm>
 #include <cmath>
-#include <cstdlib>
 
 #include "kernels.h"
 #include "select.cuh"
@@ -300,13 +299,15 @@ __device__ __forceinline__ uint64_t make_smem_desc(uint32_t smem_addr) {
     return d;
 }
 
-// CTA2 = true: the kernel runs as clusters of two CTAs (cta_group::2).  Each CTA owns its own 128 query rows
-// (its half of the M = 256 accumulator) and stages only 128 of the tile's 256 corpus rows; the leader CTA issues
-// the MMAs for the pair, so a CTA moves 32 KB instead of 48 KB per K slab and a fourth stage fits.
-template <int KIND, int METRIC, bool TILE_MIN, bool CTA2>
+// The list-maintaining form (TILE_MIN = false) runs as clusters of two CTAs (cta_group::2).  Each CTA owns its own
+// 128 query rows (its half of the M = 256 accumulator) and stages only 128 of the tile's 256 corpus rows; the leader
+// CTA issues the MMAs for the pair, so a CTA moves 32 KB instead of 48 KB per K slab and a fourth stage fits
+// (1 046 vs 964 TFLOP/s on 10 000 x 1 M x 768 bf16).  The seed layer's tile-min form is tiny and runs as single CTAs.
+template <int KIND, int METRIC, bool TILE_MIN>
 __global__ void __launch_bounds__(TC_THREADS, 1)
     exact_candidates_tc_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_x,
                                TcArgs a) {
+    constexpr bool CTA2 = !TILE_MIN;
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
     uint64_t* buf = reinterpret_cast<uint64_t*>(smem + TC_OFF_BUF);
@@ -670,11 +671,11 @@ bool make_map(CUtensorMap* map, int kind, const void* base, uint32_t rows, uint3
     return r == CUDA_SUCCESS;
 }
 
-template <int KIND, int METRIC, bool TILE_MIN, bool CTA2>
+template <int KIND, int METRIC, bool TILE_MIN>
 void launch_tc_one(const CUtensorMap& mq, const CUtensorMap& mx, const TcArgs& a, dim3 grid, cudaStream_t stream) {
-    auto kern = exact_candidates_tc_kernel<KIND, METRIC, TILE_MIN, CTA2>;
+    auto kern = exact_candidates_tc_kernel<KIND, METRIC, TILE_MIN>;
     cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TC_SMEM_BYTES);
-    if constexpr (CTA2) {
+    if constexpr (!TILE_MIN) {  // CTA pairs
         cudaLaunchConfig_t cfg{};
         cfg.gridDim = grid;
         cfg.blockDim = dim3(TC_THREADS);
@@ -694,37 +695,22 @@ void launch_tc_one(const CUtensorMap& mq, const CUtensorMap& mx, const TcArgs& a
 }
 
 template <int KIND, int METRIC>
-void launch_tc_inst(const CUtensorMap& mq, const CUtensorMap& mx, const TcArgs& a, dim3 grid, cudaStream_t stream,
-                    bool cta2) {
-    if (a.tile_min) {
-        launch_tc_one<KIND, METRIC, true, false>(mq, mx, a, grid, stream);  // the seed layer is tiny: 1-CTA form
-    } else if (cta2) {
-        launch_tc_one<KIND, METRIC, false, true>(mq, mx, a, grid, stream);
-    } else {
-        launch_tc_one<KIND, METRIC, false, false>(mq, mx, a, grid, stream);
-    }
+void launch_tc_inst(const CUtensorMap& mq, const CUtensorMap& mx, const TcArgs& a, dim3 grid, cudaStream_t stream) {
+    if (a.tile_min) launch_tc_one<KIND, METRIC, true>(mq, mx, a, grid, stream);
+    else launch_tc_one<KIND, METRIC, false>(mq, mx, a, grid, stream);
 }
 
 template <int KIND>
 void launch_tc_kind(int metric, const CUtensorMap& mq, const CUtensorMap& mx, const TcArgs& a, dim3 grid,
-                    cudaStream_t stream, bool cta2) {
+                    cudaStream_t stream) {
     switch (metric) {
-        case VSB_METRIC_L2SQ: launch_tc_inst<KIND, VSB_METRIC_L2SQ>(mq, mx, a, grid, stream, cta2); break;
-        case VSB_METRIC_COS: launch_tc_inst<KIND, VSB_METRIC_COS>(mq, mx, a, grid, stream, cta2); break;
-        default: launch_tc_inst<KIND, VSB_METRIC_IP>(mq, mx, a, grid, stream, cta2); break;
+        case VSB_METRIC_L2SQ: launch_tc_inst<KIND, VSB_METRIC_L2SQ>(mq, mx, a, grid, stream); break;
+        case VSB_METRIC_COS: launch_tc_inst<KIND, VSB_METRIC_COS>(mq, mx, a, grid, stream); break;
+        default: launch_tc_inst<KIND, VSB_METRIC_IP>(mq, mx, a, grid, stream); break;
     }
 }
 
 }  // namespace
-
-// cta_group::2 form of the list-maintaining kernel (VSB_TC_2CTA=0/1); the seed layer's tile-min kernel is always 1-CTA
-static bool tc_use_cta_pairs() {
-    static const bool on = [] {
-        const char* e = getenv("VSB_TC_2CTA");
-        return e != nullptr ? e[0] == '1' : true;  // default on: 1 046 vs 964 TFLOP/s on 10 000 x 1 M x 768 bf16
-    }();
-    return on;
-}
 
 bool exact_tc_supported(int storage, int metric) {
     if (metric == VSB_METRIC_HAMMING) return false;
@@ -749,15 +735,12 @@ uint32_t exact_tc_pick_splits(uint32_t nq, uint32_t n_rows, int sm_count, uint32
     // (k' = 96 over 131 072 rows) stay at one split.  kp = 0: tile-min mode, no lists.  CTAs of one wave walk the
     // same row split in step, so the corpus stream stays L2-resident however many splits there are.
     uint32_t q_tiles = (nq + TC_M - 1) / TC_M;
-    if (kp != 0 && tc_use_cta_pairs()) q_tiles = (q_tiles + 1) & ~1u;  // CTA pairs: an odd tail tile gets a partner
+    if (kp != 0) q_tiles = (q_tiles + 1) & ~1u;  // CTA pairs: an odd tail tile gets a partner
     const uint32_t min_tiles = kp == 0 ? 2 : 8;
     uint32_t max_by_rows = n_rows / (min_tiles * TC_N);
     if (max_by_rows < 1) max_by_rows = 1;
     const uint32_t s_max = max_by_rows < 64 ? max_by_rows : 64;
-    static const double insert_cost = [] {
-        const char* e = getenv("VSB_TC_SPLIT_PENALTY");
-        return e ? atof(e) : 200.0;
-    }();
+    constexpr double insert_cost = 200.0;  // scanned elements per list insertion, the calibrated weight above
     uint32_t best = 1;
     double best_cost = 1e30;
     for (uint32_t s = 1; s <= s_max; ++s) {
@@ -780,7 +763,7 @@ uint32_t exact_tc_pick_splits(uint32_t nq, uint32_t n_rows, int sm_count, uint32
 bool launch_exact_candidates_tc(const ExactParams& p, cudaStream_t stream, bool tile_min) {
     if (p.q.n == 0 || p.x_hi <= p.x_lo) return true;
     const int kind = p.storage == VSB_ST_F32 ? KIND_TF32 : (p.storage == VSB_ST_BF16 ? KIND_BF16 : KIND_F16);
-    const bool cta2 = tc_use_cta_pairs() && !tile_min;
+    const bool cta2 = !tile_min;  // list launches run as CTA pairs
     CUtensorMap mq, mx;
     if (!make_map(&mq, kind, p.q.rows, p.q.n, p.q.row_bytes, TC_M)) return false;
     if (!make_map(&mx, kind, p.x.rows, p.x_hi, p.x.row_bytes, cta2 ? TC_N / 2 : TC_N)) return false;
@@ -804,9 +787,9 @@ bool launch_exact_candidates_tc(const ExactParams& p, cudaStream_t stream, bool 
     if (cta2) q_tiles = (q_tiles + 1) & ~1u;  // CTA pairs: an odd tail tile gets an all-padding partner
     dim3 grid(q_tiles, row_splits);
     switch (kind) {
-        case KIND_BF16: launch_tc_kind<KIND_BF16>(p.metric, mq, mx, a, grid, stream, cta2); break;
-        case KIND_F16: launch_tc_kind<KIND_F16>(p.metric, mq, mx, a, grid, stream, cta2); break;
-        default: launch_tc_kind<KIND_TF32>(p.metric, mq, mx, a, grid, stream, cta2); break;
+        case KIND_BF16: launch_tc_kind<KIND_BF16>(p.metric, mq, mx, a, grid, stream); break;
+        case KIND_F16: launch_tc_kind<KIND_F16>(p.metric, mq, mx, a, grid, stream); break;
+        default: launch_tc_kind<KIND_TF32>(p.metric, mq, mx, a, grid, stream); break;
     }
     g_kernel_launches += 1;
     g_tc_launches += 1;

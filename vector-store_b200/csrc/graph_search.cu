@@ -1,6 +1,4 @@
 // graph_search.cu — host launcher of K4 (kernel in graph_search.cuh, instantiated per storage scalar).
-#include <cstdlib>
-
 #include "graph_search.cuh"
 
 namespace vsb {
@@ -45,16 +43,16 @@ void launch_seed_scan(int storage, int metric, const RowsView& q, const RowsView
 // Tensor-core evaluation of 16-bit rows pays for its re-rank (a fixed ~0.09 ms per 10 000 queries) and its
 // candidate-grade bookkeeping only on long searches: 10 M rows at ef = 224 gain 6 % (9.19 -> 8.66 ms), 1.25 M-row
 // shards at ef = 32 lose 10 % (1.29 -> 1.42 ms + the re-rank).  Automatic: beams of at least 96 entries.
-// VSB_K4_MMA=0 / 1 forces the SIMT / tensor-core evaluation.
 bool graph_search_uses_mma(int storage, uint32_t n_queries, bool filtered, uint32_t itopk) {
-    static const int mode = [] {
-        const char* e = getenv("VSB_K4_MMA");
-        return e == nullptr ? -1 : (e[0] != '0' ? 1 : 0);
-    }();
-    if (mode == 0 || filtered || n_queries <= graph_search_small_batch()) return false;
+    if (filtered || n_queries <= graph_search_small_batch()) return false;
     if (storage != VSB_ST_BF16 && storage != VSB_ST_F16) return false;
-    return mode == 1 || itopk >= 96;
+    return itopk >= 96;
 }
+
+// Visited hash: 16 KB per warp (4096 slots) = 3 CTAs x 4 query warps per SM, the same residency the register budget
+// allows; it is reset to "what is still in the list" when 3/4 full (forgotten nodes cost a re-evaluation, never a
+// duplicate).
+constexpr uint32_t K4_HASH_BITS = 12;
 
 void launch_graph_search(const SearchParams& p, cudaStream_t stream) {
     if (p.q.n == 0) return;
@@ -69,15 +67,7 @@ void launch_graph_search(const SearchParams& p, cudaStream_t stream) {
     a.search_width = p.search_width < 1 ? 1 : (p.search_width > (uint32_t)K4_MAX_WIDTH ? (uint32_t)K4_MAX_WIDTH : p.search_width);
     a.max_iters = p.max_iters ? p.max_iters : (2 * a.itopk) / a.search_width + 8;
     a.k = p.k;
-    // Visited hash: 16 KB per warp (4096 slots) = 3 CTAs x 4 query warps per SM, the same residency the
-    // register budget allows; it is reset to "what is still in the list" when 3/4 full (forgotten nodes
-    // cost a re-evaluation, never a duplicate).
-    static const uint32_t bits_env = [] {
-        const char* e = getenv("VSB_K4_HASH_BITS");
-        return e ? (uint32_t)atoi(e) : 0u;
-    }();
-    const uint32_t bits = bits_env >= 8 && bits_env <= 14 ? bits_env : 12;
-    a.hash_bits = bits;
+    a.hash_bits = K4_HASH_BITS;
     const uint32_t deg_pad = ((p.degree + 31) / 32) * 32;
     a.queue_cap = a.search_width * deg_pad < 32 ? 32 : a.search_width * deg_pad;
     a.metric = p.metric;
@@ -88,16 +78,6 @@ void launch_graph_search(const SearchParams& p, cudaStream_t stream) {
     a.allow_of_q = p.allow.of_q;
     a.rk = p.allow.bm != nullptr ? ((p.k + 31) / 32) * 32 : 0;
     a.mma = 0;
-    static const uint32_t compact_env = [] {
-        const char* e = getenv("VSB_K4_COMPACT");
-        return e ? (uint32_t)atoi(e) : 1u;
-    }();
-    a.compact = compact_env;
-    static const uint32_t l2pf_env = [] {
-        const char* e = getenv("VSB_K4_L2PF");
-        return e ? (uint32_t)atoi(e) : 0u;
-    }();
-    a.l2pf = l2pf_env;
     const int cpl = pick_cpl((int)(p.x.row_bytes / 16));
     // filtered ANN always runs the warp-per-query kernel (the second list lives there)
     if (p.q.n <= graph_search_small_batch() && p.allow.bm == nullptr) {
@@ -106,7 +86,7 @@ void launch_graph_search(const SearchParams& p, cudaStream_t stream) {
         a.max_iters = p.max_iters ? p.max_iters : (2 * a.itopk) / a.search_width + 8;
         a.queue_cap = a.search_width * deg_pad;
         dim3 gridb(p.q.n);
-        const size_t smemb = (size_t)a.itopk * 16 + (size_t)a.queue_cap * 16 + ((size_t)4 << bits) + 64 + 128;
+        const size_t smemb = (size_t)a.itopk * 16 + (size_t)a.queue_cap * 16 + ((size_t)4 << K4_HASH_BITS) + 64 + 128;
         switch (p.storage) {
             case VSB_ST_F32: launch_k4b_f32(a, cpl, gridb, smemb, stream); break;
             case VSB_ST_F16: launch_k4b_f16(a, cpl, gridb, smemb, stream); break;
@@ -119,7 +99,7 @@ void launch_graph_search(const SearchParams& p, cudaStream_t stream) {
     }
     dim3 grid((p.q.n + K4_WARPS - 1) / K4_WARPS);
     a.mma = (p.mma && p.allow.bm == nullptr && (p.storage == VSB_ST_BF16 || p.storage == VSB_ST_F16)) ? 1u : 0u;
-    const size_t smem = (size_t)K4_WARPS * ((size_t)a.itopk * 8 + ((size_t)2 << bits) + (size_t)a.queue_cap * 8 + (size_t)a.rk * 8 + 64 * 8);
+    const size_t smem = (size_t)K4_WARPS * ((size_t)a.itopk * 8 + ((size_t)2 << K4_HASH_BITS) + (size_t)a.queue_cap * 8 + (size_t)a.rk * 8 + 64 * 8);
     switch (p.storage) {
         case VSB_ST_F32: launch_k4_f32(a, cpl, grid, smem, stream); break;
         case VSB_ST_F16: launch_k4_f16(a, cpl, grid, smem, stream); break;

@@ -12,9 +12,6 @@
 //     into the list.
 // HBM-bound by design: bytes/query = E * row_bytes + P * R * 4 (E, P counted in-kernel).
 #pragma once
-#ifdef VSB_K4B_PROFILE
-#include <cstdio>
-#endif
 #include "kernels.h"
 #include "select.cuh"
 
@@ -51,8 +48,6 @@ struct K4Args {
     const uint32_t* allow_of_q;  // [nq] bitmap index per query (nullable: bitmap 0)
     uint32_t rk;            // length of the result list of the FILTER instantiation (k rounded up to 32)
     uint32_t mma;           // 1: 16-bit rows are evaluated on the tensor cores (mma.sync), distances are candidate-grade
-    uint32_t compact;       // 1: survivors of an iteration are compacted before the sort + merge
-    uint32_t l2pf;          // rows of prefetch distance into L2 (0 = off), warp-per-query kernel
 };
 
 __device__ __forceinline__ bool hash_insert(uint32_t* tab, uint32_t mask, uint32_t bits, uint32_t slot) {
@@ -249,26 +244,13 @@ __device__ __forceinline__ void group_reduce_mma(const VecGroup<CPL, U>& grp, co
 
 // all queue entries of this warp: index(m) = first + m * stride, m < mine.  Double buffered: the loads of
 // group m+1 are in flight while group m is reduced.
-// whole-row prefetch into L2 by the bulk-copy engine: one instruction per row, nothing comes back to the SM
-__device__ __forceinline__ void prefetch_row_l2(const void* p, uint32_t bytes) {
-    asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(p), "r"(bytes) : "memory");
-}
-
-// l2pf > 0: rows `l2pf` positions ahead of the group being loaded are prefetched into L2 (all rows of an iteration are
-// known when it starts).  The register double buffer holds at most 2 U rows in flight per warp; at HBM latency that is
-// what bounds the kernel, at L2 latency it is plenty — the bulk prefetches carry the HBM latency instead and cost
-// neither registers nor issue slots.
 template <int ST, int CPL, int U, bool MMA = false>
 __device__ __forceinline__ void evaluate_entries(const uint8_t* __restrict__ x_rows, uint32_t row_bytes,
                                                  const uint32_t* newq, float* newd, uint32_t first, uint32_t stride,
                                                  uint32_t mine, uint32_t n_new, const float* qf, const uint4* qc,
-                                                 bool is_l2, int lane, int n_chunks, bool full, uint32_t l2pf = 0) {
+                                                 bool is_l2, int lane, int n_chunks, bool full) {
     if (mine == 0) return;
     const uint32_t last = first + (mine - 1) * stride;
-    if (l2pf != 0) {
-        for (uint32_t m = 2 * U + lane; m < l2pf + 2 * U && m < mine; m += 32)
-            prefetch_row_l2(x_rows + (size_t)newq[first + m * stride] * row_bytes, row_bytes);
-    }
     auto reduce = [&](const VecGroup<CPL, U>& grp, uint32_t base) {
         if constexpr (MMA) group_reduce_mma<ST, CPL, U>(grp, qc, newd, base, stride, n_new, lane);
         else group_reduce<ST, CPL, U>(grp, qf, qc, is_l2, newd, base, stride, n_new, lane);
@@ -277,10 +259,6 @@ __device__ __forceinline__ void evaluate_entries(const uint8_t* __restrict__ x_r
     group_load<CPL, U>(ga, x_rows, row_bytes, newq, first, stride, last, lane, n_chunks, full);
     for (uint32_t m0 = 0; m0 < mine; m0 += 2 * U) {
         const bool has_b = m0 + U < mine;
-        if (l2pf != 0) {
-            const uint32_t m = m0 + 2 * U + l2pf + lane;
-            if (lane < 2 * U && m < mine) prefetch_row_l2(x_rows + (size_t)newq[first + m * stride] * row_bytes, row_bytes);
-        }
         if (has_b) group_load<CPL, U>(gb, x_rows, row_bytes, newq, first + (m0 + U) * stride, stride, last, lane, n_chunks, full);
         reduce(ga, first + m0 * stride);
         if (has_b) {
@@ -294,10 +272,7 @@ __device__ __forceinline__ void evaluate_entries(const uint8_t* __restrict__ x_r
 // Compile-time cap of search_width.  8 was measured: the wider unrolled parent / neighbour loops slow EVERY width down
 // (1.25 M x 768 bf16, ef 64, 2 parents: 3.65 ms with a cap of 4, 4.39 ms with a cap of 8), which costs more than
 // 8 parents per iteration gain on long searches.
-#ifndef VSB_K4_MAX_WIDTH
-#define VSB_K4_MAX_WIDTH 4
-#endif
-constexpr int K4_MAX_WIDTH = VSB_K4_MAX_WIDTH;  // parents expanded per iteration (search_width)
+constexpr int K4_MAX_WIDTH = 4;  // parents expanded per iteration (search_width)
 
 // resident CTAs per SM the register budget is sized for: short int8 rows (the scaled-int8 traversal copy) need
 // few load registers, and the kernel is bound by the number of rows in flight per SM, not by bytes
@@ -397,7 +372,7 @@ __global__ void __launch_bounds__(K4_WARPS * 32, k4_min_blocks<ST, CPL, MMA>()) 
             }
         }
         evaluate_entries<ST, CPL, U, MMA>(a.x_rows, a.x_row_bytes, newq, newd, 0, 1, n_new, n_new, qf, qc, is_l2, lane,
-                                          n_chunks, full, a.l2pf);
+                                          n_chunks, full);
         __syncwarp();
         // Candidates that cannot enter the list (most of them once the beam has converged) are dropped first and the
         // survivors of ALL batches of this iteration are compacted into `stage`, so the shuffle sort + list merge — the
@@ -439,7 +414,7 @@ __global__ void __launch_bounds__(K4_WARPS * 32, k4_min_blocks<ST, CPL, MMA>()) 
             const bool keep = res < worst;
             const uint32_t km = __ballot_sync(kFullMask, keep);
             if (km == 0) continue;  // nothing here can enter the list
-            if (!a.compact || n_new <= 32) {  // a single batch (or VSB_K4_COMPACT=0): sort + merge it directly
+            if (n_new <= 32) {  // a single batch: sort + merge it directly
                 res = warp_sort32(res, lane, less);
                 warp_list_merge(list, (int)a.itopk, res, lane, less);
                 continue;
@@ -588,18 +563,6 @@ constexpr int K4B_WARPS = 8;
 constexpr int K4B_MAX_WIDTH = 8;
 constexpr int K4B_PICK_ROUNDS = 4;  // list entries per thread in the parallel parent pick (itopk <= 1024)
 
-// -DVSB_K4B_PROFILE: thread 0 of CTA 0 accumulates clock64() per phase of the iteration and prints the split
-#ifdef VSB_K4B_PROFILE
-#define K4B_T(i)                                       \
-    do {                                               \
-        const long long now_ = clock64();              \
-        prof_[i] += now_ - prof_t_;                    \
-        prof_t_ = now_;                                \
-    } while (0)
-#else
-#define K4B_T(i) do { } while (0)
-#endif
-
 template <int ST, int CPL>
 __global__ void __launch_bounds__(K4B_WARPS * 32, 1) graph_search_cta_kernel(K4Args a) {
     constexpr int E = Storage<ST>::ELEMS;
@@ -647,11 +610,6 @@ __global__ void __launch_bounds__(K4B_WARPS * 32, 1) graph_search_cta_kernel(K4A
     const float qn = a.q_nrm[q];
     unsigned long long n_evals = 0, n_parents = 0;
     __syncthreads();
-#ifdef VSB_K4B_PROFILE
-    long long prof_[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-    long long prof_t_ = clock64();
-    const long long prof_start_ = prof_t_;
-#endif
 
     const uint32_t width = a.search_width;
     const uint32_t deg_pad = ((a.degree + 31) / 32) * 32;
@@ -722,9 +680,7 @@ __global__ void __launch_bounds__(K4B_WARPS * 32, 1) graph_search_cta_kernel(K4A
     // groups of 32, then merge list and groups IN PARALLEL: every element finds its final position as its own index
     // plus its rank in each other sorted run (packed values are unique), and is scattered into the other list buffer
     auto evaluate_queue = [&]() {
-        K4B_T(0);  // own share of the neighbour fetch + visited filter
         __syncthreads();
-        K4B_T(1);  // waiting for the rest of the CTA
         const uint32_t n_new = ctrl[0];
         if (n_new != 0) {
             const uint32_t mine = n_new > (uint32_t)warp ? (n_new - warp + K4B_WARPS - 1) / K4B_WARPS : 0;
@@ -734,9 +690,7 @@ __global__ void __launch_bounds__(K4B_WARPS * 32, 1) graph_search_cta_kernel(K4A
             if (is_cos && (uint32_t)tid < n_new) xn_first = __ldg(a.x_nrm + newq[tid]);
             evaluate_entries<ST, CPL, U>(a.x_rows, a.x_row_bytes, newq, newd, (uint32_t)warp, K4B_WARPS, mine, n_new, qf, qc,
                                          is_l2, lane, n_chunks, full);
-            K4B_T(2);  // row loads + partial sums of warp 0's entries
             __syncthreads();
-            K4B_T(3);  // waiting for the slowest warp
             const uint64_t worst = list[a.itopk - 1];
             for (uint32_t i = tid; i < n_new; i += K4B_WARPS * 32) {
                 const uint32_t slot = newq[i];
@@ -746,14 +700,12 @@ __global__ void __launch_bounds__(K4B_WARPS * 32, 1) graph_search_cta_kernel(K4A
             }
             for (uint32_t i = tid; i < a.itopk; i += K4B_WARPS * 32) list_alt[i] = kInvalidPacked;
             __syncthreads();
-            K4B_T(4);  // finish + filter
             const uint32_t n_keep = ctrl[3];
             for (uint32_t g = warp; g * 32 < n_keep; g += K4B_WARPS) {
                 const uint64_t res = g * 32 + lane < n_keep ? newp[g * 32 + lane] : kInvalidPacked;
                 newp[g * 32 + lane] = warp_sort32(res, lane, less);
             }
             __syncthreads();
-            K4B_T(5);  // group sort
             if (n_keep != 0) {
                 const uint32_t n_groups = (n_keep + 31) / 32;
                 for (uint32_t i = tid; i < a.itopk + n_groups * 32; i += K4B_WARPS * 32) {
@@ -778,9 +730,7 @@ __global__ void __launch_bounds__(K4B_WARPS * 32, 1) graph_search_cta_kernel(K4A
             }
             __syncthreads();
         }
-        K4B_T(6);  // parallel merge into the list
         pick_parents();
-        K4B_T(7);  // parent pick
     };
 
     // ---- seeds (warp 0) ----
@@ -832,13 +782,6 @@ __global__ void __launch_bounds__(K4B_WARPS * 32, 1) graph_search_cta_kernel(K4A
         evaluate_queue();
     }
 
-#ifdef VSB_K4B_PROFILE
-    if (tid == 0 && q == 0)
-        printf("k4b cycles: total %lld | fetch %lld wait %lld | rows %lld wait %lld | finish %lld sort %lld fold %lld pick %lld | "
-               "evals %llu parents %llu\n",
-               clock64() - prof_start_, prof_[0], prof_[1], prof_[2], prof_[3], prof_[4], prof_[5], prof_[6], prof_[7], n_evals,
-               n_parents);
-#endif
     // ---- emit (warp 0) ----
     if (warp == 0) {
         uint32_t count = 0;

@@ -446,20 +446,13 @@ vsb_status create_single(const vsb_options* o, vsb_index** out) {
     ix->trav8 = (o->flags & VSB_FLAG_I8_TRAVERSAL) != 0 && o->storage == VSB_F32 && o->metric == VSB_COS;
     if (ix->trav8) ix->trav16 = true;  // the bf16 copy feeds the build and the seed tiles
     ix->row_bytes8 = storage_row_bytes(VSB_I8, o->dimensions);
-    if (const char* v = getenv("VSB_I8_RERANK_MULT")) ix->rr_mult8 = std::max<uint32_t>(2, (uint32_t)strtoul(v, nullptr, 10));
     if (const char* v = getenv("VSB_DISABLE_TC")) ix->tc_enabled = !(v[0] == '1');
     if (const char* v = getenv("VSB_DISABLE_CERT")) ix->cert_enabled = !(v[0] == '1');
-    if (const char* v = getenv("VSB_DISABLE_REACH_FIX")) ix->reach_fix = !(v[0] == '1');
     if (const char* v = getenv("VSB_CERT_KP")) ix->cert_kp = (uint32_t)strtoul(v, nullptr, 10);
-    if (const char* v = getenv("VSB_CERT_KP16")) ix->cert_kp16 = (uint32_t)strtoul(v, nullptr, 10);
-    if (const char* v = getenv("VSB_TC_MIN_ROWS")) ix->tc_min_rows = (uint32_t)strtoul(v, nullptr, 10);
     if (const char* v = getenv("VSB_ALLPAIRS_MAX")) ix->allpairs_max = (uint32_t)strtoul(v, nullptr, 10);
     if (const char* v = getenv("VSB_ALLPAIRS_PREFIX")) ix->allpairs_prefix = (uint32_t)strtoul(v, nullptr, 10);
     if (o->flags & VSB_FLAG_BUILD_REFINE) ix->refine_passes = 1;
     if (const char* v = getenv("VSB_REFINE_PASSES")) ix->refine_passes = (uint32_t)strtoul(v, nullptr, 10);
-    if (const char* v = getenv("VSB_CHURN_REFINE")) ix->churn_refine = !(v[0] == '0');
-    if (const char* v = getenv("VSB_TC_SAMPLED_BOUNDS")) ix->sampled_bounds = !(v[0] == '0');
-    if (const char* v = getenv("VSB_BUILD_SW")) ix->build_search_width = std::min<uint32_t>(4, std::max<uint32_t>(1, (uint32_t)strtoul(v, nullptr, 10)));
     cudaDeviceProp prop;
     if (cudaGetDeviceProperties(&prop, dev) == cudaSuccess) ix->sm_count = prop.multiProcessorCount;
     // searches on a high-priority stream, mutators (build, streaming insert, refinement) on a low-priority one:
@@ -473,14 +466,12 @@ vsb_status create_single(const vsb_options* o, vsb_index** out) {
         return fail(VSB_ECUDA, "cudaStreamCreate: %s", cudaGetErrorString(e));
     }
     ix->mstream = ix->mstream_full;
-    unsigned reserve = 12;  // SMs the mutators never touch while searches are active (VSB_SEARCH_SM_RESERVE, 0 = off)
-    if (const char* v = getenv("VSB_SEARCH_SM_RESERVE")) reserve = (unsigned)strtoul(v, nullptr, 10);
-    if (reserve > 0) {
-        unsigned sms = 0;
-        if (make_green_stream(dev, reserve, prio_lo, &ix->mstream_green, &ix->green_ctx, &sms)) ix->green_sms = sms;
-        if (getenv("VSB_VERBOSE")) fprintf(stderr, "vsb200: mutator green context on device %d: %s (%u SMs, %u reserved for searches)\n", dev, ix->mstream_green ? "on" : "unavailable", sms, reserve);
-        CU(cudaSetDevice(dev));
-    }
+    // SMs the mutators never touch while searches are active; without a green context the mutators stay on the plain
+    // low-priority stream
+    constexpr unsigned kSearchSmReserve = 12;
+    unsigned sms = 0;
+    if (make_green_stream(dev, kSearchSmReserve, prio_lo, &ix->mstream_green, &ix->green_ctx, &sms)) ix->green_sms = sms;
+    CU(cudaSetDevice(dev));
     ix->w.st = std::make_shared<Store>();
     ix->publish();
     *out = ix;

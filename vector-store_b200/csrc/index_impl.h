@@ -65,17 +65,6 @@ vsb_status fail(vsb_status st, const char* fmt, ...);
 // other devices or processes map: the router's gather buffers and the IPC exchange.
 cudaStream_t pool_stream(int device);  // index.cu
 
-// Experiment knob (VSB_PLAIN_ALLOC_MB): buffers of at least this many MB come from cudaMalloc instead of the pool
-// (page size / TLB reach of a 15 GB row store).  0 = never (default).
-inline size_t big_alloc_threshold() {
-    static const size_t t = [] {
-        const char* e = getenv("VSB_PLAIN_ALLOC_MB");
-        const size_t mb = e ? (size_t)strtoull(e, nullptr, 10) : 0;
-        return mb ? mb << 20 : ~(size_t)0;
-    }();
-    return t;
-}
-
 struct DevBuf {
     void* p = nullptr;
     size_t bytes = 0;
@@ -118,7 +107,7 @@ struct DevBuf {
         release();
         const size_t sz = want ? want : 16;
         cudaGetDevice(&dev);
-        plain = plain_memory || sz >= big_alloc_threshold();
+        plain = plain_memory;
         cudaError_t e;
         if (plain) {
             e = cudaMalloc(&p, sz);
@@ -375,20 +364,15 @@ struct vsb_index {
     int metric = 0, storage = 0, device = 0, sm_count = 148;
     uint32_t degree = 32, graph_stride = 32, k_init = 64;
     bool trav16 = false, trav8 = false;
-    uint32_t rr_mult8 = 4;
     bool tc_enabled = true;       // tcgen05 path for the dense distance tiles (VSB_DISABLE_TC=1 turns it off)
-    uint32_t tc_min_rows = 8192;  // below this the SIMT K1 is used (launch + pipeline fill dominate)
+    static constexpr uint32_t tc_min_rows = 8192;  // below this the SIMT K1 is used (launch + pipeline fill dominate)
     bool cert_enabled = true;     // VSB_DISABLE_CERT=1: exact f32 search always on the SIMT tiles
-    uint32_t cert_kp = 128, cert_kp16 = 32;
-    bool reach_fix = true;
+    uint32_t cert_kp = 128;
     uint32_t reach_budget = 1024;
     uint32_t allpairs_max = 262144, allpairs_prefix = 131072;
     // refinement passes at the end of vsb_build (VSB_REFINE_PASSES).  0 by default: with detour-pruned K7 links a pass buys
     // ~2 % QPS at equal recall and costs 1.7x the rest of the build (10 M x 768: 5.7 s -> 16.6 s, profiles/r2_*)
     uint32_t refine_passes = 0;
-    bool sampled_bounds = true;  // all-pairs kNN lists start from sampled bounds (VSB_TC_SAMPLED_BOUNDS=0 turns it off)
-    bool churn_refine = true;  // one refinement pass after 10 % of the graph has churned (VSB_CHURN_REFINE=0 turns it off)
-    uint32_t build_search_width = 4;  // parents per K4 iteration in the streaming insert / refinement searches (VSB_BUILD_SW): 10 M x 768 build 6.1 s at 2, 5.6 s at 4, same graph quality
     vsbi::Sharded* sharded = nullptr;  // n_devices > 1: every entry point forwards to the router (owned; sharded.cu)
 
     // ---- published state ----

@@ -62,7 +62,8 @@ vsb_status vsb_index::exact_block(Scratch& sc, const vsb::ExactParams& in, uint3
     const bool certify = is_float && !approx_ok && cert_enabled;
     bool tc = tc_shape && (approx_ok || storage != VSB_F32 || certify);
     const uint32_t kp_simt = p.kp;
-    if (certify && tc) p.kp = std::min<uint32_t>(256, std::max<uint32_t>(p.kp, round_up(storage == VSB_F32 ? cert_kp : cert_kp16, 32)));
+    constexpr uint32_t kCertKp16 = 32;  // certified tensor-core list length of 16-bit rows (f32 rows: cert_kp)
+    if (certify && tc) p.kp = std::min<uint32_t>(256, std::max<uint32_t>(p.kp, round_up(storage == VSB_F32 ? cert_kp : kCertKp16, 32)));
     p.n_splits = tc ? vsb::exact_tc_pick_splits(q.n, x_hi - x_lo, sm_count, p.kp)
                     : vsb::exact_pick_splits(q.n, x_hi - x_lo, sm_count);
     CU(sc.part.ensure(vsb::exact_part_elems(q.n, p.n_splits, p.kp) * 8));
@@ -80,7 +81,7 @@ vsb_status vsb_index::exact_block(Scratch& sc, const vsb::ExactParams& in, uint3
         // bound is statistical: if more than 2 % of the queries end up with fewer than k rows the block is redone
         // without it (rows stored in the order of their clusters would do that).
         const uint32_t rows = x_hi - x_lo;
-        const bool sampled = sampled_bounds && approx_ok && !certify && self_base >= 0 && rows >= 65536 && p.kp >= 64 &&
+        const bool sampled = approx_ok && !certify && self_base >= 0 && rows >= 65536 && p.kp >= 64 &&
                              p.n_splits == vsb::exact_tc_halves() && p.allow.bm == nullptr;
         if (sampled) {
             const uint32_t sample_tiles = 32, halves = vsb::exact_tc_halves();
@@ -341,8 +342,9 @@ vsb_status vsb_index::graph_block(const View& v, Scratch& sc, const GraphRun& ru
         // hand the best kr bf16-ranked candidates to K3 for the canonical fp32 re-rank
         // (2k for small k, k + 32 + k/4 for large k, at least k + 6; bf16 ranking errors only reorder
         // candidates near the k-th distance and are far smaller than that margin)
-        // int8 traversal ranks more coarsely: rr_mult8 * k candidates go to the re-rank
-        const uint32_t kv = use8 ? std::min<uint32_t>(std::max(rr_mult8 * k, k + 16), 256)
+        // int8 traversal ranks more coarsely: 4k candidates go to the re-rank
+        constexpr uint32_t kRerankMult8 = 4;
+        const uint32_t kv = use8 ? std::min<uint32_t>(std::max(kRerankMult8 * k, k + 16), 256)
                                  : std::max(std::min(2 * k, k + 32 + k / 4), k + 6);
         kr = std::min<uint32_t>(round_up(kv, 32), 256);
         if (kr < k) return fail(VSB_EINVAL, "k=%u too large for the bf16-traversal re-rank (max 256)", k);
