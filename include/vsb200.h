@@ -248,6 +248,19 @@ vsb_status vsb_search_filtered_multi(vsb_index* index, const float* queries, uin
                                      const uint32_t* filter_of_query,
                                      uint64_t* keys, float* distances, uint32_t* counts);
 
+/* Range search: for query i, every live row whose canonical distance is <= max_distance[i] and, when allow_bitmap is
+ * not NULL, whose bit (key & (2^48-1)) is set (same convention as vsb_search_filtered), ascending by (distance, key).
+ * CSR output: query i's rows are keys/distances[offsets[i] .. offsets[i+1]), offsets has q+1 entries.
+ * capacity = entries keys/distances can hold.  If the total exceeds it: VSB_EFULL, offsets fully written
+ * (offsets[q] = entries needed), keys/distances untouched; VSB_EFULL costs the full computation.  Exact on every
+ * storage and metric: the rows and the fp32 distance bits are those of a canonical brute force (oracle/exact.c).
+ * Graph and un-graphed rows alike.  max_distance[i] = +inf returns every admissible live row.  VSB_EINVAL before
+ * anything runs for a NULL queries / max_distance / offsets, NULL keys or distances with capacity > 0, or a NaN
+ * max_distance[i]. */
+vsb_status vsb_search_range(vsb_index* index, const float* queries, uint64_t q, const float* max_distance,
+                            const uint32_t* allow_bitmap, uint64_t bitmap_bits,
+                            uint64_t capacity, uint64_t* keys, float* distances, uint64_t* offsets);
+
 /* Device-resident variants: d_* are device pointers on the index's device,
  * `stream` is a cudaStream_t.  No host synchronisation, except `exact` != 0 (brute force) on float rows,
  * which reads the certification count back (see vsb_stats.exact_certified). */

@@ -200,6 +200,18 @@ unsafe extern "C" {
         distances: *mut f32,
         counts: *mut u32,
     ) -> vsb_status;
+    pub fn vsb_search_range(
+        index: *mut vsb_index,
+        queries: *const f32,
+        q: u64,
+        max_distance: *const f32,
+        allow_bitmap: *const u32,
+        bitmap_bits: u64,
+        capacity: u64,
+        keys: *mut u64,
+        distances: *mut f32,
+        offsets: *mut u64,
+    ) -> vsb_status;
     pub fn vsb_search_filtered_multi(
         index: *mut vsb_index,
         queries: *const f32,

@@ -12,6 +12,8 @@
 // wants exact results (ground truth, the un-graphed tail, filtered search, kNN-graph build).
 #include <algorithm>
 
+#include <cub/device/device_segmented_sort.cuh>
+
 #include "kernels.h"
 #include "select.cuh"
 
@@ -113,9 +115,12 @@ struct K1Args {
     const uint32_t* allow_of_q;  // [nq] bitmap index per query (nullable: bitmap 0)
     uint32_t kp, n_splits, rows_per_split, n_slabs;
     uint64_t* part;
+    RangeParams range;  // RANGE instantiations only
 };
 
-template <int ST, int METRIC>
+// RANGE = false: the split's top-kp list per query.  RANGE = true: every admissible row within the query's bound
+// (count or fill pass, see RangeParams); kp = 0, no lists.
+template <int ST, int METRIC, bool RANGE>
 __global__ void __launch_bounds__(K1_THREADS, 2) exact_candidates_kernel(K1Args a) {
     extern __shared__ __align__(16) uint8_t smem_raw[];
     float* As = reinterpret_cast<float*>(smem_raw);                  // [BK][TQ]
@@ -146,6 +151,18 @@ __global__ void __launch_bounds__(K1_THREADS, 2) exact_candidates_kernel(K1Args 
         uint32_t q = q0 + ty * 4 + i;
         qsq[i] = q < a.nq ? a.q_sq[q] : 0.0f;
         qn[i] = q < a.nq ? a.q_nrm[q] : 0.0f;
+    }
+    // range mode: each row's bound (-inf for padding rows), its count from the count pass, rows counted so far
+    float rthr[4];
+    uint32_t rcap[4], rcnt[4];
+    if constexpr (RANGE) {
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+            const uint32_t q = q0 + ty * 4 + i;
+            rthr[i] = q < a.nq ? a.range.thr[q] : __int_as_float(0xFF800000);
+            rcap[i] = q < a.nq && a.range.off != nullptr ? a.range.count[q] : 0u;
+            rcnt[i] = 0;
+        }
     }
     __syncthreads();
 
@@ -199,6 +216,44 @@ __global__ void __launch_bounds__(K1_THREADS, 2) exact_candidates_kernel(K1Args 
                     for (int j = 0; j < 8; ++j) acc[i][j] = fmaf(ar[i], br[j], acc[i][j]);
             }
             __syncthreads();
+        }
+
+        if constexpr (RANGE) {
+#pragma unroll
+            for (int i = 0; i < 4; ++i) {
+                const uint32_t q = q0 + ty * 4 + i;
+                float d[8];
+                uint32_t hit = 0;
+#pragma unroll
+                for (int j = 0; j < 8; ++j) {
+                    const uint32_t n = n0 + (j < 4 ? tx * 4 + j : 64 + tx * 4 + (j - 4));
+                    const bool nvalid = n < r_hi;
+                    d[j] = candidate_distance<ST, METRIC>(acc[i][j], qsq[i], nvalid ? a.x_sq[n] : 0.0f, qn[i],
+                                                          nvalid ? a.x_nrm[n] : 0.0f);
+                    if (!nvalid || !(d[j] <= rthr[i])) continue;
+                    bool ok = !(a.deny != nullptr && bit_test(a.deny, n));
+                    if (ok && a.allow != nullptr) {
+                        const uint64_t rid = a.keys[n] & kRowMask48;
+                        ok = rid < a.allow_bits && bit_test(query_allow(a.allow, a.allow_bits, a.allow_of_q, q), (uint32_t)rid);
+                    }
+                    if (ok) hit |= 1u << j;
+                }
+                if (hit == 0) continue;
+                if (a.range.off == nullptr) {
+                    rcnt[i] += __popc(hit);
+                    continue;
+                }
+                uint32_t pos = atomicAdd(&a.range.cursor[q], (uint32_t)__popc(hit));
+                uint64_t* seg = a.range.out + a.range.off[q];
+#pragma unroll
+                for (int j = 0; j < 8; ++j) {
+                    if (!((hit >> j) & 1u)) continue;
+                    const uint32_t n = n0 + (j < 4 ? tx * 4 + j : 64 + tx * 4 + (j - 4));
+                    if (pos < rcap[i]) seg[pos] = pack_ds(d[j], n);
+                    ++pos;
+                }
+            }
+            continue;
         }
 
         // ---- fused selection epilogue ----
@@ -268,6 +323,14 @@ __global__ void __launch_bounds__(K1_THREADS, 2) exact_candidates_kernel(K1Args 
         }
     }
 
+    if constexpr (RANGE) {
+        if (a.range.off == nullptr) {
+#pragma unroll
+            for (int i = 0; i < 4; ++i)
+                if (rcnt[i] != 0) atomicAdd(&a.range.count[q0 + ty * 4 + i], rcnt[i]);
+        }
+        return;
+    }
     // write the split's lists
     for (uint32_t i = tid; i < TQ * a.kp; i += K1_THREADS) {
         const uint32_t row = i / a.kp, c = i % a.kp;
@@ -464,17 +527,8 @@ __global__ void __launch_bounds__((CTA ? K3C_WARPS : K3_WARPS) * 32) exact_reran
                 ok = false;
             } else {
                 const float floor_d = ord_to_f32(packed_hi(cand_floor)), dk = ord_to_f32(packed_hi(pk));
-                const float xm = *a.x_nrm_max;
-                // |candidate-stage distance - canonical distance| <= eps for every row of the block:
-                //   cert_rel bounds the dot-product error relative to |q||x|, cert_sum the rounding of an
-                //   fp32 sum of `dim` terms (the norms of the L2 expansion, the canonical sum itself)
-                float eps;
-                if constexpr (METRIC == VSB_METRIC_COS)
-                    eps = a.cert_rel + 1e-6f;
-                else if constexpr (METRIC == VSB_METRIC_L2SQ)
-                    eps = (a.cert_rel + a.cert_sum) * (qn * qn + xm * xm);
-                else
-                    eps = a.cert_rel * qn * xm + 0x1p-22f * (1.0f + qn * xm);
+                // |candidate-stage distance - canonical distance| <= eps for every row of the block
+                const float eps = cert_margin<METRIC>(a.cert_rel, a.cert_sum, qn, *a.x_nrm_max);
                 ok = dk + eps < floor_d;  // false for NaN
             }
         }
@@ -618,10 +672,95 @@ __global__ void max_norm_kernel(const float* nrm, uint32_t lo, uint32_t hi, floa
     if ((threadIdx.x & 31) == 0) atomicMax(reinterpret_cast<unsigned int*>(out), __float_as_uint(m));
 }
 
-template <int ST, int METRIC>
+template <int ST, int METRIC, bool RANGE = false>
 void launch_k1(const K1Args& a, dim3 grid, size_t smem, cudaStream_t stream) {
-    cudaFuncSetAttribute(exact_candidates_kernel<ST, METRIC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    exact_candidates_kernel<ST, METRIC><<<grid, K1_THREADS, smem, stream>>>(a);
+    cudaFuncSetAttribute(exact_candidates_kernel<ST, METRIC, RANGE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    exact_candidates_kernel<ST, METRIC, RANGE><<<grid, K1_THREADS, smem, stream>>>(a);
+}
+
+// ---- range search: bound, canonical re-evaluation, emit ----
+template <int ST, int METRIC>
+__global__ void range_bound_kernel(const float* q_nrm, const float* max_distance, uint32_t n, const float* x_nrm_max,
+                                   float rel, float sum, float* thr) {
+    const uint32_t q = blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= n) return;
+    const float qn = q_nrm[q], r = max_distance[q];
+    float eps = 0.0f;
+    if constexpr (Storage<ST>::kFloat)
+        eps = cert_margin<METRIC>(rel, sum, qn, *x_nrm_max);
+    else if constexpr (ST == VSB_ST_I8 && METRIC == VSB_METRIC_L2SQ)
+        eps = cert_margin<METRIC>(0.0f, sum, qn, *x_nrm_max);
+    float t = __fadd_ru(r, eps);
+    if constexpr (METRIC == VSB_METRIC_COS)
+        if (qn == 0.0f) t = __int_as_float(0x7F800000);
+    thr[q] = t;
+}
+
+constexpr int RE_WARPS = 8;
+
+template <int ST, int METRIC>
+__global__ void __launch_bounds__(RE_WARPS * 32) range_eval_kernel(K3Args a, const float* max_distance, const uint32_t* count,
+                                                                   const uint32_t* cursor, const uint32_t* seg_off,
+                                                                   const uint32_t* grp_off, uint32_t n_groups,
+                                                                   const uint64_t* cand, uint64_t* key_out,
+                                                                   uint32_t* dord_out, uint32_t* kept, uint32_t* mismatch) {
+    const int lane = threadIdx.x & 31;
+    const uint32_t w = blockIdx.x * RE_WARPS + (threadIdx.x >> 5);
+    if (w >= n_groups) return;
+    // the query of this group: the last q with grp_off[q] <= w (queries without entries own no group)
+    uint32_t lo = 0, hi = a.nq;
+    while (hi - lo > 1) {
+        const uint32_t mid = (lo + hi) / 2;
+        if (grp_off[mid] <= w) lo = mid;
+        else hi = mid;
+    }
+    const uint32_t q = lo, g = w - grp_off[q];
+    const uint32_t cnt = count[q];
+    const uint32_t have = min(cnt, cursor[q]);
+    const uint32_t base = seg_off[q] + 4 * g;
+    uint32_t slot[4];
+    bool on[4];
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+        on[u] = 4 * g + u < have;
+        slot[u] = on[u] ? packed_lo(cand[base + u]) : 0u;
+    }
+    float d[4];
+    k3_eval4<ST, METRIC>(a, reinterpret_cast<const uint4*>(a.q_rows + (size_t)q * a.q_row_bytes), a.x_row_bytes / 16,
+                         a.q_nrm[q], slot, on, d, lane);
+    const float r = max_distance[q];
+    uint32_t n_kept = 0;
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+        const bool keep = on[u] && d[u] <= r;
+        n_kept += keep ? 1u : 0u;
+        if (lane == u && 4 * g + u < cnt) {
+            key_out[base + u] = on[u] ? a.keys[slot[u]] : 0xFFFFFFFFFFFFFFFFull;
+            dord_out[base + u] = keep ? f32_to_ord(d[u]) : 0xFFFFFFFFu;
+        }
+    }
+    if (lane == 0 && n_kept != 0) atomicAdd(&kept[q], n_kept);
+}
+
+// queries whose fill-pass cursor differs from their count-pass count (queries without candidates included)
+__global__ void range_check_kernel(const uint32_t* count, const uint32_t* cursor, uint32_t n, uint32_t* mismatch) {
+    const uint32_t q = blockIdx.x * blockDim.x + threadIdx.x;
+    if (q < n && count[q] != cursor[q]) atomicAdd(mismatch, 1u);
+}
+
+__global__ void range_emit_kernel(const uint32_t* dord, const uint64_t* key, const uint32_t* seg_off, const uint32_t* out_off,
+                                  uint32_t n, uint32_t total, uint64_t* keys_out, float* dists_out) {
+    const uint32_t e = blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= total) return;
+    uint32_t lo = 0, hi = n;
+    while (hi - lo > 1) {
+        const uint32_t mid = (lo + hi) / 2;
+        if (out_off[mid] <= e) lo = mid;
+        else hi = mid;
+    }
+    const uint32_t src = seg_off[lo] + (e - out_off[lo]);
+    keys_out[e] = key[src];
+    dists_out[e] = ord_to_f32(dord[src]);
 }
 
 template <int ST, int METRIC>
@@ -751,6 +890,92 @@ void launch_exact_rerank(const ExactParams& p, uint32_t k, uint64_t* out_keys, f
     // small batches: a CTA per query (candidates spread over 8 warps) instead of a warp per query
     const bool cta = p.q.n <= 1024 && a.kp >= 8;
     VSB_DISPATCH_PAIR(p.storage, p.metric, (launch_k3<ST, METRIC>(a, cta, stream)));
+    g_kernel_launches += 1;
+}
+
+void launch_range_candidates(const ExactParams& p, const RangeParams& r, cudaStream_t stream) {
+    if (p.q.n == 0 || p.x_hi <= p.x_lo) return;
+    ExactParams pr = p;
+    pr.kp = 0;
+    K1Args a;
+    a.q_rows = pr.q.rows; a.q_sq = pr.q.sq; a.q_nrm = pr.q.nrm; a.nq = pr.q.n; a.q_row_bytes = pr.q.row_bytes;
+    a.x_rows = pr.x.rows; a.x_sq = pr.x.sq; a.x_nrm = pr.x.nrm; a.x_row_bytes = pr.x.row_bytes;
+    a.x_lo = pr.x_lo; a.x_hi = pr.x_hi;
+    a.deny = pr.deny; a.keys = pr.keys; a.allow = pr.allow.bm; a.allow_bits = pr.allow.bits; a.allow_of_q = pr.allow.of_q;
+    a.kp = 0; a.n_splits = pr.n_splits;
+    const uint32_t rows = pr.x_hi - pr.x_lo;
+    const uint32_t rps = (rows + pr.n_splits - 1) / pr.n_splits;
+    a.rows_per_split = ((rps + TN - 1) / TN) * TN;
+    const int eb = pr.storage == VSB_ST_F32 ? 32 : (pr.storage == VSB_ST_F16 || pr.storage == VSB_ST_BF16) ? 16
+                   : pr.storage == VSB_ST_I8 ? 8 : 1;
+    a.n_slabs = (pr.x.row_bytes * 8 / eb + BK - 1) / BK;
+    a.part = nullptr;
+    a.range = r;
+    dim3 grid((pr.q.n + TQ - 1) / TQ, pr.n_splits);
+    const size_t smem = (size_t)(BK * TQ + BK * TN) * 4 + (size_t)TQ * BUFCAP * 8 + TQ * 8;
+    VSB_DISPATCH_PAIR(pr.storage, pr.metric, (launch_k1<ST, METRIC, true>(a, grid, smem, stream)));
+    g_kernel_launches += 1;
+}
+
+void launch_range_bound(int storage, int metric, const float* q_nrm, const float* max_distance, uint32_t n,
+                        const float* x_nrm_max, float rel, float sum, float* thr, cudaStream_t stream) {
+    if (n == 0) return;
+    VSB_DISPATCH_PAIR(storage, metric,
+                      (range_bound_kernel<ST, METRIC><<<(n + 255) / 256, 256, 0, stream>>>(q_nrm, max_distance, n, x_nrm_max,
+                                                                                             rel, sum, thr)));
+    g_kernel_launches += 1;
+}
+
+void launch_range_eval(const ExactParams& p, const float* max_distance, const uint32_t* count, const uint32_t* cursor,
+                       const uint32_t* seg_off, const uint32_t* grp_off, uint32_t n_groups, const uint64_t* cand,
+                       uint64_t* key_out, uint32_t* dord_out, uint32_t* kept, uint32_t* mismatch, cudaStream_t stream) {
+    if (p.q.n == 0) return;
+    range_check_kernel<<<(p.q.n + 255) / 256, 256, 0, stream>>>(count, cursor, p.q.n, mismatch);
+    g_kernel_launches += 1;
+    if (n_groups == 0) return;
+    K3Args a{};
+    a.q_rows = p.q.rows; a.q_nrm = p.q.nrm; a.nq = p.q.n; a.q_row_bytes = p.q.row_bytes;
+    a.x_rows = p.x.rows; a.x_nrm = p.x.nrm; a.x_row_bytes = p.x.row_bytes;
+    a.keys = p.keys;
+    const uint32_t blocks = (n_groups + RE_WARPS - 1) / RE_WARPS;
+    VSB_DISPATCH_PAIR(p.storage, p.metric,
+                      (range_eval_kernel<ST, METRIC><<<blocks, RE_WARPS * 32, 0, stream>>>(
+                          a, max_distance, count, cursor, seg_off, grp_off, n_groups, cand, key_out, dord_out, kept, mismatch)));
+    g_kernel_launches += 1;
+}
+
+// Two segmented passes: by key (unique among live rows), then a STABLE pass by distance, which leaves equal
+// distances in key order.
+size_t range_sort_temp_bytes(uint32_t n_entries, uint32_t n_segments) {
+    size_t a = 0, b = 0;
+    cub::DeviceSegmentedSort::SortPairs(nullptr, a, (const uint64_t*)nullptr, (uint64_t*)nullptr, (const uint32_t*)nullptr,
+                                        (uint32_t*)nullptr, (int)n_entries, (int)n_segments, (const uint32_t*)nullptr,
+                                        (const uint32_t*)nullptr);
+    cub::DeviceSegmentedSort::StableSortPairs(nullptr, b, (const uint32_t*)nullptr, (uint32_t*)nullptr,
+                                              (const uint64_t*)nullptr, (uint64_t*)nullptr, (int)n_entries, (int)n_segments,
+                                              (const uint32_t*)nullptr, (const uint32_t*)nullptr);
+    return std::max(a, b);
+}
+
+cudaError_t launch_range_sort(uint32_t* dord, uint64_t* key, uint32_t* alt_dord, uint64_t* alt_key, uint32_t n_entries,
+                              const uint32_t* seg_off, uint32_t n_segments, void* temp, size_t temp_bytes,
+                              cudaStream_t stream) {
+    if (n_entries == 0) return cudaSuccess;
+    size_t tb = temp_bytes;
+    cudaError_t e = cub::DeviceSegmentedSort::SortPairs(temp, tb, key, alt_key, dord, alt_dord, (int)n_entries, (int)n_segments,
+                                                        seg_off, seg_off + 1, stream);
+    if (e != cudaSuccess) return e;
+    tb = temp_bytes;
+    e = cub::DeviceSegmentedSort::StableSortPairs(temp, tb, alt_dord, dord, alt_key, key, (int)n_entries, (int)n_segments,
+                                                  seg_off, seg_off + 1, stream);
+    g_kernel_launches += 2;
+    return e;
+}
+
+void launch_range_emit(const uint32_t* dord, const uint64_t* key, const uint32_t* seg_off, const uint32_t* out_off,
+                       uint32_t n, uint32_t total, uint64_t* keys_out, float* dists_out, cudaStream_t stream) {
+    if (total == 0) return;
+    range_emit_kernel<<<(total + 255) / 256, 256, 0, stream>>>(dord, key, seg_off, out_off, n, total, keys_out, dists_out);
     g_kernel_launches += 1;
 }
 

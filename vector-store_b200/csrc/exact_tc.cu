@@ -57,6 +57,9 @@ static_assert(TC2_STAGES * (TC_A_BYTES + TC_B_BYTES / 2) <= TC_OFF_BUF, "2-CTA s
 constexpr uint32_t kPeerBitMask = 0xFEFFFFFFu;  // shared::cluster address of the same offset in the even (leader) CTA
 
 enum { KIND_BF16 = 0, KIND_F16 = 1, KIND_TF32 = 2 };
+// epilogue modes: per-query k'-lists, each tile's best row per query (seed layer), every row within a fixed
+// per-query bound (range search: count or fill pass, see RangeParams)
+enum { MODE_LIST = 0, MODE_TILE_MIN = 1, MODE_RANGE = 2 };
 
 struct TcArgs {
     const float* q_sq;
@@ -77,6 +80,7 @@ struct TcArgs {
     uint32_t tile_step;        // rows between the starts of consecutive tiles (TC_N; larger = a tile-strided SAMPLE of the rows)
     uint32_t max_tiles;        // 0 = every tile of the split; else at most this many (sample passes)
     const float* thr_init;     // [nq] initial k'-th-best bound per query (nullable): rows farther than this are never listed
+    RangeParams range;         // MODE_RANGE only
 };
 
 // ---- PTX wrappers ------------------------------------------------------------------------------
@@ -299,14 +303,16 @@ __device__ __forceinline__ uint64_t make_smem_desc(uint32_t smem_addr) {
     return d;
 }
 
-// The list-maintaining form (TILE_MIN = false) runs as clusters of two CTAs (cta_group::2).  Each CTA owns its own
+// The list-maintaining and range forms run as clusters of two CTAs (cta_group::2).  Each CTA owns its own
 // 128 query rows (its half of the M = 256 accumulator) and stages only 128 of the tile's 256 corpus rows; the leader
 // CTA issues the MMAs for the pair, so a CTA moves 32 KB instead of 48 KB per K slab and a fourth stage fits
 // (1 046 vs 964 TFLOP/s on 10 000 x 1 M x 768 bf16).  The seed layer's tile-min form is tiny and runs as single CTAs.
-template <int KIND, int METRIC, bool TILE_MIN>
+template <int KIND, int METRIC, int MODE>
 __global__ void __launch_bounds__(TC_THREADS, 1)
     exact_candidates_tc_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_x,
                                TcArgs a) {
+    constexpr bool TILE_MIN = MODE == MODE_TILE_MIN;
+    constexpr bool RANGE = MODE == MODE_RANGE;
     constexpr bool CTA2 = !TILE_MIN;
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
@@ -447,7 +453,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1)
         const size_t list_stride = (size_t)a.n_splits * a.kp;
         uint64_t* warp_lists = a.part + ((size_t)(q0 + quarter * 32) * a.n_splits + list_id) * a.kp;
         const uint64_t* warp_buf = buf + ((size_t)half * TC_M + quarter * 32) * TC_BUFCAP;
-        if constexpr (!TILE_MIN) {  // (tile-min mode writes one dense entry per tile half; the caller pre-fills the padding)
+        if constexpr (MODE == MODE_LIST) {  // (tile-min mode writes one dense entry per tile half; the caller pre-fills the padding)
             for (int r = 0; r < 32; ++r) {
                 if (q0 + quarter * 32 + r >= a.nq) break;
                 uint64_t* list = warp_lists + (size_t)r * list_stride;
@@ -457,6 +463,12 @@ __global__ void __launch_bounds__(TC_THREADS, 1)
         }
         float thr = q_valid ? (a.thr_init != nullptr ? a.thr_init[q] : __int_as_float(0x7F800000)) : __int_as_float(0xFF800000);
         int cnt = 0;
+        // range mode: the bound is the query's own and never tightens; rcap = its count from the count pass
+        uint32_t rcnt = 0, rcap = 0;
+        if constexpr (RANGE) {
+            thr = q_valid ? a.range.thr[q] : __int_as_float(0xFF800000);
+            rcap = q_valid && a.range.off != nullptr ? a.range.count[q] : 0u;
+        }
         const uint32_t* deny = a.deny;
         // this thread's query row is tested against its own bitmap
         const uint32_t* allow = a.allow != nullptr && q_valid ? query_allow(a.allow, a.allow_bits, a.allow_of_q, q) : a.allow;
@@ -474,7 +486,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1)
             for (int c = lane; c < TC_HALF_N; c += 32) {
                 const uint32_t n = n0 + c;
                 float pv = __int_as_float(0x7FC00000);
-                if (n < r_hi) {
+                if (n < r_hi && !(RANGE && deny != nullptr && bit_test(deny, n))) {  // range mode: tombstones never hit
                     if constexpr (METRIC == VSB_METRIC_L2SQ) pv = a.x_sq[n];
                     else if constexpr (METRIC == VSB_METRIC_COS) {
                         const float xn = a.x_nrm[n];
@@ -511,6 +523,46 @@ __global__ void __launch_bounds__(TC_THREADS, 1)
                         for (int j = 31; j >= 0; --j)
                             if (d[j] == dmin) best_c = (uint32_t)(ch * 32 + j);
                         best_d = dmin;
+                    }
+                } else if constexpr (RANGE) {
+                    // hits are dense here (a bound of +inf hits every column): test, count and append straight from
+                    // the loaded registers
+                    float d[32];
+                    uint32_t hit = 0;
+#pragma unroll
+                    for (int j4 = 0; j4 < 8; ++j4) {
+                        const float4 p4 = cp4[j4];
+                        const float pj[4] = {p4.x, p4.y, p4.z, p4.w};
+#pragma unroll
+                        for (int jj = 0; jj < 4; ++jj) {
+                            const int j = j4 * 4 + jj;
+                            d[j] = tc_dist<METRIC>(__uint_as_float(v[j]), pj[jj], qpar);
+                            if (d[j] <= thr) hit |= 1u << j;  // NaN (masked column) never does
+                        }
+                    }
+                    if (allow != nullptr) {
+                        for (uint32_t h = hit; h != 0; h &= h - 1) {
+                            const int j = __ffs(h) - 1;
+                            const uint64_t rid = keys[n0 + ch * 32 + j] & kRowMask48;
+                            if (!(rid < allow_bits && bit_test(allow, (uint32_t)rid))) hit &= ~(1u << j);
+                        }
+                    }
+                    if (hit != 0) {
+                        if (a.range.off == nullptr) {
+                            rcnt += __popc(hit);
+                        } else {
+                            uint32_t pos = atomicAdd(&a.range.cursor[q], (uint32_t)__popc(hit));
+                            uint64_t* seg = a.range.out + a.range.off[q];
+#pragma unroll
+                            for (int j = 0; j < 32; ++j) {
+                                if (!((hit >> j) & 1u)) continue;
+                                float dd = d[j];
+                                if constexpr (METRIC == VSB_METRIC_L2SQ) dd = fmaxf(dd, 0.0f);
+                                if constexpr (METRIC == VSB_METRIC_COS) dd = fminf(fmaxf(dd, 0.0f), 2.0f);
+                                if (pos < rcap) seg[pos] = pack_ds(dd, n0 + ch * 32 + j);
+                                ++pos;
+                            }
+                        }
                     }
                 } else {
                     // bit j = column j of this chunk beats (or ties) the row's k'-th best; NaN never does
@@ -590,7 +642,10 @@ __global__ void __launch_bounds__(TC_THREADS, 1)
                 else mbar_arrive(&tmem_empty[acc]);
             }
         }
-        if constexpr (!TILE_MIN) {
+        if constexpr (RANGE) {
+            if (a.range.off == nullptr && rcnt != 0) atomicAdd(&a.range.count[q], rcnt);
+        }
+        if constexpr (MODE == MODE_LIST) {
             const uint32_t rest = __ballot_sync(kFullMask, cnt > 0);
             if (rest) tc_flush_rows(rest, warp_lists, list_stride, a.kp, keys, warp_buf, cnt, thr, lane);
         }
@@ -671,11 +726,11 @@ bool make_map(CUtensorMap* map, int kind, const void* base, uint32_t rows, uint3
     return r == CUDA_SUCCESS;
 }
 
-template <int KIND, int METRIC, bool TILE_MIN>
+template <int KIND, int METRIC, int MODE>
 void launch_tc_one(const CUtensorMap& mq, const CUtensorMap& mx, const TcArgs& a, dim3 grid, cudaStream_t stream) {
-    auto kern = exact_candidates_tc_kernel<KIND, METRIC, TILE_MIN>;
+    auto kern = exact_candidates_tc_kernel<KIND, METRIC, MODE>;
     cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TC_SMEM_BYTES);
-    if constexpr (!TILE_MIN) {  // CTA pairs
+    if constexpr (MODE != MODE_TILE_MIN) {  // CTA pairs
         cudaLaunchConfig_t cfg{};
         cfg.gridDim = grid;
         cfg.blockDim = dim3(TC_THREADS);
@@ -695,19 +750,59 @@ void launch_tc_one(const CUtensorMap& mq, const CUtensorMap& mx, const TcArgs& a
 }
 
 template <int KIND, int METRIC>
-void launch_tc_inst(const CUtensorMap& mq, const CUtensorMap& mx, const TcArgs& a, dim3 grid, cudaStream_t stream) {
-    if (a.tile_min) launch_tc_one<KIND, METRIC, true>(mq, mx, a, grid, stream);
-    else launch_tc_one<KIND, METRIC, false>(mq, mx, a, grid, stream);
+void launch_tc_inst(int mode, const CUtensorMap& mq, const CUtensorMap& mx, const TcArgs& a, dim3 grid, cudaStream_t stream) {
+    if (mode == MODE_TILE_MIN) launch_tc_one<KIND, METRIC, MODE_TILE_MIN>(mq, mx, a, grid, stream);
+    else if (mode == MODE_RANGE) launch_tc_one<KIND, METRIC, MODE_RANGE>(mq, mx, a, grid, stream);
+    else launch_tc_one<KIND, METRIC, MODE_LIST>(mq, mx, a, grid, stream);
 }
 
 template <int KIND>
-void launch_tc_kind(int metric, const CUtensorMap& mq, const CUtensorMap& mx, const TcArgs& a, dim3 grid,
+void launch_tc_kind(int metric, int mode, const CUtensorMap& mq, const CUtensorMap& mx, const TcArgs& a, dim3 grid,
                     cudaStream_t stream) {
     switch (metric) {
-        case VSB_METRIC_L2SQ: launch_tc_inst<KIND, VSB_METRIC_L2SQ>(mq, mx, a, grid, stream); break;
-        case VSB_METRIC_COS: launch_tc_inst<KIND, VSB_METRIC_COS>(mq, mx, a, grid, stream); break;
-        default: launch_tc_inst<KIND, VSB_METRIC_IP>(mq, mx, a, grid, stream); break;
+        case VSB_METRIC_L2SQ: launch_tc_inst<KIND, VSB_METRIC_L2SQ>(mode, mq, mx, a, grid, stream); break;
+        case VSB_METRIC_COS: launch_tc_inst<KIND, VSB_METRIC_COS>(mode, mq, mx, a, grid, stream); break;
+        default: launch_tc_inst<KIND, VSB_METRIC_IP>(mode, mq, mx, a, grid, stream); break;
     }
+}
+
+// one launch of exact_candidates_tc_kernel in `mode` (range: r = the pass's arrays)
+bool launch_tc(const ExactParams& p, cudaStream_t stream, int mode, const RangeParams* r) {
+    if (p.q.n == 0 || p.x_hi <= p.x_lo) return true;
+    const bool tile_min = mode == MODE_TILE_MIN;
+    const int kind = p.storage == VSB_ST_F32 ? KIND_TF32 : (p.storage == VSB_ST_BF16 ? KIND_BF16 : KIND_F16);
+    const bool cta2 = !tile_min;  // list and range launches run as CTA pairs
+    CUtensorMap mq, mx;
+    if (!make_map(&mq, kind, p.q.rows, p.q.n, p.q.row_bytes, TC_M)) return false;
+    if (!make_map(&mx, kind, p.x.rows, p.x_hi, p.x.row_bytes, cta2 ? TC_N / 2 : TC_N)) return false;
+    TcArgs a;
+    a.q_sq = p.q.sq; a.q_nrm = p.q.nrm; a.nq = p.q.n;
+    a.x_sq = p.x.sq; a.x_nrm = p.x.nrm; a.x_lo = p.x_lo; a.x_hi = p.x_hi; a.row_bytes = p.x.row_bytes;
+    a.deny = p.deny; a.keys = p.keys; a.allow = p.allow.bm; a.allow_bits = p.allow.bits; a.allow_of_q = p.allow.of_q;
+    a.kp = p.kp; a.n_splits = p.n_splits;
+    if (p.n_splits % TC_HALVES != 0) return false;  // callers size the lists with exact_tc_pick_splits
+    const uint32_t row_splits = p.n_splits / TC_HALVES;
+    const uint32_t rows = p.x_hi - p.x_lo;
+    const uint32_t rps = (rows + row_splits - 1) / row_splits;
+    a.rows_per_split = ((rps + TC_N - 1) / TC_N) * TC_N;
+    a.part = p.part;
+    a.tile_min = tile_min ? 1 : 0;
+    a.tile_min_stride = exact_tc_tile_min_entries(p.x_hi - p.x_lo);
+    a.tile_step = (mode == MODE_LIST && p.tile_step >= (uint32_t)TC_N) ? p.tile_step / TC_N * TC_N : (uint32_t)TC_N;
+    a.max_tiles = mode == MODE_LIST ? p.max_tiles : 0u;
+    a.thr_init = mode == MODE_LIST ? p.thr_init : nullptr;
+    if (r != nullptr) a.range = *r;
+    uint32_t q_tiles = (p.q.n + TC_M - 1) / TC_M;
+    if (cta2) q_tiles = (q_tiles + 1) & ~1u;  // CTA pairs: an odd tail tile gets an all-padding partner
+    dim3 grid(q_tiles, row_splits);
+    switch (kind) {
+        case KIND_BF16: launch_tc_kind<KIND_BF16>(p.metric, mode, mq, mx, a, grid, stream); break;
+        case KIND_F16: launch_tc_kind<KIND_F16>(p.metric, mode, mq, mx, a, grid, stream); break;
+        default: launch_tc_kind<KIND_TF32>(p.metric, mode, mq, mx, a, grid, stream); break;
+    }
+    g_kernel_launches += 1;
+    g_tc_launches += 1;
+    return true;
 }
 
 }  // namespace
@@ -761,39 +856,12 @@ uint32_t exact_tc_pick_splits(uint32_t nq, uint32_t n_rows, int sm_count, uint32
 // Same contract as launch_exact_candidates (exact.cu); returns false if the TMA descriptors could
 // not be encoded (caller falls back to the SIMT K1, which is still the CUDA path).
 bool launch_exact_candidates_tc(const ExactParams& p, cudaStream_t stream, bool tile_min) {
-    if (p.q.n == 0 || p.x_hi <= p.x_lo) return true;
-    const int kind = p.storage == VSB_ST_F32 ? KIND_TF32 : (p.storage == VSB_ST_BF16 ? KIND_BF16 : KIND_F16);
-    const bool cta2 = !tile_min;  // list launches run as CTA pairs
-    CUtensorMap mq, mx;
-    if (!make_map(&mq, kind, p.q.rows, p.q.n, p.q.row_bytes, TC_M)) return false;
-    if (!make_map(&mx, kind, p.x.rows, p.x_hi, p.x.row_bytes, cta2 ? TC_N / 2 : TC_N)) return false;
-    TcArgs a;
-    a.q_sq = p.q.sq; a.q_nrm = p.q.nrm; a.nq = p.q.n;
-    a.x_sq = p.x.sq; a.x_nrm = p.x.nrm; a.x_lo = p.x_lo; a.x_hi = p.x_hi; a.row_bytes = p.x.row_bytes;
-    a.deny = p.deny; a.keys = p.keys; a.allow = p.allow.bm; a.allow_bits = p.allow.bits; a.allow_of_q = p.allow.of_q;
-    a.kp = p.kp; a.n_splits = p.n_splits;
-    if (p.n_splits % TC_HALVES != 0) return false;  // callers size the lists with exact_tc_pick_splits
-    const uint32_t row_splits = p.n_splits / TC_HALVES;
-    const uint32_t rows = p.x_hi - p.x_lo;
-    const uint32_t rps = (rows + row_splits - 1) / row_splits;
-    a.rows_per_split = ((rps + TC_N - 1) / TC_N) * TC_N;
-    a.part = p.part;
-    a.tile_min = tile_min ? 1 : 0;
-    a.tile_min_stride = exact_tc_tile_min_entries(p.x_hi - p.x_lo);
-    a.tile_step = (!tile_min && p.tile_step >= (uint32_t)TC_N) ? p.tile_step / TC_N * TC_N : (uint32_t)TC_N;
-    a.max_tiles = tile_min ? 0u : p.max_tiles;
-    a.thr_init = tile_min ? nullptr : p.thr_init;
-    uint32_t q_tiles = (p.q.n + TC_M - 1) / TC_M;
-    if (cta2) q_tiles = (q_tiles + 1) & ~1u;  // CTA pairs: an odd tail tile gets an all-padding partner
-    dim3 grid(q_tiles, row_splits);
-    switch (kind) {
-        case KIND_BF16: launch_tc_kind<KIND_BF16>(p.metric, mq, mx, a, grid, stream); break;
-        case KIND_F16: launch_tc_kind<KIND_F16>(p.metric, mq, mx, a, grid, stream); break;
-        default: launch_tc_kind<KIND_TF32>(p.metric, mq, mx, a, grid, stream); break;
-    }
-    g_kernel_launches += 1;
-    g_tc_launches += 1;
-    return true;
+    return launch_tc(p, stream, tile_min ? MODE_TILE_MIN : MODE_LIST, nullptr);
+}
+
+// Same contract as launch_range_candidates (exact.cu); p.n_splits from exact_tc_pick_splits.
+bool launch_range_candidates_tc(const ExactParams& p, const RangeParams& r, cudaStream_t stream) {
+    return launch_tc(p, stream, MODE_RANGE, &r);
 }
 
 void launch_tc_sample_threshold(const uint64_t* sample_part, uint32_t nq, uint32_t m, float* thr, cudaStream_t stream) {

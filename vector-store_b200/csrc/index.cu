@@ -762,6 +762,34 @@ vsb_status vsb_search_filtered_multi(vsb_index* ix, const float* queries, uint64
     return ix->search_host(queries, q, k, keys, distances, counts, false, hf);
 }
 
+vsb_status vsb_search_range(vsb_index* ix, const float* queries, uint64_t q, const float* max_distance,
+                            const uint32_t* allow_bitmap, uint64_t bitmap_bits, uint64_t capacity, uint64_t* keys,
+                            float* distances, uint64_t* offsets) {
+    if (!ix) return fail(VSB_EINVAL, "null index");
+    if (!queries || !max_distance || !offsets) return fail(VSB_EINVAL, "null queries, max_distance or offsets");
+    if (capacity > 0 && (!keys || !distances)) return fail(VSB_EINVAL, "null keys or distances with capacity %llu",
+                                                           (unsigned long long)capacity);
+    for (uint64_t i = 0; i < q; ++i)
+        if (std::isnan(max_distance[i])) return fail(VSB_EINVAL, "max_distance[%llu] is NaN", (unsigned long long)i);
+    vsbi::HostFilters hf;
+    hf.bitmaps = allow_bitmap;
+    hf.n = allow_bitmap ? 1 : 0;
+    hf.bits = bitmap_bits;
+    vsbi::RangeResult r;
+    ST(ix->sharded ? vsbi::sharded_search_range(ix, queries, q, max_distance, hf, capacity, r)
+                   : ix->search_range(queries, q, max_distance, hf, capacity, keys, distances, r));
+    std::memcpy(offsets, r.off.data(), (size_t)(q + 1) * 8);
+    const uint64_t total = r.off[q];
+    if (total > capacity)
+        return fail(VSB_EFULL, "range search: %llu rows do not fit capacity %llu", (unsigned long long)total,
+                    (unsigned long long)capacity);
+    if (total > 0 && !r.in_place) {
+        std::memcpy(keys, r.keys.data(), (size_t)total * 8);
+        std::memcpy(distances, r.dists.data(), (size_t)total * 4);
+    }
+    return VSB_OK;
+}
+
 vsb_status vsb_search_dev(vsb_index* ix, const float* d_queries, uint64_t q, uint32_t k, uint64_t* d_keys,
                           float* d_distances, uint32_t* d_counts, void* stream, int exact) {
     if (!ix) return fail(VSB_EINVAL, "null index");

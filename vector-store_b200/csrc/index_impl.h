@@ -185,8 +185,11 @@ struct PinBuf {
     PinBuf() = default;
     PinBuf(const PinBuf&) = delete;
     PinBuf& operator=(const PinBuf&) = delete;
-    ~PinBuf() {
+    ~PinBuf() { release(); }
+    void release() {
         if (p) cudaFreeHost(p);
+        p = nullptr;
+        bytes = 0;
     }
     cudaError_t ensure(size_t want) {
         if (want <= bytes) return cudaSuccess;
@@ -311,10 +314,14 @@ struct Scratch {
     DevBuf rt_map, rt_fidx, rt_keys, rt_dists, rt_counts;
     RowBuf rt;
     DevBuf thr_part, thr, thr_cnt;                       // sampled list bounds of the all-pairs build (exact_block)
+    // range search: per-query arrays and the tombstone copy, candidate entries (at most 32 bytes x 2^24 are kept
+    // between calls; a larger sub-chunk's buffers are released when its call ends), sort scratch
+    DevBuf rg_q, rg_e, rg_sort;
     PinBuf pin;                                          // pinned staging of this caller class's read-backs
     size_t bytes() const {
         const DevBuf* all[] = {&q_in, &part, &seed_part, &tmp_keys, &tmp_dists, &rr_packed, &counters, &allow, &cert_state,
-                               &fb_map, &fb_fidx, &rt_map, &rt_fidx, &rt_keys, &rt_dists, &rt_counts, &thr_part, &thr, &thr_cnt};
+                               &fb_map, &fb_fidx, &rt_map, &rt_fidx, &rt_keys, &rt_dists, &rt_counts, &thr_part, &thr, &thr_cnt,
+                               &rg_q, &rg_e, &rg_sort};
         size_t s = q.bytes() + q16.bytes() + q8.bytes() + fb.bytes() + rt.bytes();
         for (auto* b : all) s += b->bytes;
         return s;
@@ -351,6 +358,15 @@ struct TopK {
     uint32_t* counts = nullptr;
     uint64_t* packed = nullptr;
     int64_t self_base = -1;
+};
+
+// the answer of a range search in host memory: query i's rows are keys / dists[off[i] .. off[i + 1]), ascending by
+// (distance, key); off has one entry per query plus one.  in_place: the rows were written to the caller's buffers
+// instead and keys / dists are empty.  When off.back() exceeds the call's capacity, keys and dists hold only a prefix.
+struct RangeResult {
+    std::vector<uint64_t> off, keys;
+    std::vector<float> dists;
+    bool in_place = false;
 };
 
 struct Sharded;  // sharded.cu: the multi-device router behind the same handle type
@@ -471,6 +487,16 @@ struct vsb_index {
     vsb_status stream_insert();
     vsb_status sample_seeds(uint32_t n_rows, bool ensure_reach = true);
 
+    // Error bounds of a tiled candidate stage over rows of `dim` elements (ExactCert.rel / .sum).  An fp32 sum of `dim`
+    // products, in any order, is within dim * 2^-24 |q||x| of the real dot product (2^-23 per add if the adder
+    // truncates); candidate and canonical evaluation together: dim * 2^-22 with margin.  TF32 tiles additionally keep
+    // only 10 mantissa bits of each operand: <= 2^-10 relative each, 2^-9 on the product.
+    float cert_rel(bool tf32) const {
+        const float rel_fp32 = (float)dim * 0x1p-22f;
+        return tf32 ? 1.25f * 0x1p-9f + rel_fp32 : rel_fp32;
+    }
+    float cert_sum() const { return (float)dim * 0x1p-23f; }
+
     // search building blocks: run on stream `s` with scratch `sc` against view `v`
     // the fixed inputs of an exact search of `q` over rows [x_lo, x_hi) of the view's store
     vsb::ExactParams exact_in(const vsbi::View& v, const vsb::RowsView& q, uint32_t x_lo, uint32_t x_hi,
@@ -498,6 +524,11 @@ struct vsb_index {
                           uint32_t* d_counts, cudaStream_t s, bool exact, const vsbi::Filters& f = vsbi::Filters());
     vsb_status search_host(const float* queries, uint64_t nq, uint32_t k, uint64_t* keys_out, float* dists_out,
                            uint32_t* counts_out, bool exact, const vsbi::HostFilters& hf = vsbi::HostFilters());
+    // range search (index_range.cu): every live admissible row within max_distance[i] of query i, exact.  out.off gets
+    // the offsets; the rows go straight to keys_out / dists_out (nullable) when the call's candidates fit `capacity`
+    // (out.in_place), into out.keys / out.dists otherwise; rows past `capacity` in total are counted, not collected
+    vsb_status search_range(const float* queries, uint64_t nq, const float* max_distance, const vsbi::HostFilters& hf,
+                            uint64_t capacity, uint64_t* keys_out, float* dists_out, vsbi::RangeResult& out);
 };
 
 namespace vsbi {

@@ -141,13 +141,8 @@ vsb_status vsb_index::exact_block(Scratch& sc, const vsb::ExactParams& in, uint3
     cert.x_nrm_max = d_xmax;
     cert.flags = d_flags;
     cert.count = d_count;
-    // An fp32 sum of `dim` products, in any order, is within dim * 2^-24 |q||x| of the real dot product (2^-23 per
-    // add if the adder truncates); candidate and canonical evaluation together: dim * 2^-22 with margin.
-    // TF32 additionally keeps only 10 mantissa bits of each operand: <= 2^-10 relative each, 2^-9 on the product.
-    const float rel_fp32 = (float)dim * 0x1p-22f;
-    const float rel_tf32 = 1.25f * 0x1p-9f + rel_fp32;
-    cert.sum = (float)dim * 0x1p-23f;
-    cert.rel = (tc && storage == VSB_F32) ? rel_tf32 : rel_fp32;
+    cert.sum = cert_sum();
+    cert.rel = cert_rel(tc && storage == VSB_F32);
 
     // flagged queries of one stage -> compact map (indices into the caller's query block) + gathered rows, and the
     // gathered bitmap index of each query (a filtered call whose queries carry their own bitmaps)
@@ -189,7 +184,7 @@ vsb_status vsb_index::exact_block(Scratch& sc, const vsb::ExactParams& in, uint3
         pf.part = sc.part.as<uint64_t>();
         vsb::launch_exact_candidates(pf, s);
         CU(cudaGetLastError());
-        cert.rel = rel_fp32;
+        cert.rel = cert_rel(false);
         CU(cudaMemsetAsync(d_count, 0, 4, s));
         vsb::launch_exact_rerank(pf, k, out.keys, out.dists, out.counts, out.packed, self_base, s, &cert,
                                  sc.fb_map.as<uint32_t>());

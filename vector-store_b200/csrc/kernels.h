@@ -94,6 +94,58 @@ uint32_t exact_scan_lists_per_query(uint32_t n_splits);
 void launch_exact_scan(const ExactParams& p, uint32_t k, cudaStream_t stream);
 void launch_max_norm(const float* nrm, uint32_t lo, uint32_t hi, float* out, cudaStream_t stream);
 
+// Bound on |candidate-stage distance - canonical distance| for every row of a block whose largest row norm is xm:
+// rel bounds the dot-product error relative to |q||x|, sum the rounding of an fp32 sum of `dim` terms (the norms of
+// the L2 expansion, the canonical sum itself).  The K3 certificate and the range-search margin both use it.
+template <int METRIC>
+__host__ __device__ __forceinline__ float cert_margin(float rel, float sum, float qn, float xm) {
+    if constexpr (METRIC == VSB_METRIC_COS)
+        return rel + 1e-6f;
+    else if constexpr (METRIC == VSB_METRIC_L2SQ)
+        return (rel + sum) * (qn * qn + xm * xm);
+    else
+        return rel * qn * xm + 0x1p-22f * (1.0f + qn * xm);
+}
+
+// Range search: the K1 tiles with a fixed per-query bound instead of a k'-list (exact.cu, exact_tc.cu).
+//   count pass (off == nullptr): count[q] += admissible rows whose candidate-stage distance is <= thr[q]
+//   fill pass: the same rows, as packed (candidate distance, slot) entries, go to out[off[q] + i] for
+//              i = cursor[q]++ (space reserved once per flush), and only while i < count[q]; the caller checks that
+//              every cursor ends equal to its count
+struct RangeParams {
+    const float* thr = nullptr;     // [q.n]
+    uint32_t* count = nullptr;      // [q.n]
+    const uint32_t* off = nullptr;  // [q.n] segment starts in out (fill pass)
+    uint32_t* cursor = nullptr;     // [q.n] zeroed by the caller (fill pass)
+    uint64_t* out = nullptr;
+};
+void launch_range_candidates(const ExactParams& p, const RangeParams& r, cudaStream_t stream);
+// false if the TMA descriptors could not be encoded (nothing launched)
+bool launch_range_candidates_tc(const ExactParams& p, const RangeParams& r, cudaStream_t stream);
+// thr[q] = max_distance[q] + cert_margin(rel, sum, |q|, *x_nrm_max), rounded up; integer storages are exact in the
+// candidate stage (margin 0) except int8 L2sq, whose norm expansion can round above 2^24; cosine queries of norm 0
+// get +inf (their candidate distance is 1, the canonical one 0 or 1)
+void launch_range_bound(int storage, int metric, const float* q_nrm, const float* max_distance, uint32_t n,
+                        const float* x_nrm_max, float rel, float sum, float* thr, cudaStream_t stream);
+// Canonical re-evaluation of the fill pass's entries, four rows per warp (K3's evaluation).  Query q's segment is
+// cand[seg_off[q] .. seg_off[q + 1]), its warps are groups grp_off[q] .. grp_off[q + 1] (ceil(count / 4) each).  Per
+// entry: key_out = its key, dord_out = ord(canonical distance) if that is <= max_distance[q], else 0xFFFFFFFF;
+// kept[q] += rows kept.  *mismatch += queries of p.q whose cursor differs from their count, every query checked
+// (entries past the smaller of the two are never read).
+void launch_range_eval(const ExactParams& p, const float* max_distance, const uint32_t* count, const uint32_t* cursor,
+                       const uint32_t* seg_off, const uint32_t* grp_off, uint32_t n_groups, const uint64_t* cand,
+                       uint64_t* key_out, uint32_t* dord_out, uint32_t* kept, uint32_t* mismatch, cudaStream_t stream);
+// Sorts every segment of (dord, key) by (dord, key) in place; alt_* are buffers of the same size, temp from
+// range_sort_temp_bytes.  Deterministic.
+size_t range_sort_temp_bytes(uint32_t n_entries, uint32_t n_segments);
+cudaError_t launch_range_sort(uint32_t* dord, uint64_t* key, uint32_t* alt_dord, uint64_t* alt_key, uint32_t n_entries,
+                              const uint32_t* seg_off, uint32_t n_segments, void* temp, size_t temp_bytes,
+                              cudaStream_t stream);
+// Output entry e of query q (out_off[q] <= e < out_off[q + 1]) = entry seg_off[q] + (e - out_off[q]) of the sorted
+// segments, as (key, float distance).
+void launch_range_emit(const uint32_t* dord, const uint64_t* key, const uint32_t* seg_off, const uint32_t* out_off,
+                       uint32_t n, uint32_t total, uint64_t* keys_out, float* dists_out, cudaStream_t stream);
+
 // K1 on tcgen05 tensor cores (exact_tc.cu): same contract as launch_exact_candidates.
 bool exact_tc_supported(int storage, int metric);
 uint32_t exact_tc_pick_splits(uint32_t nq, uint32_t n_rows, int sm_count, uint32_t kp);

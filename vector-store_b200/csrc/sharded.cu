@@ -471,6 +471,48 @@ vsb_status sharded_search_host(vsb_index* ix, const float* queries, uint64_t nq,
     return VSB_OK;
 }
 
+vsb_status sharded_search_range(vsb_index* ix, const float* queries, uint64_t nq, const float* max_distance,
+                                const HostFilters& hf, uint64_t capacity, RangeResult& out) {
+    Sharded& S = *ix->sharded;
+    std::lock_guard<std::mutex> g(S.search);
+    const uint32_t G = S.G();
+    // a shard's total never exceeds the merged one, so each shard may stop collecting at the same capacity
+    std::vector<RangeResult> part(G);
+    ST(S.for_each([&](uint32_t i) { return S.shards[i]->search_range(queries, nq, max_distance, hf, capacity, nullptr, nullptr, part[i]); }));
+    out.off.assign(nq + 1, 0);
+    for (uint64_t q = 0; q < nq; ++q) {
+        uint64_t n = 0;
+        for (uint32_t i = 0; i < G; ++i) n += part[i].off[q + 1] - part[i].off[q];
+        out.off[q + 1] = out.off[q] + n;
+    }
+    out.keys.clear();
+    out.dists.clear();
+    if (out.off[nq] > capacity) return VSB_OK;
+    out.keys.resize(out.off[nq]);
+    out.dists.resize(out.off[nq]);
+    // per query: G-way merge of the shards' sorted segments (keys are unique across shards)
+    std::vector<uint64_t> pos(G);
+    for (uint64_t q = 0; q < nq; ++q) {
+        for (uint32_t i = 0; i < G; ++i) pos[i] = part[i].off[q];
+        for (uint64_t o = out.off[q]; o < out.off[q + 1]; ++o) {
+            uint32_t best = G;
+            for (uint32_t i = 0; i < G; ++i) {
+                if (pos[i] == part[i].off[q + 1]) continue;
+                if (best == G) {
+                    best = i;
+                    continue;
+                }
+                const float d = part[i].dists[pos[i]], db = part[best].dists[pos[best]];
+                if (d < db || (d == db && part[i].keys[pos[i]] < part[best].keys[pos[best]])) best = i;
+            }
+            out.keys[o] = part[best].keys[pos[best]];
+            out.dists[o] = part[best].dists[pos[best]];
+            ++pos[best];
+        }
+    }
+    return VSB_OK;
+}
+
 vsb_status sharded_save(vsb_index* ix, const char* path) {
     Sharded& S = *ix->sharded;
     std::lock_guard<std::mutex> g(S.mut);

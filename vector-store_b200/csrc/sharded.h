@@ -24,6 +24,9 @@ vsb_status sharded_search_host(vsb_index* ix, const float* queries, uint64_t nq,
                                float* dists, uint32_t* counts, bool exact, const HostFilters& hf = HostFilters());
 vsb_status sharded_search_dev(vsb_index* ix, const float* d_queries, uint64_t nq, uint32_t k, uint64_t* d_keys,
                               float* d_dists, uint32_t* d_counts, cudaStream_t stream, bool exact);
+// every shard's range search, merged per query by (distance, key); capacity as in search_range
+vsb_status sharded_search_range(vsb_index* ix, const float* queries, uint64_t nq, const float* max_distance,
+                                const HostFilters& hf, uint64_t capacity, RangeResult& out);
 vsb_status sharded_save(vsb_index* ix, const char* path);
 
 // snapshot_io.cu

@@ -230,6 +230,38 @@ class GpuIndex:
                                                   _ptr(keys), _ptr(dists), _ptr(counts)))
         return keys, dists, counts
 
+    def search_range(self, queries, max_distance, allow_mask=None):
+        """Range search, exact: for query i every live row whose distance is <= max_distance[i] (and, with allow_mask,
+        whose id key & 2^48-1 is admitted, as in search_filtered), ascending by (distance, key).  max_distance is a
+        scalar or one value per query (+inf returns every admissible row).  -> (offsets u64 [n + 1], keys u64 [total],
+        dists f32 [total]); query i's rows are keys[offsets[i]:offsets[i + 1]].  The result size is not known before
+        the call: the first attempt has room for 256 rows per query, and if that is too small (VSB_EFULL, which
+        costs a full search) the call is made once more with exactly offsets[-1] rows of room."""
+        q = np.ascontiguousarray(queries, dtype=np.float32)
+        self._check_dim(q)
+        n = q.shape[0]
+        r = np.ascontiguousarray(np.broadcast_to(np.asarray(max_distance, dtype=np.float32), (n,)))
+        bm, bits = None, 0
+        if allow_mask is not None:
+            mask = np.asarray(allow_mask, dtype=bool)
+            bm = np.packbits(mask, bitorder="little")
+            bm = np.concatenate([bm, np.zeros((-len(bm)) % 4, np.uint8)]).view(np.uint32)
+            bits = len(mask)
+        offsets = np.zeros(n + 1, dtype=np.uint64)
+        cap = 256 * n
+        for attempt in range(2):
+            keys = np.empty(cap, dtype=np.uint64)
+            dists = np.empty(cap, dtype=np.float32)
+            st = self._lib.vsb_search_range(self._h, _ptr(q), n, _ptr(r), _ptr(bm), bits, cap, _ptr(keys), _ptr(dists),
+                                            _ptr(offsets))
+            if st == native.VSB_EFULL and attempt == 0:
+                cap = int(offsets[-1])
+                continue
+            check(st)
+            break
+        total = int(offsets[-1])
+        return offsets, keys[:total], dists[:total]
+
     def search_raw(self, q_ptr: int, n: int, k: int, keys_ptr: int, dists_ptr: int, counts_ptr: int,
                    exact: bool = False) -> None:
         """Host-pointer call without NumPy marshalling (bench e2e leg uses pinned torch buffers)."""

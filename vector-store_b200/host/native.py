@@ -76,6 +76,7 @@ SYMBOLS = [
     ("vsb_search_exact", C.c_int, [_P, _P, C.c_uint64, C.c_uint32, _P, _P, _P]),
     ("vsb_search_filtered", C.c_int, [_P, _P, C.c_uint64, C.c_uint32, _P, C.c_uint64, _P, _P, _P]),
     ("vsb_search_filtered_multi", C.c_int, [_P, _P, C.c_uint64, C.c_uint32, _P, C.c_uint32, C.c_uint64, _P, _P, _P, _P]),
+    ("vsb_search_range", C.c_int, [_P, _P, C.c_uint64, _P, _P, C.c_uint64, C.c_uint64, _P, _P, _P]),
     ("vsb_search_dev", C.c_int, [_P, _P, C.c_uint64, C.c_uint32, _P, _P, _P, _P, C.c_int]),
     ("vsb_merge_topk_dev", C.c_int, [_P, _P, C.c_uint32, C.c_uint64, C.c_uint32, _P, _P, _P, C.c_int, _P]),
     ("vsb_batcher_create", C.c_int, [_P, C.c_uint32, C.c_uint32, C.c_uint32, C.POINTER(_P)]),
