@@ -286,6 +286,59 @@ constexpr int k4_min_blocks() { return (ST == VSB_ST_I8 && CPL <= 2) ? 4 : 3; }
 template <int CPL, bool MMA>
 constexpr int k4_rows_per_group() { return CPL <= 3 ? 4 : (CPL <= 6 ? 2 : 1); }
 
+// Searches return hits ascending by (distance, key) (vsb200.h), but the beam list is ordered by the packed word, i.e. by
+// (distance, slot | kExpandedBit).  Before keys are emitted, one warp re-sorts the part of `list` that the emit loop
+// reads, up to the end of the run of equal distances that holds the last emitted entry, by (distance, key): ties are
+// then returned in key order, and a run of ties that crosses position k gives up its smallest keys.  The expanded bit
+// is dropped on the way.  `tmp` holds at least that part rounded up to 32 entries.  Lists without two adjacent equal
+// distances in that part are left alone.  `valid_of(e)` is the emit loop's test of an entry.
+template <class Valid>
+__device__ __forceinline__ void order_ties_by_key(uint64_t* list, uint32_t len, uint64_t* tmp, uint32_t k,
+                                                  const uint64_t* keys, int lane, Valid valid_of) {
+    // distance of the last entry the emit loop will write
+    uint32_t count = 0, hi_last = 0;
+    for (uint32_t b = 0; b < len && count < k; b += 32) {
+        const uint64_t e = list[b + lane];
+        const bool valid = valid_of(e);
+        const uint32_t m = __ballot_sync(kFullMask, valid);
+        const uint32_t em = __ballot_sync(kFullMask, valid && count + __popc(m & ((1u << lane) - 1)) < k);
+        const uint32_t hi_src = __shfl_sync(kFullMask, packed_hi(e), em ? 31 - __clz(em) : 0);
+        if (em) hi_last = hi_src;
+        count += __popc(m);
+    }
+    if (count == 0) return;
+    // the prefix [0, n_pre) that ends with the last entry at or below that distance, whether two of its entries are
+    // tied, and whether it holds an empty entry (K4b's parallel merge can leave one where two candidates coincide)
+    uint32_t n_pre = 0, first_hole = len;
+    bool tie = false;
+    for (uint32_t b = 0; b < len; b += 32) {
+        const uint64_t e = list[b + lane];
+        const uint32_t hi = packed_hi(e);
+        const bool in = e != kInvalidPacked && hi <= hi_last;
+        uint32_t hi_next = __shfl_down_sync(kFullMask, hi, 1);
+        if (lane == 31) hi_next = b + 32 < len ? packed_hi(list[b + 32]) : 0xFFFFFFFFu;
+        const uint32_t mi = __ballot_sync(kFullMask, in);
+        const uint32_t mh = __ballot_sync(kFullMask, e == kInvalidPacked);
+        tie = tie || __ballot_sync(kFullMask, in && hi_next == hi) != 0;
+        if (mi) n_pre = b + 32 - __clz(mi);
+        if (mh && first_hole == len) first_hole = b + __ffs(mh) - 1;
+        if (__ballot_sync(kFullMask, e != kInvalidPacked && hi > hi_last)) break;
+    }
+    if (!tie && first_hole >= n_pre) return;
+    const LessByKey by_key{keys};
+    const uint32_t pad = (n_pre + 31) & ~31u;
+    for (uint32_t i = lane; i < pad; i += 32) tmp[i] = kInvalidPacked;
+    __syncwarp();
+    for (uint32_t b = 0; b < pad; b += 32) {
+        uint64_t v = b + lane < n_pre ? list[b + lane] : kInvalidPacked;
+        if (v != kInvalidPacked) v &= ~(uint64_t)kExpandedBit;  // empty entries stay empty and sort last
+        v = warp_sort32(v, lane, by_key);
+        warp_list_merge(tmp, (int)(b + 32), v, lane, by_key);
+    }
+    for (uint32_t i = lane; i < n_pre; i += 32) list[i] = tmp[i];
+    __syncwarp();
+}
+
 // FILTER = true (vsb_search_filtered): the traversal is unchanged, but every evaluated row whose key is admissible is
 // ALSO folded into a second list of rk entries, and that list is what the kernel emits.  The beam still walks through
 // inadmissible rows, exactly like usearch's predicate search (usearch.rs:224-248).
@@ -406,9 +459,12 @@ __global__ void __launch_bounds__(K4_WARPS * 32, k4_min_blocks<ST, CPL, MMA>()) 
                     const uint64_t row_id = a.keys[packed_lo(res)] & kRowMask48;
                     if (row_id < a.allow_bits && (allow[row_id >> 5] >> (row_id & 31) & 1u)) adm = res;
                 }
-                if (__ballot_sync(kFullMask, adm < rlist[a.rk - 1]) != 0) {
-                    adm = warp_sort32(adm, lane, less);
-                    warp_list_merge(rlist, (int)a.rk, adm, lane, less);
+                // the result list is kept by (distance, key) from the start: it is truncated at rk while it fills, and
+                // of more than rk tied rows the ones with the smallest keys must stay
+                const LessByKey by_key{a.keys};
+                if (__ballot_sync(kFullMask, by_key(adm, rlist[a.rk - 1])) != 0) {
+                    adm = warp_sort32(adm, lane, by_key);
+                    warp_list_merge(rlist, (int)a.rk, adm, lane, by_key);
                 }
             }
             const bool keep = res < worst;
@@ -513,15 +569,24 @@ __global__ void __launch_bounds__(K4_WARPS * 32, k4_min_blocks<ST, CPL, MMA>()) 
 
     // ---- emit the first k live entries (of the admissible list when filtering) ----
     __syncwarp();
-    const uint64_t* src_list = FILTER ? rlist : list;
+    uint64_t* src_list = FILTER ? rlist : list;
     const uint32_t src_len = FILTER ? a.rk : a.itopk;
-    uint32_t count = 0;
-    for (uint32_t b = 0; b < src_len; b += 32) {
-        const uint64_t e = src_list[b + lane];
+    auto valid_of = [&](uint64_t e) {
         const uint32_t slot = packed_lo(e) & ~kExpandedBit;
         bool valid = e != kInvalidPacked;
         if (valid && a.deny != nullptr && bit_test(a.deny, slot)) valid = false;
         if (valid && a.self_base >= 0 && slot == (uint32_t)(a.self_base + q)) valid = false;
+        return valid;
+    };
+    // the visited hash (2 << hash_bits bytes, 1024 entries at K4_HASH_BITS = 12 >= itopk) is free from here on; the
+    // FILTER result list is already ordered by key
+    if (!FILTER && a.out_packed == nullptr)
+        order_ties_by_key(src_list, src_len, reinterpret_cast<uint64_t*>(hash), a.k, a.keys, lane, valid_of);
+    uint32_t count = 0;
+    for (uint32_t b = 0; b < src_len; b += 32) {
+        const uint64_t e = src_list[b + lane];
+        const uint32_t slot = packed_lo(e) & ~kExpandedBit;
+        const bool valid = valid_of(e);
         const uint32_t m = __ballot_sync(kFullMask, valid);
         const uint32_t pos = count + __popc(m & ((1u << lane) - 1));
         if (valid && pos < a.k) {
@@ -784,13 +849,20 @@ __global__ void __launch_bounds__(K4B_WARPS * 32, 1) graph_search_cta_kernel(K4A
 
     // ---- emit (warp 0) ----
     if (warp == 0) {
-        uint32_t count = 0;
-        for (uint32_t b = 0; b < a.itopk; b += 32) {
-            const uint64_t e = list[b + lane];
+        auto valid_of = [&](uint64_t e) {
             const uint32_t slot = packed_lo(e) & ~kExpandedBit;
             bool valid = e != kInvalidPacked;
             if (valid && a.deny != nullptr && bit_test(a.deny, slot)) valid = false;
             if (valid && a.self_base >= 0 && slot == (uint32_t)(a.self_base + q)) valid = false;
+            return valid;
+        };
+        // the other list buffer is free from here on
+        if (a.out_packed == nullptr) order_ties_by_key(list, a.itopk, list_alt, a.k, a.keys, lane, valid_of);
+        uint32_t count = 0;
+        for (uint32_t b = 0; b < a.itopk; b += 32) {
+            const uint64_t e = list[b + lane];
+            const uint32_t slot = packed_lo(e) & ~kExpandedBit;
+            const bool valid = valid_of(e);
             const uint32_t m = __ballot_sync(kFullMask, valid);
             const uint32_t pos = count + __popc(m & ((1u << lane) - 1));
             if (valid && pos < a.k) {
